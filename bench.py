@@ -5,9 +5,15 @@ lamda = 0.1), reported as masks/s (one mask = one image's 14-class stack = 14 ma
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the oracle port on host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also write the last timed step's outputs
 
 Under torchrun (N > 1) every rank processes its own 64 images (weak scaling); the only collective is
 the all-reduce of the scalar loss.  Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR writes what the last timed (device-resident) step handed its caller, so that two builds can be
+compared output for output on identical seeded inputs: DIR/loss.npy (float32, 0-d) and DIR/grad_sample.npy
+(float32, rank 0's gradient d loss / d pred flattened and taken at sample_index(pred.numel()), a fixed seeded
+set of at most DUMP_MAX_ELEMS positions: 32 MB).
 """
 from __future__ import annotations
 
@@ -31,6 +37,31 @@ E2E_CHUNKS = 16  # upper bound on the groups of whole images whose H2D copy over
 # full-resolution stress test (1024^2 x 14, bs 128 over 8 GPUs = 16 images per GPU)
 CONFIGS = {"c2": dict(side=256, batch=64, seed=2, name="C2"), "c5": dict(side=1024, batch=16, seed=5, name="C5")}
 METRIC = "topo-loss fwd+bwd masks/sec (256^2, 14 cls)"
+DUMP_SEED = 0
+DUMP_MAX_ELEMS = 1 << 23  # float32 gradient positions written by --dump-outputs (32 MB)
+
+
+def input_seed(cfg, rank=0):
+    """Seed of make_batch for a config's inputs on one rank: the same arguments give the same inputs."""
+    return 1234 + 1000 * cfg["seed"] + rank
+
+
+def sample_index(n: int):
+    """Sorted flat positions of the fixed, seeded sample that --dump-outputs takes of an n-element output."""
+    import torch
+    if n <= DUMP_MAX_ELEMS:
+        return torch.arange(n)
+    g = torch.Generator().manual_seed(DUMP_SEED)
+    return torch.unique(torch.randint(0, n, (DUMP_MAX_ELEMS,), generator=g))
+
+
+def dump_outputs(out_dir, loss, grad):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    flat = grad.detach().reshape(-1)
+    sample = flat[sample_index(flat.numel()).to(flat.device)]
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "grad_sample.npy"), sample.float().cpu().numpy())
 
 
 def _metric(side):
@@ -217,7 +248,7 @@ def run_reference(args, rank, world):
     B = args.batch or cfg["batch"]
     cores = _host_cores()
     sample = min(args.ref_images or B, B)
-    pred, truth = make_batch(B, H, W, seed=1234 + 1000 * cfg["seed"], device="cpu")
+    pred, truth = make_batch(B, H, W, seed=input_seed(cfg), device="cpu")
     pred, truth = pred[:sample].contiguous(), truth[:sample].contiguous()
     value, dt = cpu_arm(pred, truth, cores, args.steps, max(1, min(args.warmup, 1)))
     what = "the whole batch" if sample == B else f"the first {sample} of {B} images"
@@ -249,7 +280,13 @@ def main():
     ap.add_argument("--ref-images", type=int, default=0, help="images per step of the CPU arm (default: the whole batch)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="images of the cpu_baseline sample (default: ~10 s of CPU work)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss and a seeded sample of its "
+                                                          "gradient as DIR/<name>.npy (CUDA path only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -285,7 +322,7 @@ def main():
     B = args.batch or cfg["batch"]
     gb = B * world
 
-    pred, truth = make_batch(B, H, W, seed=1234 + 1000 * cfg["seed"] + rank, device=dev)
+    pred, truth = make_batch(B, H, W, seed=input_seed(cfg, rank), device=dev)
     pred_h = pred.cpu().pin_memory()
     # one-hot ground truth is {0, 1}: it crosses PCIe as bits (numpy.packbits) and is widened on the device
     # (the reference builds these masks on the CPU, training_utils.py:413, :432)
@@ -300,9 +337,10 @@ def main():
             part = topo_loss_sharded(p, truth, LAMDA, feat_d=FEAT_D, loss_q=LOSS_Q, global_batch=gb, reduce="local")
             total = reduce_scalar_async(part)
             part.backward()
-            total.result()
-        else:
-            tlb.topo_loss(p, truth, LAMDA, feat_d=FEAT_D, loss_q=LOSS_Q).backward()
+            return total.result()
+        loss = tlb.topo_loss(p, truth, LAMDA, feat_d=FEAT_D, loss_q=LOSS_Q)
+        loss.backward()
+        return loss
 
     def step_e2e():
         # host-resident (pinned) inputs through the public host API: H2D copies are pipelined against
@@ -324,13 +362,13 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         sync_all()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms) / steps
+        return float(ms) / steps, out  # out: what the last step returned
 
     try:
         uuid = "GPU-" + str(torch.cuda.get_device_properties(dev).uuid)
@@ -349,7 +387,7 @@ def main():
     if rank == 0:
         sampler.mark()
     L.tl_timing_enable(1)
-    ms_step = timed(step_resident, args.steps)
+    ms_step, last_loss = timed(step_resident, args.steps)
     sums = (ctypes.c_float * 6)()
     calls = (ctypes.c_int * 2)()
     L.tl_timing_read(sums, calls)
@@ -359,7 +397,7 @@ def main():
 
     for _ in range(3):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     clocks = None
     if rank == 0:
         try:
@@ -371,6 +409,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:  # the end-to-end steps use their own buffers: p.grad is still the last timed step's
+        dump_outputs(args.dump_outputs, last_loss, p.grad)
 
     value = gb / (ms_step * 1e-3)
     e2e_value = gb / (ms_e2e * 1e-3)
