@@ -13,6 +13,9 @@
 // per warp and channel) and walks the channels once, carrying the online-softmax state of its pixels;
 // the per-channel Dice sums are reduced per warp with shuffles, per tile in shared memory and per image with
 // fp64 atomics.  The backward recomputes the per-pixel log-sum-exp and writes the dense logit gradient.
+// expf / logf, not the __expf / __logf intrinsics: the intrinsics' error grows with |x| (2 + 1.173 |x| ulp), and a
+// trained decoder's logits reach +-20..40, where the Dice term of an empty mask is as sensitive as sum sigmoid(x) is
+// small (tests/test_fused_ops_edges.py, the saturated cases).  The kernel is memory-bound either way.
 #pragma once
 #include "tl_common.cuh"
 
@@ -62,10 +65,10 @@ __global__ void __launch_bounds__(kDcThreads) dice_ce_fwd_kernel(DiceCeArgs A) {
             for (int k = 0; k < kDcPix; ++k) {
                 if (p0 + k * kDcThreads < HW) {
                     const float x = xv[k], t = tv[k];
-                    const float sg = 1.f / (1.f + __expf(-x));
+                    const float sg = 1.f / (1.f + expf(-x));
                     I += sg * t; P += sg; G += t;
                     const float mn = fmaxf(m[k], x);
-                    s[k] = s[k] * __expf(m[k] - mn) + __expf(x - mn);
+                    s[k] = s[k] * expf(m[k] - mn) + expf(x - mn);
                     m[k] = mn;
                     dot[k] += t * x; ts[k] += t;
                 }
@@ -78,7 +81,7 @@ __global__ void __launch_bounds__(kDcThreads) dice_ce_fwd_kernel(DiceCeArgs A) {
         }
 #pragma unroll
         for (int k = 0; k < kDcPix; ++k)
-            if (p0 + k * kDcThreads < HW) ce_total += (double)(ts[k] * (m[k] + __logf(s[k])) - dot[k]);
+            if (p0 + k * kDcThreads < HW) ce_total += (double)(ts[k] * (m[k] + logf(s[k])) - dot[k]);
         __syncthreads();
         for (int i = tid; i < 3 * C; i += kDcThreads) atomicAdd(A.acc + (size_t)b * C * 3 + i, (double)(&s_acc[0][0])[i]);
         __syncthreads();
@@ -128,7 +131,7 @@ __global__ void __launch_bounds__(kDcThreads) dice_ce_bwd_kernel(DiceCeArgs A) {
                 if (p < HW) {
                     const float x = __ldg(xb + (size_t)c * HW + p);
                     const float mn = fmaxf(m[k], x);
-                    s[k] = s[k] * __expf(m[k] - mn) + __expf(x - mn);
+                    s[k] = s[k] * expf(m[k] - mn) + expf(x - mn);
                     m[k] = mn;
                     ts[k] += __ldg(tb + (size_t)c * HW + p);
                 }
@@ -141,8 +144,8 @@ __global__ void __launch_bounds__(kDcThreads) dice_ce_bwd_kernel(DiceCeArgs A) {
                 const int p = p0 + k * kDcThreads;
                 if (p < HW) {
                     const float x = __ldg(xb + (size_t)c * HW + p), t = __ldg(tb + (size_t)c * HW + p);
-                    const float sg = 1.f / (1.f + __expf(-x));
-                    const float soft = __expf(x - m[k]) / s[k];
+                    const float sg = 1.f / (1.f + expf(-x));
+                    const float soft = expf(x - m[k]) / s[k];
                     gb[(size_t)c * HW + p] = w_dice * (bb - a * t) * sg * (1.f - sg) + w_ce * (soft * ts[k] - t);
                 }
             }

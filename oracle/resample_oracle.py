@@ -69,11 +69,19 @@ def resample_backward(grad_out, x, apply_sigmoid: bool = False) -> np.ndarray:
 
 # ------------------------------------------------------------------ F3: SAM post-processing chain
 
-def _axis_half_pixel(n_in: int, n_out: int):
-    """ATen upsample_bilinear2d, align_corners=False: scale = in / out, src = max(0, scale (dst + .5) - .5)."""
+def _axis_half_pixel(n_in: int, n_out: int, fused: bool = False):
+    """ATen upsample_bilinear2d, align_corners=False: scale = in / out, src = max(0, scale (dst + .5) - .5).
+
+    ``fused``: round ``scale (dst + .5) - .5`` once, as a fused multiply-add.  nvcc contracts it so in the F3
+    kernels and in ATen's CUDA kernel; the two roundings of the default differ from it by one ulp of ``src`` at a
+    few positions when ``scale`` is not a power of two."""
     f32 = np.float32
     scale = f32(n_in) / f32(n_out)
-    src = (scale * (np.arange(n_out, dtype=np.float32) + f32(0.5)) - f32(0.5)).astype(np.float32)
+    half = np.arange(n_out, dtype=np.float32) + f32(0.5)
+    if fused:  # the float64 product of two fp32 values and the subtraction of .5 are exact here
+        src = (np.float64(scale) * half.astype(np.float64) - 0.5).astype(np.float32)
+    else:
+        src = (scale * half - f32(0.5)).astype(np.float32)
     src = np.maximum(src, f32(0)).astype(np.float32)
     i0 = src.astype(np.int64)
     i1 = i0 + (i0 < n_in - 1)
@@ -97,3 +105,24 @@ def interpolate_half_pixel(x, out_h: int, out_w: int) -> np.ndarray:
 def postprocess(x, T: int, rh: int, rw: int, oh: int, ow: int) -> np.ndarray:
     """training_utils.py:57-59: upsample to T x T, crop to [rh, rw], resample to [oh, ow]."""
     return interpolate_half_pixel(interpolate_half_pixel(x, T, T)[..., :rh, :rw], oh, ow)
+
+
+# ------------------------------------------------------------------ float64 references (dense weight matrices)
+# Bilinear resampling is separable and linear: along one axis it is an [n_out, n_in] matrix whose row o holds
+# the two tap weights of output o.  The taps and weights are ATen's float32 ones (_axis / _axis_half_pixel), so
+# the matrix is exactly the operation the fp32 kernels compute; only the products and sums are done in float64.
+# (Sampling positions computed in float64 would be a different operation: src moves by up to src * eps32.)
+
+def axis_matrix(n_in: int, n_out: int, align_corners: bool, fused: bool = False) -> np.ndarray:
+    """[n_out, n_in] float64 weights of one axis of F.interpolate(mode='bilinear') (``fused``: see _axis_half_pixel)."""
+    i0, i1, l0, l1 = _axis(n_in, n_out) if align_corners else _axis_half_pixel(n_in, n_out, fused)
+    m = np.zeros((n_out, n_in), dtype=np.float64)
+    r = np.arange(n_out)
+    np.add.at(m, (r, i0), l0.astype(np.float64))
+    np.add.at(m, (r, i1), l1.astype(np.float64))
+    return m
+
+
+def postprocess_axis_matrix(n_src: int, T: int, r: int, n_out: int, fused: bool = False) -> np.ndarray:
+    """[n_out, n_src] float64 weights of one axis of ``postprocess``: A2 . A1[:r] (up to T, crop to r, to n_out)."""
+    return axis_matrix(r, n_out, False, fused) @ axis_matrix(n_src, T, False, fused)[:r]

@@ -142,7 +142,8 @@ def test_postprocess_oracle_matches_pytorch_cpu(Hs, T, rh, rw, oh, ow):
                                                (32, 64, 64, 64, 700, 650, 2), (16, 64, 62, 64, 31, 32, 5)])
 def test_gpu_postprocess_matches_torch_and_oracle(Hs, T, rh, rw, oh, ow, n):
     """Forward against the oracle and torch's two-step chain on the GPU; backward against torch autograd
-    (the third case up-samples, so the backward's shared-memory window falls back to global atomics)."""
+    (the third case up-samples, so the backward takes the scatter kernel; every tile's source window still fits
+    in shared memory.  tests/test_fused_ops_edges.py reaches the global-atomic fallback and the other paths.)"""
     import dilabhelmholtzoct_b200 as tlb
     gen = torch.Generator(device="cuda").manual_seed(Hs + oh)
     x = 3.0 * torch.randn((n, Hs, Hs), device="cuda", generator=gen)
