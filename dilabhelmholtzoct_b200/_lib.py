@@ -11,7 +11,7 @@ _LIB = None
 
 c_fp = ctypes.c_void_p  # device pointers travel as integers
 TL_OK = 0
-ABI_VERSION = 3
+ABI_VERSION = 4
 OPT_FORCE_GLOBAL_KERNEL, OPT_PROFILE, OPT_NO_BINARY_PATH, OPT_WORST_CASE_WORKSPACE, OPT_NO_FUSED_MATCH, OPT_NO_FUSED_GRAD = 0, 1, 2, 3, 4, 5
 OPT_LIST_MODE = 6
 STATUS_BITS = {1: "pair arena exhausted (pass a larger state buffer: TL_ARENA_FACTOR / set_arena_factor)",
@@ -50,6 +50,12 @@ SIGNATURES = {
     "tl_dice_ce_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, c_fp]),
     "tl_dice_ce_backward": (ctypes.c_int, [c_fp, c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, c_fp]),
     "tl_wasserstein_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)]),
+    "tl_diagrams_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.POINTER(ctypes.c_size_t)]),
+    "tl_diagrams_compute": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
+    "tl_diagrams_gather": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp,
+                                          ctypes.c_longlong, c_fp, c_fp, c_fp]),
+    "tl_diagrams_backward": (ctypes.c_int, [c_fp] * 3 + [ctypes.c_longlong] + [ctypes.c_int] * 3 + [c_fp, c_fp]),
+    "tl_wasserstein_backward": (ctypes.c_int, [c_fp] * 4 + [ctypes.c_int, ctypes.c_float] + [c_fp] * 5),
 }
 
 

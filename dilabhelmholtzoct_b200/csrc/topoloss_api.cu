@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "diagram_kernel.cuh"
 #include "dice_ce_kernel.cuh"
 #include "mask_kernel.cuh"
 #include "match_kernel.cuh"
@@ -613,6 +614,41 @@ PairsLayout make_pairs_layout(int n_maps, int H, int W, int dim) {
     return P;
 }
 
+// The persistence launch for one set of maps, then the segmented sort into gudhi's emission order: the pairs of
+// map i are records ps.offs[0][i] .. + ps.counts[0][i] of the arena in `ws`
+int sorted_pairs(const float* maps, int n_maps, int H, int W, int dim, void* ws, const PairsLayout& P, cudaStream_t st,
+                 tl::PairStore* ps_out) {
+    void* scratch = static_cast<char*>(ws) + P.scratch_off;
+    const tl::PairStore ps = pair_store(ws, P.S, P.state_bytes, at<uint64_t>(scratch, P.L.skeys), 2.0f);
+    int rc = launch_ph(maps, nullptr, 1, n_maps, ps, P.L, H, W, dim, ws, scratch, st);
+    if (rc != TL_OK) return rc;
+    tl::SortArgs a;
+    a.ps = ps; a.n_sets = 1; a.n_maps = n_maps; a.cap = P.L.cap;
+    a.key_tmp = at<uint64_t>(scratch, P.L.key_tmp);
+    a.idx_a = at<uint32_t>(scratch, P.L.idx_a);
+    a.idx_b = at<uint32_t>(scratch, P.L.idx_b);
+    a.rec_tmp = at<tl::PairRec>(scratch, P.L.rec_tmp);
+    tl::seg_sort_kernel<<<n_maps < kSortSlots ? n_maps : kSortSlots, tl::kSortThreads, 0, st>>>(a);
+    TL_CUDA(cudaGetLastError());
+    *ps_out = ps;
+    return TL_OK;
+}
+
+// [rows][2] buffers are read and written as int2 / float2: they must be 8-byte aligned (a null pointer passes)
+inline bool misaligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7) != 0; }
+
+// argument checks shared by tl_diagrams_compute / tl_diagrams_gather; the packed offsets are int32
+int diagrams_args(int n_maps, int H, int W, int dim, const void* ws, size_t ws_bytes, PairsLayout* P) {
+    int rc = check_shape(n_maps, 1, H, W, dim);
+    if (rc != TL_OK) return rc;
+    if (!ws) return fail(TL_ERR_ARG, "null pointer");
+    *P = make_pairs_layout(n_maps, H, W, dim);
+    if (ws_bytes < P->total) return fail(TL_ERR_ARG, "workspace %zu < %zu bytes (tl_diagrams_workspace_bytes)", ws_bytes, P->total);
+    if ((P->state_bytes - P->S.fixed) / sizeof(tl::PairRec) > 0x7FFFFFFFull)
+        return fail(TL_ERR_ARG, "%d maps of %dx%d can hold more pairs than int32 offsets address", n_maps, H, W);
+    return TL_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -633,19 +669,89 @@ int tl_persistence_pairs(const float* maps, int n_maps, int H, int W, int dim, v
     const PairsLayout P = make_pairs_layout(n_maps, H, W, dim);
     if (ws_bytes < P.total) return fail(TL_ERR_WORKSPACE, "workspace %zu < %zu bytes", ws_bytes, P.total);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    void* scratch = static_cast<char*>(ws) + P.scratch_off;
-    const tl::PairStore ps = pair_store(ws, P.S, P.state_bytes, at<uint64_t>(scratch, P.L.skeys), 2.0f);
-    rc = launch_ph(maps, nullptr, 1, n_maps, ps, P.L, H, W, dim, ws, scratch, st);
+    tl::PairStore ps;
+    rc = sorted_pairs(maps, n_maps, H, W, dim, ws, P, st, &ps);
     if (rc != TL_OK) return rc;
-    tl::SortArgs a;
-    a.ps = ps; a.n_sets = 1; a.n_maps = n_maps; a.cap = P.L.cap;
-    a.key_tmp = at<uint64_t>(scratch, P.L.key_tmp);
-    a.idx_a = at<uint32_t>(scratch, P.L.idx_a);
-    a.idx_b = at<uint32_t>(scratch, P.L.idx_b);
-    a.rec_tmp = at<tl::PairRec>(scratch, P.L.rec_tmp);
-    tl::seg_sort_kernel<<<n_maps < kSortSlots ? n_maps : kSortSlots, tl::kSortThreads, 0, st>>>(a);
-    TL_CUDA(cudaGetLastError());
     export_pairs_kernel<<<n_maps < 1184 ? n_maps : 1184, 256, 0, st>>>(ps, n_maps, pairs, cap, counts);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+// ---- persistence diagrams as packed, differentiable tensors (tl_diagrams_*)
+
+int tl_diagrams_workspace_bytes(int n_maps, int H, int W, int dim, size_t* bytes) {
+    if (!bytes) return fail(TL_ERR_ARG, "bytes is null");
+    int rc = check_shape(n_maps, 1, H, W, dim);
+    if (rc != TL_OK) return rc;
+    *bytes = make_pairs_layout(n_maps, H, W, dim).total;
+    return TL_OK;
+}
+
+int tl_diagrams_compute(const float* maps, int n_maps, int H, int W, int dim, void* ws, size_t ws_bytes,
+                        int32_t* offsets, int32_t* status, void* stream) {
+    PairsLayout P;
+    int rc = diagrams_args(n_maps, H, W, dim, ws, ws_bytes, &P);
+    if (rc != TL_OK) return rc;
+    if (!maps || !offsets) return fail(TL_ERR_ARG, "null pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    tl::PairStore ps;
+    rc = sorted_pairs(maps, n_maps, H, W, dim, ws, P, st, &ps);
+    if (rc != TL_OK) return rc;
+    tl::diagram_offsets_kernel<<<1, tl::kScanThreads, 0, st>>>(ps.counts[0], n_maps, ps.status, offsets, status);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+int tl_diagrams_gather(const float* maps, int n_maps, int H, int W, int dim, const void* ws, size_t ws_bytes,
+                       const int32_t* offsets, const int32_t* host_offsets, long long P, int32_t* pairs, float* diagram,
+                       void* stream) {
+    PairsLayout L;
+    int rc = diagrams_args(n_maps, H, W, dim, ws, ws_bytes, &L);
+    if (rc != TL_OK) return rc;
+    if (!maps || !offsets || !host_offsets) return fail(TL_ERR_ARG, "null pointer");
+    if (P < 0 || (P > 0 && (!pairs || !diagram))) return fail(TL_ERR_ARG, "null output buffer for %lld pairs", P);
+    if (misaligned8(pairs) || misaligned8(diagram)) return fail(TL_ERR_ARG, "pairs and diagram must be 8-byte aligned");
+    if (host_offsets[0] != 0) return fail(TL_ERR_ARG, "offsets[0] = %d, not 0", host_offsets[0]);
+    for (int i = 0; i < n_maps; ++i)
+        if (host_offsets[i + 1] < host_offsets[i]) return fail(TL_ERR_ARG, "offsets decrease at map %d", i);
+    if ((long long)host_offsets[n_maps] != P) return fail(TL_ERR_ARG, "P = %lld disagrees with offsets[%d] = %d", P, n_maps, host_offsets[n_maps]);
+    if (P == 0) return TL_OK;
+    void* w = const_cast<void*>(ws);
+    const int grid = n_maps < 1184 ? n_maps : 1184;
+    tl::diagram_gather_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        at<tl::PairRec>(w, L.S.arena), at<uint32_t>(w, L.S.offs[0]), maps, (long long)H * W, n_maps, offsets,
+        reinterpret_cast<int2*>(pairs), reinterpret_cast<float2*>(diagram));
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+int tl_diagrams_backward(const int32_t* pairs, const int32_t* offsets, const float* grad_diagram, long long P,
+                         int n_maps, int H, int W, float* grad_maps, void* stream) {
+    if (n_maps <= 0 || H <= 0 || W <= 0 || (long long)H * W >= 0x7FFFFFF0LL) return fail(TL_ERR_ARG, "bad shape [%d,%d,%d]", n_maps, H, W);
+    if (P < 0 || !offsets || !grad_maps || (P > 0 && (!pairs || !grad_diagram))) return fail(TL_ERR_ARG, "null pointer");
+    if (misaligned8(pairs) || misaligned8(grad_diagram)) return fail(TL_ERR_ARG, "pairs and grad_diagram must be 8-byte aligned");
+    const int grid = n_maps < 1184 ? n_maps : 1184;
+    tl::diagram_backward_kernel<<<grid, 512, 0, static_cast<cudaStream_t>(stream)>>>(
+        reinterpret_cast<const int2*>(pairs), offsets, reinterpret_cast<const float2*>(grad_diagram), n_maps, H * W, grad_maps);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+int tl_wasserstein_backward(const float* D1, const int32_t* off1, const float* D2, const int32_t* off2, int n_diag,
+                            float q, const int32_t* match1, const float* grad_cost, float* grad_D1, float* grad_D2,
+                            void* stream) {
+    if (n_diag <= 0) return fail(TL_ERR_ARG, "n_diag must be positive, got %d", n_diag);
+    if (!D1 || !off1 || !D2 || !off2 || !match1 || !grad_cost) return fail(TL_ERR_ARG, "null pointer");
+    if (!(q > 0.f)) return fail(TL_ERR_ARG, "q must be positive");
+    if (misaligned8(D1) || misaligned8(D2) || misaligned8(grad_D1) || misaligned8(grad_D2))
+        return fail(TL_ERR_ARG, "D1, D2, grad_D1 and grad_D2 must be 8-byte aligned");
+    if (!grad_D1 && !grad_D2) return TL_OK;
+    tl::WassersteinBwdArgs a;
+    a.d1 = reinterpret_cast<const float2*>(D1); a.off1 = off1;
+    a.d2 = reinterpret_cast<const float2*>(D2); a.off2 = off2;
+    a.n_diag = n_diag; a.q = q; a.match1 = match1; a.grad_cost = grad_cost;
+    a.g1 = reinterpret_cast<float2*>(grad_D1); a.g2 = reinterpret_cast<float2*>(grad_D2);
+    tl::wasserstein_backward_kernel<<<n_diag < 1184 ? n_diag : 1184, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }

@@ -52,7 +52,7 @@ extern "C" {
 #define TL_ERR_WORKSPACE (-2) /* workspace too small */
 #define TL_ERR_CUDA (-3)      /* a CUDA runtime call failed; see tl_last_error() */
 
-#define TL_ABI_VERSION 3
+#define TL_ABI_VERSION 4
 
 /* ABI version of the loaded library (TL_ABI_VERSION it was built with). */
 int tl_version(void);
@@ -265,6 +265,46 @@ int tl_dice_ce_backward(const float* grad_loss, const float* logits, const float
 
 /* Bytes of workspace tl_wasserstein needs. */
 int tl_wasserstein_workspace_bytes(int n_diag, int max_rows1, int max_rows2, size_t* bytes);
+
+/*
+ * Persistence diagrams as building blocks (torch_topological's CubicalComplex._forward on n_maps HxW maps, homology
+ * dimension dim in {0, 1}), in two calls that share one workspace `ws` of tl_diagrams_workspace_bytes bytes:
+ *
+ * tl_diagrams_compute   the pipeline of tl_persistence_pairs (pairs of every map in gudhi's emission order, the
+ *                       essential H0 class last, paired with argmax), then offsets[n_maps + 1] (int32, device) = the
+ *                       exclusive scan of the per-map pair counts, and *status (int32, device, may be NULL) = the
+ *                       status word (TL_STATUS_*: a NaN map or an exhausted arena; its pairs are then incomplete).
+ * tl_diagrams_gather    after the host has read offsets[n_maps] and allocated P rows: map i's pairs go to rows
+ *                       offsets[i] .. offsets[i+1]-1 of  pairs[P][2] = (creator, destroyer) flat pixel indices  and
+ *                       diagram[P][2] = (maps[i][creator], maps[i][destroyer]), bit for bit.  `maps` and `ws` are
+ *                       those of the compute call; host_offsets is the host copy of `offsets` (checked against P).
+ *
+ * tl_diagrams_backward  grad_maps[n_maps][H*W], fully overwritten = scatter-add of grad_diagram[P][2] into the
+ *                       creator and destroyer pixels of each row (a pixel critical for several pairs adds them up).
+ *
+ * The [P][2] buffers (pairs, diagram, grad_diagram) are read and written as 8-byte pairs and must be 8-byte aligned.
+ * Every argument error, a workspace smaller than the query asks for and a misaligned buffer included, returns TL_ERR_ARG.
+ */
+int tl_diagrams_workspace_bytes(int n_maps, int H, int W, int dim, size_t* bytes);
+int tl_diagrams_compute(const float* maps, int n_maps, int H, int W, int dim, void* ws, size_t ws_bytes,
+                        int32_t* offsets, int32_t* status, void* stream);
+int tl_diagrams_gather(const float* maps, int n_maps, int H, int W, int dim, const void* ws, size_t ws_bytes,
+                       const int32_t* offsets, const int32_t* host_offsets, long long P, int32_t* pairs, float* diagram,
+                       void* stream);
+int tl_diagrams_backward(const int32_t* pairs, const int32_t* offsets, const float* grad_diagram, long long P,
+                         int n_maps, int H, int W, float* grad_maps, void* stream);
+
+/*
+ * Backward of tl_wasserstein: D1/off1, D2/off2 and match1 as tl_wasserstein took and wrote them, grad_cost[n_diag]
+ * (fp32) the upstream gradient of each cost.  grad_D1[P1][2] and grad_D2[P2][2] (either may be NULL: not computed)
+ * are fully overwritten with grad_cost[k] * d cost_k / d (birth, death): the gradient ot.emd2 -> pow(q) ->
+ * cdist(p=inf) / distance to the diagonal give with the optimal plan.  A D1 row matched to D2 row j gets the
+ * matched term and row j its negation; a row of either side matched to the diagonal gets the diagonal term.
+ * D1, D2, grad_D1 and grad_D2 must be 8-byte aligned (TL_ERR_ARG otherwise).
+ */
+int tl_wasserstein_backward(const float* D1, const int32_t* off1, const float* D2, const int32_t* off2, int n_diag,
+                            float q, const int32_t* match1, const float* grad_cost, float* grad_D1, float* grad_D2,
+                            void* stream);
 
 #ifdef __cplusplus
 }
