@@ -56,6 +56,12 @@ SIGNATURES = {
                                           ctypes.c_longlong, c_fp, c_fp, c_fp]),
     "tl_diagrams_backward": (ctypes.c_int, [c_fp] * 3 + [ctypes.c_longlong] + [ctypes.c_int] * 3 + [c_fp, c_fp]),
     "tl_wasserstein_backward": (ctypes.c_int, [c_fp] * 4 + [ctypes.c_int, ctypes.c_float] + [c_fp] * 5),
+    "tl_betti_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.POINTER(ctypes.c_size_t)]),
+    "tl_betti_compute": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp, c_fp]),
+    "tl_betti_gather": (ctypes.c_int, [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp] + [ctypes.c_longlong] * 3 +
+                        [c_fp] * 4),
+    "tl_betti_backward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_longlong, c_fp,
+                          ctypes.c_longlong, c_fp, ctypes.c_longlong] + [c_fp] * 4),
 }
 
 

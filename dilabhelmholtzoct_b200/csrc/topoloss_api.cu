@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "betti_kernel.cuh"
 #include "diagram_kernel.cuh"
 #include "dice_ce_kernel.cuh"
 #include "mask_kernel.cuh"
@@ -960,6 +961,156 @@ int tl_dice_ce_backward(const float* grad_loss, const float* logits, const float
     if (!grad_logits) return fail(TL_ERR_ARG, "null pointer");
     a.grad_loss = grad_loss; a.gx = grad_logits;
     tl::dice_ce_bwd_kernel<<<dice_ce_grid(a), tl::kDcThreads, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+}  // extern "C"
+
+// ---- Betti matching (tl_betti_*)
+namespace {
+
+constexpr int kBettiSlots = 148;  // CTAs of betti_kernel (one 1024-thread CTA per SM of a B200), each with its own tables
+
+// [header 256 | counts [3][n] | recoff [n] | record arena | per-slot merge trees | per-slot node / edge tables]
+//   header: [0] job counter (u32) | [8] arena head (u64) | [16] status (u32)
+struct BettiLayout {
+    size_t counts, recoff, arena, T, tabs, total;
+    size_t t_stride, n_stride, e_stride, tab_stride;
+    unsigned long long cap;
+    int slots;
+};
+BettiLayout make_betti_layout(int n_maps, int H, int W, int dim) {
+    BettiLayout B;
+    memset(&B, 0, sizeof(B));
+    size_t o = 256;
+    auto take = [&](size_t bytes) { size_t at = o; o = align_up(o + bytes); return at; };
+    B.counts = take(sizeof(int32_t) * 3 * (size_t)n_maps);
+    B.recoff = take(sizeof(uint32_t) * (size_t)n_maps);
+    // a map's records: every interval of the prediction (matched or not) and every unmatched one of the target
+    unsigned long long recs = (unsigned long long)n_maps * 2ull * (unsigned long long)max_pairs(H, W, dim);
+    if (!opt(TL_OPT_WORST_CASE_WORKSPACE) && recs > (1ull << 28)) recs = 1ull << 28;  // 4 GiB of records
+    if (recs > 0xFFFFFFFFull) recs = 0xFFFFFFFFull;
+    B.cap = recs;
+    B.arena = take(sizeof(int4) * (size_t)recs);
+    B.slots = n_maps < kBettiSlots ? n_maps : kBettiSlots;
+    const size_t nn = dim == 1 ? (size_t)H * W + 1 : (size_t)(H + 1) * (W + 1);
+    const size_t ne = (size_t)H * (W + 1) + (size_t)(H + 1) * W;
+    B.t_stride = align_up(sizeof(uint64_t) * nn) / sizeof(uint64_t);
+    B.T = take(sizeof(uint64_t) * B.t_stride * B.slots);
+    B.n_stride = align_up(sizeof(int32_t) * nn) / sizeof(int32_t);
+    B.e_stride = align_up(sizeof(int32_t) * ne) / sizeof(int32_t);
+    B.tab_stride = 6 * B.n_stride + 2 * B.e_stride;
+    B.tabs = take(sizeof(int32_t) * B.tab_stride * B.slots);
+    B.total = o;
+    return B;
+}
+
+int betti_args(int n_maps, int H, int W, int dim, const void* ws, size_t ws_bytes, BettiLayout* B) {
+    int rc = check_shape(n_maps, 1, H, W, dim);
+    if (rc != TL_OK) return rc;
+    if (!ws) return fail(TL_ERR_ARG, "null pointer");
+    *B = make_betti_layout(n_maps, H, W, dim);
+    if (ws_bytes < B->total) return fail(TL_ERR_ARG, "workspace %zu < %zu bytes (tl_betti_workspace_bytes)", ws_bytes, B->total);
+    if (B->cap > 0x7FFFFFFFull) return fail(TL_ERR_ARG, "%d maps of %dx%d can hold more records than int32 offsets address", n_maps, H, W);
+    return TL_OK;
+}
+
+// host copy of offsets [3][n_maps + 1]: each list starts at 0, never decreases and ends at its total
+int check_host_offsets(const int32_t* host, int n_maps, const long long* totals) {
+    static const char* what[3] = {"matched", "unmatched_pred", "unmatched_target"};
+    for (int k = 0; k < 3; ++k) {
+        const int32_t* h = host + (size_t)k * (n_maps + 1);
+        if (h[0] != 0) return fail(TL_ERR_ARG, "%s offsets[0] = %d, not 0", what[k], h[0]);
+        for (int i = 0; i < n_maps; ++i)
+            if (h[i + 1] < h[i]) return fail(TL_ERR_ARG, "%s offsets decrease at map %d", what[k], i);
+        if ((long long)h[n_maps] != totals[k]) return fail(TL_ERR_ARG, "%s count %lld disagrees with offsets[%d] = %d", what[k], totals[k], n_maps, h[n_maps]);
+    }
+    return TL_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tl_betti_workspace_bytes(int n_maps, int H, int W, int dim, size_t* bytes) {
+    if (!bytes) return fail(TL_ERR_ARG, "bytes is null");
+    int rc = check_shape(n_maps, 1, H, W, dim);
+    if (rc != TL_OK) return rc;
+    *bytes = make_betti_layout(n_maps, H, W, dim).total;
+    return TL_OK;
+}
+
+int tl_betti_compute(const float* pred, const float* target, int n_maps, int H, int W, int dim, void* ws, size_t ws_bytes,
+                     float* cost, int32_t* offsets, int32_t* status, void* stream) {
+    BettiLayout B;
+    int rc = betti_args(n_maps, H, W, dim, ws, ws_bytes, &B);
+    if (rc != TL_OK) return rc;
+    if (!pred || !target || !cost || !offsets) return fail(TL_ERR_ARG, "null pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    TL_CUDA(cudaMemsetAsync(ws, 0, 256, st));  // job counter, arena head, status
+    tl::BettiArgs a;
+    a.pred = pred; a.target = target; a.n_maps = n_maps; a.H = H; a.W = W;
+    a.job_counter = at<unsigned int>(ws, 0);
+    a.head = at<unsigned long long>(ws, 8);
+    a.cap = B.cap;
+    a.arena = at<int4>(ws, B.arena);
+    a.recoff = at<uint32_t>(ws, B.recoff);
+    a.counts = at<int32_t>(ws, B.counts);
+    a.cost = cost;
+    a.status = at<unsigned int>(ws, 16);
+    a.T = at<uint64_t>(ws, B.T); a.t_stride = B.t_stride;
+    a.tabs = at<int32_t>(ws, B.tabs); a.tab_stride = B.tab_stride; a.n_stride = B.n_stride; a.e_stride = B.e_stride;
+    if (dim == 1) tl::betti_kernel<1><<<B.slots, tl::kBmThreads, 0, st>>>(a);
+    else tl::betti_kernel<0><<<B.slots, tl::kBmThreads, 0, st>>>(a);
+    TL_CUDA(cudaGetLastError());
+    for (int k = 0; k < 3; ++k) {
+        tl::diagram_offsets_kernel<<<1, tl::kScanThreads, 0, st>>>(a.counts + (size_t)k * n_maps, n_maps, a.status,
+                                                                    offsets + (size_t)k * (n_maps + 1), k == 2 ? status : nullptr);
+        TL_CUDA(cudaGetLastError());
+    }
+    return TL_OK;
+}
+
+int tl_betti_gather(int n_maps, int H, int W, int dim, const void* ws, size_t ws_bytes, const int32_t* offsets,
+                    const int32_t* host_offsets, long long M, long long Kp, long long Kt, int32_t* matched,
+                    int32_t* unmatched_pred, int32_t* unmatched_target, void* stream) {
+    BettiLayout B;
+    int rc = betti_args(n_maps, H, W, dim, ws, ws_bytes, &B);
+    if (rc != TL_OK) return rc;
+    if (!offsets || !host_offsets) return fail(TL_ERR_ARG, "null pointer");
+    if (M < 0 || Kp < 0 || Kt < 0 || (M > 0 && !matched) || (Kp > 0 && !unmatched_pred) || (Kt > 0 && !unmatched_target))
+        return fail(TL_ERR_ARG, "null output buffer for %lld / %lld / %lld records", M, Kp, Kt);
+    if (misaligned8(matched) || misaligned8(unmatched_pred) || misaligned8(unmatched_target))
+        return fail(TL_ERR_ARG, "matched, unmatched_pred and unmatched_target must be 8-byte aligned");
+    const long long totals[3] = {M, Kp, Kt};
+    rc = check_host_offsets(host_offsets, n_maps, totals);
+    if (rc != TL_OK) return rc;
+    if (M + Kp + Kt == 0) return TL_OK;
+    void* w = const_cast<void*>(ws);
+    tl::betti_gather_kernel<<<n_maps < 1184 ? n_maps : 1184, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        at<int4>(w, B.arena), at<uint32_t>(w, B.recoff), n_maps, offsets, reinterpret_cast<int2*>(matched),
+        reinterpret_cast<int2*>(unmatched_pred), reinterpret_cast<int2*>(unmatched_target));
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+int tl_betti_backward(const float* pred, const float* target, int n_maps, int H, int W, const int32_t* offsets,
+                      const int32_t* matched, long long M, const int32_t* unmatched_pred, long long Kp,
+                      const int32_t* unmatched_target, long long Kt, const float* grad_cost, float* grad_pred,
+                      float* grad_target, void* stream) {
+    if (n_maps <= 0 || H <= 0 || W <= 0 || (long long)H * W >= 0x7FFFFFF0LL) return fail(TL_ERR_ARG, "bad shape [%d,%d,%d]", n_maps, H, W);
+    if (!pred || !target || !offsets || !grad_cost || !grad_pred) return fail(TL_ERR_ARG, "null pointer");
+    if (M < 0 || Kp < 0 || Kt < 0 || (M > 0 && !matched) || (Kp > 0 && !unmatched_pred) || (Kt > 0 && !unmatched_target))
+        return fail(TL_ERR_ARG, "null record buffer for %lld / %lld / %lld records", M, Kp, Kt);
+    if (misaligned8(matched) || misaligned8(unmatched_pred) || misaligned8(unmatched_target))
+        return fail(TL_ERR_ARG, "matched, unmatched_pred and unmatched_target must be 8-byte aligned");
+    tl::BettiBwdArgs a;
+    a.pred = pred; a.target = target; a.n_maps = n_maps; a.N = H * W; a.offsets = offsets;
+    a.matched = reinterpret_cast<const int2*>(matched);
+    a.up = reinterpret_cast<const int2*>(unmatched_pred); a.ut = reinterpret_cast<const int2*>(unmatched_target);
+    a.grad_cost = grad_cost; a.grad_pred = grad_pred; a.grad_target = grad_target;
+    tl::betti_backward_kernel<<<n_maps < 1184 ? n_maps : 1184, 512, 0, static_cast<cudaStream_t>(stream)>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }

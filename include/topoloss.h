@@ -306,6 +306,43 @@ int tl_wasserstein_backward(const float* D1, const int32_t* off1, const float* D
                             float q, const int32_t* match1, const float* grad_cost, float* grad_D1, float* grad_D2,
                             void* stream);
 
+/*
+ * Betti matching loss (Stucki et al., ICML 2023) of n_maps prediction / target pairs of HxW fp32 maps, homology
+ * dimension dim in {0, 1}, sublevel filtration of the T-construction (the complex and pixel rules of tl_diagrams_*,
+ * maps read as H rows of W pixels).  With C = min(pred, target): a prediction interval and a target interval are
+ * matched when the intervals of the images H_dim(pred_t) -> H_dim(C_t) and H_dim(target_t) -> H_dim(C_t) born at
+ * their birth cells die at the same cell of C; the two essential H0 classes (global minimum -> argmax) are always
+ * matched.  Per map, in fp64, returned as fp32:
+ *   cost = sum_matched (b_p - b_t)^2 + (d_p - d_t)^2 + sum_unmatched (d - b)^2 / 2.
+ * Three calls share one workspace `ws` of tl_betti_workspace_bytes bytes:
+ *
+ * tl_betti_compute   cost[n_maps] (fp32, device), offsets[3][n_maps + 1] (int32, device) = the exclusive scans of the
+ *                    per-map counts of matched, unmatched prediction and unmatched target intervals, and *status
+ *                    (int32, device, may be NULL) = the status word (TL_STATUS_*: a NaN map or an exhausted arena).
+ * tl_betti_gather    after the host has read the offsets (host_offsets: the same [3][n_maps + 1]; M, Kp, Kt their
+ *                    totals): packed pixel indices, map i's records at rows offsets[k][i] .. offsets[k][i+1]-1 of
+ *                    matched[M][4] = (pred creator, pred destroyer, target creator, target destroyer),
+ *                    unmatched_pred[Kp][2] and unmatched_target[Kt][2] = (creator, destroyer).  Order within a map:
+ *                    the node that owns an interval in the pixel graph (H0: birth vertex, H1: death pixel), raster
+ *                    order; the H0 essential pair is the map's last matched row.
+ * tl_betti_backward  grad_pred[n_maps][H*W] and, when not NULL, grad_target, fully overwritten with grad_cost[i] *
+ *                    d cost_i / d map, scattered into the critical pixels of the records (atomics: a pixel critical
+ *                    for several intervals adds them up).  pred / target are the maps of the compute call.
+ *
+ * The record buffers are read and written as 8-byte pairs and must be 8-byte aligned.  Every argument error, a
+ * workspace smaller than the query asks for and a misaligned buffer included, returns TL_ERR_ARG.
+ */
+int tl_betti_workspace_bytes(int n_maps, int H, int W, int dim, size_t* bytes);
+int tl_betti_compute(const float* pred, const float* target, int n_maps, int H, int W, int dim, void* ws, size_t ws_bytes,
+                     float* cost, int32_t* offsets, int32_t* status, void* stream);
+int tl_betti_gather(int n_maps, int H, int W, int dim, const void* ws, size_t ws_bytes, const int32_t* offsets,
+                    const int32_t* host_offsets, long long M, long long Kp, long long Kt, int32_t* matched,
+                    int32_t* unmatched_pred, int32_t* unmatched_target, void* stream);
+int tl_betti_backward(const float* pred, const float* target, int n_maps, int H, int W, const int32_t* offsets,
+                      const int32_t* matched, long long M, const int32_t* unmatched_pred, long long Kp,
+                      const int32_t* unmatched_target, long long Kt, const float* grad_cost, float* grad_pred,
+                      float* grad_target, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
