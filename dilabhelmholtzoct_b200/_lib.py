@@ -62,6 +62,10 @@ SIGNATURES = {
                         [c_fp] * 4),
     "tl_betti_backward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_longlong, c_fp,
                           ctypes.c_longlong, c_fp, ctypes.c_longlong] + [c_fp] * 4),
+    "tl_prior_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.POINTER(ctypes.c_size_t)] * 2),
+    "tl_prior_forward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, c_fp, ctypes.c_size_t, c_fp, ctypes.c_size_t,
+                                        c_fp, c_fp]),
+    "tl_prior_backward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
 }
 
 

@@ -18,6 +18,7 @@
 #include "match_kernel.cuh"
 #include "ph_kernel.cuh"
 #include "ph_small.cuh"
+#include "prior_kernel.cuh"
 #include "resample_kernel.cuh"
 #include "seg_sort.cuh"
 
@@ -616,12 +617,12 @@ PairsLayout make_pairs_layout(int n_maps, int H, int W, int dim) {
 }
 
 // The persistence launch for one set of maps, then the segmented sort into gudhi's emission order: the pairs of
-// map i are records ps.offs[0][i] .. + ps.counts[0][i] of the arena in `ws`
-int sorted_pairs(const float* maps, int n_maps, int H, int W, int dim, void* ws, const PairsLayout& P, cudaStream_t st,
-                 tl::PairStore* ps_out) {
-    void* scratch = static_cast<char*>(ws) + P.scratch_off;
-    const tl::PairStore ps = pair_store(ws, P.S, P.state_bytes, at<uint64_t>(scratch, P.L.skeys), 2.0f);
-    int rc = launch_ph(maps, nullptr, 1, n_maps, ps, P.L, H, W, dim, ws, scratch, st);
+// map i are records ps.offs[0][i] .. + ps.counts[0][i] of the arena in `state` (P.state_bytes of layout P.S);
+// `scratch` holds P.L (the persistence tables, the sort keys and the sort's buffers)
+int sorted_pairs(const float* maps, int n_maps, int H, int W, int dim, void* state, void* scratch, const PairsLayout& P,
+                 cudaStream_t st, tl::PairStore* ps_out) {
+    const tl::PairStore ps = pair_store(state, P.S, P.state_bytes, at<uint64_t>(scratch, P.L.skeys), 2.0f);
+    int rc = launch_ph(maps, nullptr, 1, n_maps, ps, P.L, H, W, dim, state, scratch, st);
     if (rc != TL_OK) return rc;
     tl::SortArgs a;
     a.ps = ps; a.n_sets = 1; a.n_maps = n_maps; a.cap = P.L.cap;
@@ -671,7 +672,7 @@ int tl_persistence_pairs(const float* maps, int n_maps, int H, int W, int dim, v
     if (ws_bytes < P.total) return fail(TL_ERR_WORKSPACE, "workspace %zu < %zu bytes", ws_bytes, P.total);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     tl::PairStore ps;
-    rc = sorted_pairs(maps, n_maps, H, W, dim, ws, P, st, &ps);
+    rc = sorted_pairs(maps, n_maps, H, W, dim, ws, static_cast<char*>(ws) + P.scratch_off, P, st, &ps);
     if (rc != TL_OK) return rc;
     export_pairs_kernel<<<n_maps < 1184 ? n_maps : 1184, 256, 0, st>>>(ps, n_maps, pairs, cap, counts);
     TL_CUDA(cudaGetLastError());
@@ -696,7 +697,7 @@ int tl_diagrams_compute(const float* maps, int n_maps, int H, int W, int dim, vo
     if (!maps || !offsets) return fail(TL_ERR_ARG, "null pointer");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     tl::PairStore ps;
-    rc = sorted_pairs(maps, n_maps, H, W, dim, ws, P, st, &ps);
+    rc = sorted_pairs(maps, n_maps, H, W, dim, ws, static_cast<char*>(ws) + P.scratch_off, P, st, &ps);
     if (rc != TL_OK) return rc;
     tl::diagram_offsets_kernel<<<1, tl::kScanThreads, 0, st>>>(ps.counts[0], n_maps, ps.status, offsets, status);
     TL_CUDA(cudaGetLastError());
@@ -1111,6 +1112,87 @@ int tl_betti_backward(const float* pred, const float* target, int n_maps, int H,
     a.up = reinterpret_cast<const int2*>(unmatched_pred); a.ut = reinterpret_cast<const int2*>(unmatched_target);
     a.grad_cost = grad_cost; a.grad_pred = grad_pred; a.grad_target = grad_target;
     tl::betti_backward_kernel<<<n_maps < 1184 ? n_maps : 1184, 512, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+}  // extern "C"
+
+// ---- topological prior (tl_prior_*)
+namespace {
+
+// STATE: the pairs layout's state part (header, bookkeeping, the sorted arena), then the per-map threshold keys;
+// SCRATCH: the pairs layout's scratch part (its sort-key array holds the records' p bits during the forward)
+struct PriorLayout { PairsLayout P; size_t thr, state_bytes, scratch_bytes; };
+PriorLayout make_prior_layout(int n_maps, int H, int W, int dim) {
+    PriorLayout R;
+    R.P = make_pairs_layout(n_maps, H, W, dim);
+    R.thr = R.P.state_bytes;  // 256-byte aligned
+    R.state_bytes = R.thr + align_up(sizeof(uint64_t) * (size_t)n_maps);
+    R.scratch_bytes = R.P.L.total;
+    return R;
+}
+
+int prior_args(int n_maps, int H, int W, int dim, const float* maps, const void* state, size_t state_bytes, PriorLayout* R) {
+    int rc = check_shape(n_maps, 1, H, W, dim);
+    if (rc != TL_OK) return rc;
+    if (!maps || !state) return fail(TL_ERR_ARG, "null pointer");
+    *R = make_prior_layout(n_maps, H, W, dim);
+    if (state_bytes < R->state_bytes) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_prior_workspace_bytes)", state_bytes, R->state_bytes);
+    return TL_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tl_prior_workspace_bytes(int n_maps, int H, int W, int dim, size_t* state_bytes, size_t* scratch_bytes) {
+    if (!state_bytes || !scratch_bytes) return fail(TL_ERR_ARG, "null pointer");
+    int rc = check_shape(n_maps, 1, H, W, dim);
+    if (rc != TL_OK) return rc;
+    const PriorLayout R = make_prior_layout(n_maps, H, W, dim);
+    *state_bytes = R.state_bytes;
+    *scratch_bytes = R.scratch_bytes;
+    return TL_OK;
+}
+
+int tl_prior_forward(const float* maps, int n_maps, int H, int W, int dim, const int32_t* betti, void* state,
+                     size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream) {
+    PriorLayout R;
+    int rc = prior_args(n_maps, H, W, dim, maps, state, state_bytes, &R);
+    if (rc != TL_OK) return rc;
+    if (!betti || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
+    if (scratch_bytes < R.scratch_bytes) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_prior_workspace_bytes)", scratch_bytes, R.scratch_bytes);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    tl::PairStore ps;
+    rc = sorted_pairs(maps, n_maps, H, W, dim, state, scratch, R.P, st, &ps);
+    if (rc != TL_OK) return rc;
+    tl::PriorArgs a;
+    a.arena = ps.arena; a.offs = ps.offs[0]; a.counts = ps.counts[0];
+    a.maps = maps; a.N = (long long)H * W; a.n_maps = n_maps;
+    a.betti = betti; a.status = ps.status;
+    a.pbits = reinterpret_cast<uint32_t*>(ps.skeys);  // the sort is done with its keys; half of each 8-byte slot is used
+    a.thr = at<uint64_t>(state, R.thr);
+    a.cost = cost;
+    tl::prior_cost_kernel<<<n_maps < 1184 ? n_maps : 1184, tl::kPriorThreads, 0, st>>>(a);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+int tl_prior_backward(const float* maps, int n_maps, int H, int W, int dim, const void* state, size_t state_bytes,
+                      const float* grad_cost, float* grad_maps, void* stream) {
+    PriorLayout R;
+    int rc = prior_args(n_maps, H, W, dim, maps, state, state_bytes, &R);
+    if (rc != TL_OK) return rc;
+    if (!grad_cost || !grad_maps) return fail(TL_ERR_ARG, "null pointer");
+    void* w = const_cast<void*>(state);
+    tl::PriorBwdArgs a;
+    a.arena = at<tl::PairRec>(w, R.P.S.arena); a.offs = at<uint32_t>(w, R.P.S.offs[0]); a.counts = at<int32_t>(w, R.P.S.counts[0]);
+    a.maps = maps; a.N = H * W; a.n_maps = n_maps;
+    a.thr = at<uint64_t>(w, R.thr);
+    a.status = at<unsigned int>(w, 16);
+    a.grad_cost = grad_cost; a.grad_maps = grad_maps;
+    tl::prior_backward_kernel<<<n_maps < 1184 ? n_maps : 1184, 512, 0, static_cast<cudaStream_t>(stream)>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }

@@ -45,11 +45,17 @@ def _buffers(B: int, C: int, H: int, W: int, feat_d: int, device) -> Tuple[torch
     ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
     _lib.check(_lib.lib().tl_workspace_bytes(B, C, H, W, feat_d, ctypes.byref(ns), ctypes.byref(nc)), "tl_workspace_bytes")
     state = torch.empty(int(ns.value * _ARENA_FACTOR), dtype=torch.uint8, device=device)
+    return state, _scratch(nc.value, device)
+
+
+def _scratch(nbytes: int, device) -> torch.Tensor:
+    """The cached scratch buffer of (device, current stream), grown to at least ``nbytes``: a scratch is only live
+    inside one call, and calls on one stream run one after the other."""
     key = (device.index, torch.cuda.current_stream(device).cuda_stream)
     scratch = _SCRATCH.get(key)
-    if scratch is None or scratch.numel() < nc.value:
-        scratch = _SCRATCH[key] = torch.empty(nc.value, dtype=torch.uint8, device=device)
-    return state, scratch
+    if scratch is None or scratch.numel() < nbytes:
+        scratch = _SCRATCH[key] = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    return scratch
 
 
 class _StatusRing:
@@ -61,9 +67,10 @@ class _StatusRing:
     def __init__(self):
         self.host = torch.zeros(self.SLOTS, dtype=torch.int32).pin_memory()
         self.events = [None] * self.SLOTS
+        self.ops = ["topo_loss"] * self.SLOTS  # the op whose status word each slot holds (named in the error)
         self.next = 0
 
-    def post(self, state: torch.Tensor, device) -> None:
+    def post(self, state: torch.Tensor, device, op: str = "topo_loss") -> None:
         i = self.next
         self.next = (i + 1) % self.SLOTS
         if self.events[i] is not None:
@@ -73,6 +80,7 @@ class _StatusRing:
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream(device))
         self.events[i] = ev
+        self.ops[i] = op
 
     def _raise_if_set(self, i: int) -> None:
         v = int(self.host[i])
@@ -80,7 +88,7 @@ class _StatusRing:
         self.host[i] = 0
         if v:
             why = "; ".join(msg for bit, msg in _lib.STATUS_BITS.items() if v & bit)
-            raise RuntimeError(f"topo_loss: an earlier call reported status {v}: {why} (its loss was NaN)")
+            raise RuntimeError(f"{self.ops[i]}: an earlier call reported status {v}: {why} (its loss was NaN)")
 
     def poll(self, sync: bool = False) -> None:
         for i, ev in enumerate(self.events):
@@ -101,8 +109,8 @@ def _status_ring(device) -> _StatusRing:
 
 
 def check_status(sync: bool = True) -> None:
-    """Raise if any earlier ``topo_loss`` call on this process reported a device-side problem
-    (``sync=True`` waits for the outstanding status copies first)."""
+    """Raise if any earlier ``topo_loss`` or ``topological_prior`` call on this process reported a device-side
+    problem (``sync=True`` waits for the outstanding status copies first)."""
     for ring in _STATUS.values():
         ring.poll(sync)
 

@@ -343,6 +343,35 @@ int tl_betti_backward(const float* pred, const float* target, int n_maps, int H,
                       const int32_t* unmatched_target, long long Kt, const float* grad_cost, float* grad_pred,
                       float* grad_target, void* stream);
 
+/*
+ * Topological prior loss (Clough et al., IPMI 2019 / TPAMI 2022) of n_maps HxW fp32 maps in homology dimension
+ * dim in {0, 1}: a cost per map that asks for betti[i] features and no more, with no ground-truth map.  D is the map's
+ * diagram as tl_diagrams_* computes it (same pairs, same order, the H0 essential class paired with argmax); per
+ * record p = |f[destroyer] - f[creator]| (fp32 subtraction, then fabsf, values read from the map); records are
+ * ranked by p descending, ties by position in D (earlier first: a stable descending sort).  In fp64, returned as fp32:
+ *   cost = sum_{rank < beta} (1 - p^2) + sum_{rank >= beta} p^2 + max(0, beta - |D|)
+ * (a missing interval counts as persistence 0: it adds 1 and no gradient).  The state keeps the sorted records and one
+ * threshold key per map for the backward; the scratch is only live inside the forward.
+ *
+ * tl_prior_workspace_bytes  *state_bytes and *scratch_bytes (host pointers).
+ * tl_prior_forward          betti[n_maps] (int32, device) -> cost[n_maps] (fp32, device): the persistence launch, the
+ *                           sort into gudhi's emission order and one select / cost kernel.  A status bit of the
+ *                           persistence launch (a NaN map, an exhausted arena) makes every cost of the call NaN; a
+ *                           negative betti[i] makes cost[i] NaN.  The status word is at byte 16 of the state.
+ * tl_prior_backward         grad_maps[n_maps][H*W], fully overwritten with grad_cost[i] * d cost_i / d map: for a
+ *                           selected record (rank < beta) d/d death = -2 (d - b) and d/d birth = +2 (d - b), otherwise
+ *                           the opposite signs, scatter-added into the critical pixels.  maps and state are those of the
+ *                           forward; a map whose cost was NaN gets NaN everywhere.
+ *
+ * Every argument error (null pointer, a buffer smaller than the query asks for, a bad shape or dim) returns TL_ERR_ARG
+ * before any launch.
+ */
+int tl_prior_workspace_bytes(int n_maps, int H, int W, int dim, size_t* state_bytes, size_t* scratch_bytes);
+int tl_prior_forward(const float* maps, int n_maps, int H, int W, int dim, const int32_t* betti, void* state,
+                     size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream);
+int tl_prior_backward(const float* maps, int n_maps, int H, int W, int dim, const void* state, size_t state_bytes,
+                      const float* grad_cost, float* grad_maps, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
