@@ -66,6 +66,12 @@ SIGNATURES = {
     "tl_prior_forward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, c_fp, ctypes.c_size_t, c_fp, ctypes.c_size_t,
                                         c_fp, c_fp]),
     "tl_prior_backward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
+    "tl_edt_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)]),
+    "tl_edt": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_hausdorff_dt_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)] * 2),
+    "tl_hausdorff_dt_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, c_fp, ctypes.c_size_t,
+                                               c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_hausdorff_dt_backward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
 }
 
 

@@ -14,6 +14,7 @@
 #include "betti_kernel.cuh"
 #include "diagram_kernel.cuh"
 #include "dice_ce_kernel.cuh"
+#include "edt_kernel.cuh"
 #include "mask_kernel.cuh"
 #include "match_kernel.cuh"
 #include "ph_kernel.cuh"
@@ -1193,6 +1194,118 @@ int tl_prior_backward(const float* maps, int n_maps, int H, int W, int dim, cons
     a.status = at<unsigned int>(w, 16);
     a.grad_cost = grad_cost; a.grad_maps = grad_maps;
     tl::prior_backward_kernel<<<n_maps < 1184 ? n_maps : 1184, 512, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+}  // extern "C"
+
+// ---- exact Euclidean distance transform (tl_edt) and the Hausdorff distance-transform loss (tl_hausdorff_dt_*)
+namespace {
+
+int edt_shape(int n_maps, int H, int W) {
+    if (n_maps <= 0 || H < 1 || W < 1 || H > tl::kEdtMaxDim || W > tl::kEdtMaxDim)
+        return fail(TL_ERR_ARG, "bad shape [%d,%d,%d] (n_maps > 0, H and W in [1, %d])", n_maps, H, W, tl::kEdtMaxDim);
+    return TL_OK;
+}
+
+// STATE: D = F(P)^alpha + F(T)^alpha, fp32 per pixel (the backward reads it); SCRATCH: the row pass's h0 / h1 of one
+// mask, a uint2 per pixel (P, then T)
+size_t edt_pixels(int n_maps, int H, int W) { return (size_t)n_maps * H * W; }
+
+int edt_grid(long long work, int per_block) {
+    const long long b = (work + per_block - 1) / per_block;
+    return (int)(b < (1ll << 20) ? b : (1ll << 20));
+}
+
+template <class Src, int NL>
+int edt_rows(Src src, int n_maps, int H, int W, uint32_t* h, cudaStream_t st) {
+    const long long rows = (long long)n_maps * H;
+    tl::edt_row_kernel<Src, NL><<<edt_grid(rows, tl::kEdtRowWarps), tl::kEdtRowWarps * 32, 0, st>>>(src, rows, W, h);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+template <int Mode>
+int edt_cols(const tl::EdtColArgs& a, cudaStream_t st) {
+    tl::edt_col_kernel<Mode><<<a.n_maps < (1 << 20) ? a.n_maps : (1 << 20), tl::kEdtColThreads, 0, st>>>(a);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tl_edt_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
+    if (!bytes) return fail(TL_ERR_ARG, "null pointer");
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    *bytes = align_up(sizeof(uint32_t) * edt_pixels(n_maps, H, W));
+    return TL_OK;
+}
+
+int tl_edt(const uint8_t* mask, int n_maps, int H, int W, void* ws, size_t ws_bytes, float* out, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!mask || !ws || !out) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(ws) & 3) return fail(TL_ERR_ARG, "workspace must be 4-byte aligned");
+    const size_t need = align_up(sizeof(uint32_t) * edt_pixels(n_maps, H, W));
+    if (ws_bytes < need) return fail(TL_ERR_ARG, "workspace %zu < %zu bytes (tl_edt_workspace_bytes)", ws_bytes, need);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint32_t* h = static_cast<uint32_t*>(ws);
+    rc = edt_rows<tl::EdtMaskSrc, 1>(tl::EdtMaskSrc{mask}, n_maps, H, W, h, st);
+    if (rc != TL_OK) return rc;
+    tl::EdtColArgs a = {};
+    a.h = h; a.n_maps = n_maps; a.H = H; a.W = W; a.field = out;
+    return edt_cols<tl::kEdtField>(a, st);
+}
+
+int tl_hausdorff_dt_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes) {
+    if (!state_bytes || !scratch_bytes) return fail(TL_ERR_ARG, "null pointer");
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    *state_bytes = align_up(sizeof(float) * edt_pixels(n_maps, H, W));
+    *scratch_bytes = align_up(sizeof(uint2) * edt_pixels(n_maps, H, W));
+    return TL_OK;
+}
+
+int tl_hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
+                            void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
+                            void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!logits || !target || !state || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
+    if (!(alpha > 0.0) || !(alpha < HUGE_VAL)) return fail(TL_ERR_ARG, "alpha must be finite and positive, got %g", alpha);
+    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
+        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
+    const size_t ns = align_up(sizeof(float) * edt_pixels(n_maps, H, W)), nc = align_up(sizeof(uint2) * edt_pixels(n_maps, H, W));
+    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", state_bytes, ns);
+    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", scratch_bytes, nc);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    tl::EdtColArgs a = {};
+    a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W;
+    a.sp = static_cast<int32_t*>(state); a.D = static_cast<float*>(state);
+    a.x = logits; a.t = target; a.half_alpha = 0.5 * alpha; a.cost = cost;
+    rc = edt_rows<tl::EdtLogitSrc, 2>(tl::EdtLogitSrc{logits}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtPred>(a, st);
+    if (rc == TL_OK) rc = edt_rows<tl::EdtTargetSrc, 2>(tl::EdtTargetSrc{target}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtTarget>(a, st);
+    return rc;
+}
+
+int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_maps, int H, int W, const void* state,
+                             size_t state_bytes, const float* grad_cost, float* grad_logits, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!logits || !target || !state || !grad_cost || !grad_logits) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(state) & 3) return fail(TL_ERR_ARG, "state must be 4-byte aligned");
+    const size_t ns = align_up(sizeof(float) * edt_pixels(n_maps, H, W));
+    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", state_bytes, ns);
+    const long long N = (long long)H * W;
+    tl::hausdorff_dt_backward_kernel<<<edt_grid((long long)n_maps * ((N + 1023) / 1024), 1), 256, 0,
+                                       static_cast<cudaStream_t>(stream)>>>(
+        logits, target, static_cast<const float*>(state), grad_cost, n_maps, N, grad_logits);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }

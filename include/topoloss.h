@@ -372,6 +372,43 @@ int tl_prior_forward(const float* maps, int n_maps, int H, int W, int dim, const
 int tl_prior_backward(const float* maps, int n_maps, int H, int W, int dim, const void* state, size_t state_bytes,
                       const float* grad_cost, float* grad_maps, void* stream);
 
+/*
+ * Exact Euclidean distance transform of n_maps HxW binary maps (H, W in [1, 4096]), unit spacing, pixel centres.
+ *
+ * tl_edt_workspace_bytes  *bytes (host pointer): the scratch tl_edt needs, 4 bytes per pixel.
+ * tl_edt                  mask[n_maps][H][W] (uint8, device; nonzero = feature) -> out[n_maps][H][W] (fp32, device):
+ *                         0 at a zero pixel; at a nonzero pixel float32(sqrt(float64(s))) with s the exact integer
+ *                         squared distance to the nearest zero pixel of the same map -- what
+ *                         scipy.ndimage.distance_transform_edt(m).astype(float32) gives, bit for bit, on a map with a
+ *                         zero pixel.  A map without a zero pixel gets +inf everywhere.  ws must be 4-byte aligned.
+ *
+ * Hausdorff distance-transform loss (Karimi & Salcudean, IEEE TMI 2020) of n_maps HxW maps of fp32 logits x and
+ * targets t.  Per map, p = sigmoid(x) (fp32, as torch.sigmoid), P = p > 0.5, T = t > 0.5, F(M) the distance of each
+ * pixel to the nearest pixel of the other label of M if M holds both labels and 0 otherwise, D = F(P)^alpha +
+ * F(T)^alpha (fp64), and
+ *   cost = (1 / HW) * sum_i (p_i - t_i)^2 * D_i      (fp64, fixed order, rounded to fp32)
+ *
+ * tl_hausdorff_dt_workspace_bytes  *state_bytes (D, 4 bytes per pixel: written by the forward, read by the backward)
+ *                                  and *scratch_bytes (8 bytes per pixel, only live inside the forward).
+ * tl_hausdorff_dt_forward          cost[n_maps] (fp32, device); alpha finite and > 0.  state 4-byte, scratch 8-byte
+ *                                  aligned.  A NaN logit makes its map's cost NaN.  The cost is bit-identical from
+ *                                  run to run.
+ * tl_hausdorff_dt_backward         grad_logits[n_maps][H][W], fully overwritten with
+ *                                  grad_cost[i] * (2 / HW) * (p - t) * D * p * (1 - p); logits, target and state are
+ *                                  those of the forward; state 4-byte aligned.
+ *
+ * Every argument error (null pointer, H or W out of range, a non-finite or non-positive alpha, a buffer smaller than
+ * the query asks for or misaligned) returns TL_ERR_ARG before any launch.
+ */
+int tl_edt_workspace_bytes(int n_maps, int H, int W, size_t* bytes);
+int tl_edt(const uint8_t* mask, int n_maps, int H, int W, void* ws, size_t ws_bytes, float* out, void* stream);
+int tl_hausdorff_dt_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes);
+int tl_hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
+                            void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
+                            void* stream);
+int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_maps, int H, int W, const void* state,
+                             size_t state_bytes, const float* grad_cost, float* grad_logits, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
