@@ -39,26 +39,6 @@ struct PriorArgs {
 
 __device__ __forceinline__ float prior_diff(const float* f, const PairRec& r) { return __ldg(f + r.des) - __ldg(f + r.cre); }
 
-// The digit of the k-th largest (1-based) among the 256 bins of s_hist, scanning from digit 255 down.  Warp 0 only;
-// lane l owns digits 255 - 8l .. 248 - 8l.  Writes the digit and k minus the count of larger digits.
-__device__ __forceinline__ void prior_pick_digit(const uint32_t* s_hist, uint32_t k, uint32_t* s_digit, uint32_t* s_k) {
-    const int lane = threadIdx.x & 31;
-    uint32_t c[8], sum = 0;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { c[j] = s_hist[255 - 8 * lane - j]; sum += c[j]; }
-    uint32_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, incl, o); if (lane >= o) incl += t; }
-    uint32_t run = incl - sum;
-    if (run < k && k <= incl) {  // exactly one lane
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            if (run + c[j] >= k) { *s_digit = (uint32_t)(255 - 8 * lane - j); *s_k = k - run; break; }
-            run += c[j];
-        }
-    }
-}
-
 __global__ void __launch_bounds__(kPriorThreads) prior_cost_kernel(PriorArgs A) {
     __shared__ uint32_t s_hist[256];
     __shared__ uint32_t s_digit, s_k, s_idx;
@@ -84,29 +64,10 @@ __global__ void __launch_bounds__(kPriorThreads) prior_cost_kernel(PriorArgs A) 
             thr = 0ull;  // every record
         } else {
             __syncthreads();  // pb is complete
-            // 1. radix select of the beta-th largest p bits, 8 bits per pass from the top; prefix / k are uniform
-            uint32_t prefix = 0u, k = (uint32_t)beta;
-            for (int shift = 24; shift >= 0; shift -= 8) {
-                for (int i = tid; i < 256; i += kPriorThreads) s_hist[i] = 0u;
-                __syncthreads();
-                const uint32_t hi_mask = shift == 24 ? 0u : ~0u << (shift + 8);
-                for (int i0 = 0; i0 < n; i0 += kPriorThreads) {  // uniform trip count: the whole warp reaches the match
-                    const int i = i0 + tid;
-                    uint32_t d = 256u + (uint32_t)lane;  // distinct dummy digit for lanes without a candidate
-                    if (i < n) {
-                        const uint32_t v = pb[i];
-                        if ((v & hi_mask) == prefix) d = (v >> shift) & 255u;
-                    }
-                    const unsigned peers = __match_any_sync(0xFFFFFFFFu, d);
-                    if (d < 256u && (peers & lanemask_lt()) == 0u) atomicAdd(&s_hist[d], (uint32_t)__popc(peers));
-                }
-                __syncthreads();
-                if (warp == 0) prior_pick_digit(s_hist, k, &s_digit, &s_k);
-                __syncthreads();
-                prefix |= s_digit << shift;
-                k = s_k;
-                __syncthreads();  // s_hist / s_digit / s_k are rewritten by the next pass
-            }
+            // 1. radix select of the beta-th largest p bits; prefix / k are uniform
+            const RadixPick pick = block_radix_select<kPriorThreads>([&](int i) { return pb[i]; }, n, (uint32_t)beta,
+                                                                     s_hist, &s_digit, &s_k);
+            const uint32_t prefix = pick.value, k = pick.k;
             // 2. among the records with p bits == prefix, the k-th in position order is the last one selected
             if (tid == 0) s_idx = 0xFFFFFFFFu;
             uint32_t run = 0u;

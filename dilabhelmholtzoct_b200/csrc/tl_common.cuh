@@ -134,6 +134,66 @@ __device__ __forceinline__ unsigned lanemask_lt() {
     return m;
 }
 
+// The digit of the k-th largest (1-based) among the 256 bins of s_hist, scanning from digit 255 down.  Warp 0 only;
+// lane l owns digits 255 - 8l .. 248 - 8l.  Writes the digit and k minus the count of larger digits.
+__device__ __forceinline__ void radix_pick_digit(const uint32_t* s_hist, uint32_t k, uint32_t* s_digit, uint32_t* s_k) {
+    const int lane = threadIdx.x & 31;
+    uint32_t c[8], sum = 0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { c[j] = s_hist[255 - 8 * lane - j]; sum += c[j]; }
+    uint32_t incl = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, incl, o); if (lane >= o) incl += t; }
+    uint32_t run = incl - sum;
+    if (run < k && k <= incl) {  // exactly one lane
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            if (run + c[j] >= k) { *s_digit = (uint32_t)(255 - 8 * lane - j); *s_k = k - run; break; }
+            run += c[j];
+        }
+    }
+}
+
+struct RadixPick {
+    uint32_t value;  // the k-th largest value
+    uint32_t k;      // its rank (1-based) among the values equal to it
+    uint32_t count;  // how many values equal it
+};
+
+// Exact block-wide radix select of the k-th largest (1 <= k <= n) of the n words key(0) .. key(n - 1), 8 bits per pass
+// from the top.  Every thread of a kThreads-thread block calls it with the same n and k; the trip counts are uniform,
+// so whole warps reach __match_any_sync.  s_hist is 256 words of shared memory, s_digit and s_k one word each; the
+// last barrier leaves them free for the caller.  For the k-th smallest, select over ~key.
+template <int kThreads, class Key>
+__device__ __forceinline__ RadixPick block_radix_select(const Key& key, int n, uint32_t k, uint32_t* s_hist,
+                                                        uint32_t* s_digit, uint32_t* s_k) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    uint32_t prefix = 0u, count = 0u;
+    for (int shift = 24; shift >= 0; shift -= 8) {
+        for (int i = tid; i < 256; i += kThreads) s_hist[i] = 0u;
+        __syncthreads();
+        const uint32_t hi_mask = shift == 24 ? 0u : ~0u << (shift + 8);
+        for (int i0 = 0; i0 < n; i0 += kThreads) {
+            const int i = i0 + tid;
+            uint32_t d = 256u + (uint32_t)lane;  // distinct dummy digit for lanes without a candidate
+            if (i < n) {
+                const uint32_t v = key(i);
+                if ((v & hi_mask) == prefix) d = (v >> shift) & 255u;
+            }
+            const unsigned peers = __match_any_sync(0xFFFFFFFFu, d);
+            if (d < 256u && (peers & lanemask_lt()) == 0u) atomicAdd(&s_hist[d], (uint32_t)__popc(peers));
+        }
+        __syncthreads();
+        if ((tid >> 5) == 0) radix_pick_digit(s_hist, k, s_digit, s_k);
+        __syncthreads();
+        prefix |= *s_digit << shift;
+        k = *s_k;
+        count = s_hist[*s_digit];
+        __syncthreads();  // s_hist / s_digit / s_k are rewritten by the next pass or the caller
+    }
+    return RadixPick{prefix, k, count};
+}
+
 // Exact n / d for n < 2^24, d <= 8193 via multiply-shift (magic = ceil(2^40 / d)); avoids the
 // ~30-instruction integer division in the per-node / per-edge loops.
 struct FastDiv {

@@ -22,6 +22,7 @@
 #include "prior_kernel.cuh"
 #include "resample_kernel.cuh"
 #include "seg_sort.cuh"
+#include "surface_kernel.cuh"
 
 namespace {
 
@@ -1306,6 +1307,66 @@ int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_map
     tl::hausdorff_dt_backward_kernel<<<edt_grid((long long)n_maps * ((N + 1023) / 1024), 1), 256, 0,
                                        static_cast<cudaStream_t>(stream)>>>(
         logits, target, static_cast<const float*>(state), grad_cost, n_maps, N, grad_logits);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+}  // extern "C"
+
+// ---- surface-distance metrics (tl_surface_*)
+namespace {
+
+// the row pass's h of both surfaces, then the keys of both directions (uint32 per pixel each), then [4][n] stats
+struct SurfLayout {
+    size_t keys, stats, total;
+};
+
+SurfLayout surface_layout(int n_maps, int H, int W) {
+    SurfLayout L;
+    const size_t px = edt_pixels(n_maps, H, W);
+    L.keys = align_up(sizeof(uint32_t) * 2 * px);
+    L.stats = L.keys + align_up(sizeof(uint32_t) * 2 * px);
+    L.total = L.stats + align_up(sizeof(uint32_t) * 4 * (size_t)n_maps);
+    return L;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
+    if (!bytes) return fail(TL_ERR_ARG, "null pointer");
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    *bytes = surface_layout(n_maps, H, W).total;
+    return TL_OK;
+}
+
+int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
+                         double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!pred || !target || !ws || !out) return fail(TL_ERR_ARG, "null pointer");
+    if (!(percentile >= 0.0 && percentile <= 100.0)) return fail(TL_ERR_ARG, "percentile must be in [0, 100], got %g", percentile);
+    if (!(tolerance >= 0.0 && tolerance < HUGE_VAL)) return fail(TL_ERR_ARG, "tolerance must be finite and >= 0, got %g", tolerance);
+    if (reinterpret_cast<uintptr_t>(ws) & 3) return fail(TL_ERR_ARG, "workspace must be 4-byte aligned");
+    const SurfLayout L = surface_layout(n_maps, H, W);
+    if (ws_bytes < L.total) return fail(TL_ERR_ARG, "workspace %zu < %zu bytes (tl_surface_workspace_bytes)", ws_bytes, L.total);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    char* base = static_cast<char*>(ws);
+    tl::SurfArgs a = {};
+    a.h = reinterpret_cast<uint32_t*>(base);
+    a.keys = reinterpret_cast<uint32_t*>(base + L.keys);
+    a.stats = reinterpret_cast<uint32_t*>(base + L.stats);
+    a.n_maps = n_maps; a.H = H; a.W = W;
+    a.tol = tolerance; a.qq = percentile / 100.0; a.out = out;
+    rc = edt_rows<tl::SurfSrc, 1>(tl::SurfSrc{pred, H, W}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_rows<tl::SurfSrc, 1>(tl::SurfSrc{target, H, W}, n_maps, H, W, a.h + edt_pixels(n_maps, H, W), st);
+    if (rc != TL_OK) return rc;
+    const int grid = n_maps < (1 << 20) ? n_maps : (1 << 20);
+    tl::surface_col_kernel<<<grid, tl::kEdtColThreads, 0, st>>>(a);
+    TL_CUDA(cudaGetLastError());
+    tl::surface_select_kernel<<<grid, tl::kSurfSelThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }

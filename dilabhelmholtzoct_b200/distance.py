@@ -4,7 +4,9 @@
 uint8 CUDA tensor (``tl_edt``).  ``hausdorff_dt_loss(masks, gt_masks, alpha)`` is the Hausdorff distance-transform
 loss of Karimi & Salcudean (IEEE TMI 2020) per ``(b, c)`` map of decoder logits, differentiable with respect to the
 logits (``tl_hausdorff_dt_*``).  Both transforms of each map (prediction and target, foreground and background) run
-in the same kernels as the loss; nothing goes through the host.
+in the same kernels as the loss; nothing goes through the host.  ``surface_distances(pred, target)`` gives the
+boundary metrics of mask pairs -- Hausdorff distance, percentile Hausdorff distance, ASSD and normalized surface Dice
+-- from the same transform measured at surface pixels (``tl_surface_distances``).
 
 There is no CPU path: the inputs must be CUDA tensors.
 """
@@ -12,6 +14,7 @@ from __future__ import annotations
 
 import ctypes
 import math
+from typing import NamedTuple
 
 import torch
 from torch.autograd.function import once_differentiable
@@ -25,6 +28,77 @@ MAX_DIM = 4096
 def _check_hw(H: int, W: int, what: str) -> None:
     if not (1 <= H <= MAX_DIM and 1 <= W <= MAX_DIM):
         raise ValueError(f"{what}: H and W must each be in [1, {MAX_DIM}], got {H} x {W}")
+
+
+class SurfaceDistances(NamedTuple):
+    """Per-map surface-distance metrics of ``surface_distances``: float32, shape ``pred.shape[:-2]``."""
+    hausdorff: torch.Tensor
+    hausdorff_percentile: torch.Tensor
+    assd: torch.Tensor
+    nsd: torch.Tensor
+
+
+def surface_distances(pred: torch.Tensor, target: torch.Tensor, percentile: float = 95.0,
+                      tolerance: float = 1.0) -> SurfaceDistances:
+    """Boundary metrics of every ``[H, W]`` map pair of ``pred`` and ``target`` (``[..., H, W]``, same shape, bool or
+    uint8, CUDA; a nonzero pixel is foreground): the Hausdorff distance, its ``percentile``-th percentile (HD95 by
+    default), the average symmetric surface distance and the normalized surface Dice at ``tolerance`` pixels.  No
+    autograd, no host synchronisation.
+
+    Per map, the surface ``S(M) = M & ~scipy.ndimage.binary_erosion(M)`` (cross structure, outside = 0) is the
+    foreground pixels with a background or outside 4-neighbour.  ``d_pt`` is the exact Euclidean distance (unit
+    spacing) from each pixel of ``S(pred)`` to the nearest pixel of ``S(target)``, ``sqrt(float64(s))`` of an integer
+    ``s``; ``d_tp`` the same the other way.  In fp64, rounded to float32::
+
+        hausdorff            = max(max d_pt, max d_tp)
+        hausdorff_percentile = max(np.percentile(d_pt, q), np.percentile(d_tp, q))      # numpy's linear method
+        assd                 = (sum d_pt + sum d_tp) / (|S(pred)| + |S(target)|)
+        nsd                  = (#{d_pt <= tolerance} + #{d_tp <= tolerance}) / (|S(pred)| + |S(target)|)
+
+    ``hausdorff``, ``hausdorff_percentile`` and ``nsd`` equal that numpy / scipy computation in float64 rounded to
+    float32 bit for bit; ``assd`` sums in another order and is within one float32 ulp of it.  Both masks empty: all
+    four are NaN (an all-zero padded mask pair; reduce with ``nanmean``).  One mask empty: ``hausdorff``,
+    ``hausdorff_percentile`` and ``assd`` are ``+inf`` and ``nsd`` is 0.  By recollection this is monai's
+    ``get_mask_edges`` with ``compute_hausdorff_distance``, ``compute_average_surface_distance(symmetric=True)`` and
+    ``compute_surface_dice``; monai is not a dependency, so that parity is unpinned.
+
+    ``percentile`` is in [0, 100], ``tolerance`` finite and >= 0, H and W each in [1, 4096].  About 16 bytes per pixel
+    of scratch are taken from PyTorch's caching allocator for the duration of the call."""
+    if not (torch.is_tensor(pred) and torch.is_tensor(target)):
+        raise TypeError("pred and target must be tensors")
+    if pred.dim() < 2 or pred.shape != target.shape:
+        raise ValueError(f"expected two [..., H, W] tensors of the same shape, got {tuple(pred.shape)} and "
+                         f"{tuple(target.shape)}")
+    if not pred.is_cuda or not target.is_cuda:
+        raise ValueError("surface_distances runs on a CUDA device only: there is no CPU fallback")
+    if pred.device != target.device:
+        raise ValueError(f"pred is on {pred.device}, target on {target.device}")
+    for name, m in (("pred", pred), ("target", target)):
+        if m.dtype not in (torch.bool, torch.uint8):
+            raise ValueError(f"surface_distances expects a bool or uint8 {name}, got {m.dtype}")
+    percentile, tolerance = float(percentile), float(tolerance)
+    if not 0.0 <= percentile <= 100.0:
+        raise ValueError(f"percentile must be in [0, 100], got {percentile}")
+    if not (math.isfinite(tolerance) and tolerance >= 0.0):
+        raise ValueError(f"tolerance must be finite and >= 0, got {tolerance}")
+    H, W = int(pred.shape[-2]), int(pred.shape[-1])
+    _check_hw(H, W, "surface_distances")
+    n = pred.numel() // (H * W)
+    dev = pred.device
+    out = torch.empty((4, n), dtype=torch.float32, device=dev)
+    if n > 0:
+        p, t = (m.detach().contiguous() for m in (pred, target))
+        p, t = (m.view(torch.uint8) if m.dtype == torch.bool else m for m in (p, t))
+        L = _lib.lib()
+        nb = ctypes.c_size_t(0)
+        _lib.check(L.tl_surface_workspace_bytes(n, H, W, ctypes.byref(nb)), "tl_surface_workspace_bytes")
+        with torch.cuda.device(dev):
+            ws = torch.empty(nb.value, dtype=torch.uint8, device=dev)  # per call: released to the caching allocator
+            rc = L.tl_surface_distances(p.data_ptr(), t.data_ptr(), n, H, W, percentile, tolerance, ws.data_ptr(),
+                                        ws.numel(), out.data_ptr(), _stream_ptr(dev))
+        _lib.check(rc, "tl_surface_distances")
+    lead = pred.shape[:-2]
+    return SurfaceDistances(*(o.view(lead) for o in out))
 
 
 def distance_transform_edt(mask: torch.Tensor) -> torch.Tensor:

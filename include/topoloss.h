@@ -409,6 +409,30 @@ int tl_hausdorff_dt_forward(const float* logits, const float* target, int n_maps
 int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_maps, int H, int W, const void* state,
                              size_t state_bytes, const float* grad_cost, float* grad_logits, void* stream);
 
+/*
+ * Surface-distance metrics of n_maps pairs of HxW binary maps (H, W in [1, 4096]), unit spacing, pixel centres.
+ * Per map: the surface S(M) = M & ~binary_erosion(M) (cross structure, outside = 0) -- the nonzero pixels with a zero
+ * or an outside 4-neighbour; d_pt the exact distance sqrt(float64(s)) from each pixel of S(pred) to the nearest pixel
+ * of S(target), d_tp the same the other way; n_p = |S(pred)|, n_t = |S(target)|.  Computed in fp64, rounded to fp32:
+ *   hausdorff             max(max d_pt, max d_tp)
+ *   hausdorff_percentile  max(pct(d_pt, q), pct(d_tp, q)), pct numpy's default (linear) percentile, q = percentile
+ *   assd                  (sum d_pt + sum d_tp) / (n_p + n_t)
+ *   nsd                   (#{d_pt <= tolerance} + #{d_tp <= tolerance}) / (n_p + n_t)
+ * Both surfaces empty: all four NaN.  One empty: hausdorff, hausdorff_percentile and assd +inf, nsd 0.
+ *
+ * tl_surface_workspace_bytes  *bytes (host pointer): the scratch tl_surface_distances needs, about 16 bytes per pixel.
+ * tl_surface_distances        pred, target [n_maps][H][W] (uint8, device; nonzero = foreground) -> out[4][n_maps]
+ *                             (fp32, device): hausdorff, hausdorff_percentile, assd, nsd.  percentile in [0, 100],
+ *                             tolerance finite and >= 0; ws 4-byte aligned.  Four launches, no host synchronisation,
+ *                             bit-identical from run to run.
+ *
+ * Every argument error (null pointer, H or W out of range, a percentile outside [0, 100] or NaN, a negative or
+ * non-finite tolerance, a workspace smaller than the query asks for or misaligned) returns TL_ERR_ARG before any launch.
+ */
+int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes);
+int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
+                         double tolerance, void* ws, size_t ws_bytes, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
