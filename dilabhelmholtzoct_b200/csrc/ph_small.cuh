@@ -1654,6 +1654,8 @@ __global__ void __launch_bounds__(kPhThreads, 1) ph_small_kernel(const __grid_co
             unsigned long long tj = 0ull;
             if (S.prof && tid == 0) tj = now_ns();
             if (kind == 1) {
+                // this launch's dynamic shared memory is match_one_map's kColCache-point column cache
+                static_assert(kSmallSmemBytes >= kColCache * sizeof(float2), "the column cache must fit the tail's shared memory");
                 const bool heavy = match_one_map(S.mf, k, reinterpret_cast<float2*>(smem));
                 if (S.fuse_grad && tid == 0) map_matched(k, heavy);  // thread 0 wrote the map's cost and matched points itself
             } else {
