@@ -75,6 +75,11 @@ SIGNATURES = {
     "tl_surface_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)]),
     "tl_surface_distances": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, ctypes.c_double, c_fp,
                                             ctypes.c_size_t, c_fp, c_fp]),
+    "tl_edt_spaced": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_hausdorff_dt_forward_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, c_fp, c_fp,
+                                                      ctypes.c_size_t, c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_surface_distances_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_double,
+                                                   ctypes.c_double, c_fp, ctypes.c_size_t, c_fp, c_fp]),
 }
 
 

@@ -12,7 +12,13 @@
 //
 // Every quantity of the envelope is an integer below 2^26 (H, W <= 4096: s <= 2 * 4095^2), so int32 holds all of it
 // and no float enters before the final root.  Entry point checks keep H and W in [1, 4096].
+//
+// With a physical pixel spacing (sy, sx) per map (tl_*_spaced, DESIGN §3.10) the row pass is the same, and the column
+// pass builds the weighted envelope (EdtEnvW / EdtWalkW) instead: row i's parabola is the fp64 value
+// s(u) = (float64(u - i) * sy)^2 + (float64(h_i) * sx)^2, each operation rounded, and the walk yields the offset
+// (|u - v|, h) of the nearest pixel, packed in 24 bits (edt_pack), from which s is recomputed where it is needed.
 #pragma once
+#include <type_traits>
 #include "tl_common.cuh"
 
 namespace tl {
@@ -169,11 +175,125 @@ struct EdtWalk {
     }
 };
 
+// ---- the weighted envelope (physical spacing)
+
+struct EdtSpacing {
+    double sy, sx;  // size of a pixel along rows (dim -2) and along columns (dim -1)
+};
+
+// float64(d) * sp, squared, each operation rounded to fp64 (no contraction)
+__device__ __forceinline__ double edt_sq1(int d, double sp) {
+    const double a = __dmul_rn((double)d, sp);
+    return __dmul_rn(a, a);
+}
+// the squared distance of offset (dy, dx) as scipy's distance_transform_edt(sampling=...) evaluates it
+__device__ __forceinline__ double edt_sq(int dy, int dx, const EdtSpacing& sp) {
+    return __dadd_rn(edt_sq1(dy, sp.sy), edt_sq1(dx, sp.sx));
+}
+// offsets below 4096 each, packed in 24 bits; 0 exactly at offset (0, 0)
+__device__ __forceinline__ uint32_t edt_pack(int dy, int dx) { return (uint32_t)dy | ((uint32_t)dx << 12); }
+__device__ __forceinline__ double edt_packed_sq(uint32_t p, const EdtSpacing& sp) {
+    return edt_sq((int)(p & 0xFFFu), (int)(p >> 12), sp);
+}
+
+// a1 + b1 <= a2 + b2 for doubles, exactly as real numbers: a rounded sum orders the reals (round to nearest is
+// monotone), and on equal rounded sums the exact rounding errors (TwoSum) decide
+__device__ __forceinline__ double edt_two_sum_err(double a, double b, double s) {
+    const double t = __dsub_rn(s, a);
+    return __dadd_rn(__dsub_rn(a, __dsub_rn(s, t)), __dsub_rn(b, t));
+}
+__device__ __forceinline__ bool edt_sum_le(double a1, double b1, double a2, double b2) {
+    const double s1 = __dadd_rn(a1, b1), s2 = __dadd_rn(a2, b2);
+    if (s1 != s2) return s1 < s2;
+    return edt_two_sum_err(a1, b1, s1) <= edt_two_sum_err(a2, b2, s2);
+}
+
+// Row i (horizontal term bi = edt_sq1(hi, sx)) is <= row v (bv) at u, in the exact sums of the rounded terms.  For
+// i > v the set of u where this holds is a suffix of [0, H) (DESIGN §3.10)
+__device__ __forceinline__ bool edt_beats(int i, double bi, int v, double bv, int u, double sy) {
+    return edt_sum_le(edt_sq1(abs(u - i), sy), bi, edt_sq1(abs(u - v), sy), bv);
+}
+
+// The first u in [0, H] at which row i > v beats row v (H: none): the crossing of the exact parabolas as an fp64
+// estimate, then corrected by the exact predicate, which is monotone in u, so the answer does not depend on the estimate
+__device__ __forceinline__ int edt_sep_w(int v, int hv, int i, int hi, int H, const EdtSpacing& sp) {
+    const double bv = edt_sq1(hv, sp.sx), bi = edt_sq1(hi, sp.sx);
+    // the estimate only has to land near the answer, so fp32 does (|error| << 1 wherever it is in [0, H]); the fp64
+    // division or reciprocal would bring a slow-path call, which spills
+    const float est = 0.5f * (float)(i + v) + __fdividef((float)(bi - bv), (float)(2.0 * (double)(i - v) * (sp.sy * sp.sy)));
+    int u = (int)fminf(fmaxf(ceilf(est), 0.f), (float)H);
+    while (u > 0 && edt_beats(i, bi, v, bv, u - 1, sp.sy)) --u;
+    while (u < H && !edt_beats(i, bi, v, bv, u, sp.sy)) ++u;
+    return u;
+}
+
+// EdtEnv with the weighted parabolas: same stack, same in-place layout, same order of pushes and pops.  The pop test
+// and the skip test are single comparisons at the top's start and at the last row; the separator (with its division)
+// is only computed for an entry that is pushed or becomes the top.
+struct EdtEnvW {
+    uint32_t* col;
+    size_t stride;
+    int top, v, h, z;
+    EdtSpacing sp;
+
+    __device__ __forceinline__ void load(int k, int& vk, int& hk) const {
+        const uint32_t e = col[(size_t)k * stride];
+        vk = (int)(e & 0xFFFFu);
+        hk = (int)(e >> 16);
+    }
+    __device__ __forceinline__ void put(int k, int vk, int hk) { col[(size_t)k * stride] = (uint32_t)vk | ((uint32_t)hk << 16); }
+
+    __device__ __forceinline__ void push(int i, int hi, int H) {
+        const double bi = edt_sq1(hi, sp.sx);
+        while (top >= 0) {
+            const double bv = edt_sq1(h, sp.sx);
+            if (!edt_beats(i, bi, v, bv, z, sp.sy)) {  // row i is above the top at its start: it starts later, if at all
+                if (edt_beats(i, bi, v, bv, H - 1, sp.sy)) {
+                    const int s = edt_sep_w(v, h, i, hi, H, sp);
+                    put(++top, i, hi); v = i; h = hi; z = s;
+                }
+                return;
+            }
+            if (--top >= 0) {  // row i is <= the top over the top's whole range: pop it
+                load(top, v, h);
+                if (top == 0) {
+                    z = 0;
+                } else {
+                    int pv, ph;
+                    load(top - 1, pv, ph);
+                    z = edt_sep_w(pv, ph, v, h, H, sp);
+                }
+            }
+        }
+        top = 0;
+        put(0, i, hi);
+        v = i; h = hi; z = 0;
+    }
+};
+
+// Walks a weighted envelope top to bottom: the packed offset (|u - v|, h) of the nearest pixel for u = 0, 1, ..., H - 1
+struct EdtWalkW {
+    int k, top, v, h, nv, nh, znext, H;
+    __device__ __forceinline__ void start(const EdtEnvW& e, int H_) {
+        top = e.top; H = H_; k = 0;
+        if (top < 0) return;
+        e.load(0, v, h);
+        znext = H;
+        if (top >= 1) { e.load(1, nv, nh); znext = edt_sep_w(v, h, nv, nh, H, e.sp); }
+    }
+    __device__ __forceinline__ uint32_t at(const EdtEnvW& e, int u) {
+        while (u >= znext) {
+            ++k; v = nv; h = nh; znext = H;
+            if (k < top) { e.load(k + 1, nv, nh); znext = edt_sep_w(v, h, nv, nh, H, e.sp); }
+        }
+        return edt_pack(abs(u - v), h);
+    }
+};
+
 enum EdtMode { kEdtField = 0, kEdtPred = 1, kEdtTarget = 2 };
 
 // s^(alpha / 2) = F^alpha in fp64
-__device__ __forceinline__ double edt_pow(int s, double half_alpha) {
-    const double d = (double)s;
+__device__ __forceinline__ double edt_pow(double d, double half_alpha) {
     return half_alpha == 1.0 ? d : half_alpha == 0.5 ? sqrt(d) : d == 0.0 ? 0.0 : exp(half_alpha * log(d));
 }
 
@@ -187,23 +307,30 @@ struct EdtColArgs {
     const float* t;         // kEdtTarget: targets
     double half_alpha;
     float* cost;            // kEdtTarget: [n]
+    const double* spacing;  // kSp: [n][2] (sy, sx) per map
 };
 
-template <int Mode>
+// kSp: the weighted envelope of the map's spacing; sp then holds the packed offset of P's nearest other-label pixel
+template <int Mode, bool kSp = false>
 __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
     constexpr int NL = Mode == kEdtField ? 1 : 2;
+    using Env = std::conditional_t<kSp, EdtEnvW, EdtEnv>;
+    using Walk = std::conditional_t<kSp, EdtWalkW, EdtWalk>;
     __shared__ double s_red[32];
     const int H = A.H, W = A.W;
     const size_t N = (size_t)H * W;
     for (int map = blockIdx.x; map < A.n_maps; map += gridDim.x) {
         double acc = 0.0;
+        EdtSpacing sp{};
+        if constexpr (kSp) sp = EdtSpacing{__ldg(A.spacing + 2 * map), __ldg(A.spacing + 2 * map + 1)};
         for (int j = threadIdx.x; j < W; j += blockDim.x) {
-            EdtEnv env[NL];
+            Env env[NL];
 #pragma unroll
             for (int L = 0; L < NL; ++L) {
                 env[L].col = A.h + ((size_t)map * N + j) * NL + L;
                 env[L].stride = (size_t)W * NL;
                 env[L].top = -1;
+                if constexpr (kSp) env[L].sp = sp;
             }
             for (int i = 0; i < H; ++i) {
 #pragma unroll
@@ -212,14 +339,22 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                     if (hi != kEdtNone) env[L].push(i, (int)hi, H);
                 }
             }
-            EdtWalk walk[NL];
+            Walk walk[NL];
 #pragma unroll
             for (int L = 0; L < NL; ++L) walk[L].start(env[L], H);
             const size_t o = (size_t)map * N + j;
             if (Mode == kEdtField) {
-                for (int u = 0; u < H; ++u)
-                    A.field[o + (size_t)u * W] = env[0].top < 0 ? __int_as_float(0x7F800000)
-                                                                : (float)sqrt((double)walk[0].at(env[0], u));
+                if constexpr (kSp) {
+                    if (env[0].top < 0) {
+                        for (int u = 0; u < H; ++u) A.field[o + (size_t)u * W] = __int_as_float(0x7F800000);
+                    } else {
+                        for (int u = 0; u < H; ++u) A.field[o + (size_t)u * W] = (float)sqrt(edt_packed_sq(walk[0].at(env[0], u), sp));
+                    }
+                } else {
+                    for (int u = 0; u < H; ++u)
+                        A.field[o + (size_t)u * W] = env[0].top < 0 ? __int_as_float(0x7F800000)
+                                                                    : (float)sqrt((double)walk[0].at(env[0], u));
+                }
             } else {
                 // a map with both labels: exactly one of s0, s1 is 0 per pixel; with one label only the field is 0
                 const bool mixed = env[0].top >= 0 && env[1].top >= 0;
@@ -229,7 +364,12 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                     if (Mode == kEdtPred) {
                         A.sp[q] = s;
                     } else {
-                        const double d = edt_pow(A.sp[q], A.half_alpha) + edt_pow(s, A.half_alpha);
+                        double d;
+                        if constexpr (kSp)
+                            d = edt_pow(edt_packed_sq((uint32_t)A.sp[q], sp), A.half_alpha) +
+                                edt_pow(edt_packed_sq((uint32_t)s, sp), A.half_alpha);
+                        else
+                            d = edt_pow(A.sp[q], A.half_alpha) + edt_pow(s, A.half_alpha);
                         const double p = (double)edt_sigmoid(__ldg(A.x + q)), diff = p - (double)__ldg(A.t + q);
                         acc += diff * diff * d;
                         A.D[q] = (float)d;

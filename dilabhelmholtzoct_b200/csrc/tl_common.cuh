@@ -154,31 +154,36 @@ __device__ __forceinline__ void radix_pick_digit(const uint32_t* s_hist, uint32_
     }
 }
 
-struct RadixPick {
-    uint32_t value;  // the k-th largest value
+template <class T>
+struct RadixPickT {
+    T value;         // the k-th largest value
     uint32_t k;      // its rank (1-based) among the values equal to it
     uint32_t count;  // how many values equal it
 };
+using RadixPick = RadixPickT<uint32_t>;
 
-// Exact block-wide radix select of the k-th largest (1 <= k <= n) of the n words key(0) .. key(n - 1), 8 bits per pass
-// from the top.  Every thread of a kThreads-thread block calls it with the same n and k; the trip counts are uniform,
-// so whole warps reach __match_any_sync.  s_hist is 256 words of shared memory, s_digit and s_k one word each; the
-// last barrier leaves them free for the caller.  For the k-th smallest, select over ~key.
-template <int kThreads, class Key>
-__device__ __forceinline__ RadixPick block_radix_select(const Key& key, int n, uint32_t k, uint32_t* s_hist,
-                                                        uint32_t* s_digit, uint32_t* s_k) {
+// Exact block-wide radix select of the k-th largest (1 <= k <= n) of the n keys key(0) .. key(n - 1) (T = uint32_t:
+// 4 passes, uint64_t: 8), 8 bits per pass from the top.  Every thread of a kThreads-thread block calls it with the
+// same n and k; the trip counts are uniform, so whole warps reach __match_any_sync.  s_hist is 256 words of shared
+// memory, s_digit and s_k one word each; the last barrier leaves them free for the caller.  For the k-th smallest,
+// select over ~key.
+template <int kThreads, class T = uint32_t, class Key>
+__device__ __forceinline__ RadixPickT<T> block_radix_select(const Key& key, int n, uint32_t k, uint32_t* s_hist,
+                                                            uint32_t* s_digit, uint32_t* s_k) {
+    constexpr int kTop = 8 * (int)sizeof(T) - 8;
     const int tid = threadIdx.x, lane = tid & 31;
-    uint32_t prefix = 0u, count = 0u;
-    for (int shift = 24; shift >= 0; shift -= 8) {
+    T prefix = 0u;
+    uint32_t count = 0u;
+    for (int shift = kTop; shift >= 0; shift -= 8) {
         for (int i = tid; i < 256; i += kThreads) s_hist[i] = 0u;
         __syncthreads();
-        const uint32_t hi_mask = shift == 24 ? 0u : ~0u << (shift + 8);
+        const T hi_mask = shift == kTop ? (T)0u : ~(T)0u << (shift + 8);
         for (int i0 = 0; i0 < n; i0 += kThreads) {
             const int i = i0 + tid;
             uint32_t d = 256u + (uint32_t)lane;  // distinct dummy digit for lanes without a candidate
             if (i < n) {
-                const uint32_t v = key(i);
-                if ((v & hi_mask) == prefix) d = (v >> shift) & 255u;
+                const T v = key(i);
+                if ((v & hi_mask) == prefix) d = (uint32_t)(v >> shift) & 255u;
             }
             const unsigned peers = __match_any_sync(0xFFFFFFFFu, d);
             if (d < 256u && (peers & lanemask_lt()) == 0u) atomicAdd(&s_hist[d], (uint32_t)__popc(peers));
@@ -186,12 +191,12 @@ __device__ __forceinline__ RadixPick block_radix_select(const Key& key, int n, u
         __syncthreads();
         if ((tid >> 5) == 0) radix_pick_digit(s_hist, k, s_digit, s_k);
         __syncthreads();
-        prefix |= *s_digit << shift;
+        prefix |= (T)*s_digit << shift;
         k = *s_k;
         count = s_hist[*s_digit];
         __syncthreads();  // s_hist / s_digit / s_k are rewritten by the next pass or the caller
     }
-    return RadixPick{prefix, k, count};
+    return RadixPickT<T>{prefix, k, count};
 }
 
 // Exact n / d for n < 2^24, d <= 8193 via multiply-shift (magic = ceil(2^40 / d)); avoids the

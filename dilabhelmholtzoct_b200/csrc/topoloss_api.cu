@@ -1227,11 +1227,56 @@ int edt_rows(Src src, int n_maps, int H, int W, uint32_t* h, cudaStream_t st) {
     return TL_OK;
 }
 
-template <int Mode>
+template <int Mode, bool kSp = false>
 int edt_cols(const tl::EdtColArgs& a, cudaStream_t st) {
-    tl::edt_col_kernel<Mode><<<a.n_maps < (1 << 20) ? a.n_maps : (1 << 20), tl::kEdtColThreads, 0, st>>>(a);
+    tl::edt_col_kernel<Mode, kSp><<<a.n_maps < (1 << 20) ? a.n_maps : (1 << 20), tl::kEdtColThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
+}
+
+// tl_edt and tl_edt_spaced (kSp: spacing is a device [n][2] array, checked non-null by the caller)
+template <bool kSp>
+int edt_field(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes,
+              float* out, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!mask || !ws || !out) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(ws) & 3) return fail(TL_ERR_ARG, "workspace must be 4-byte aligned");
+    const size_t need = align_up(sizeof(uint32_t) * edt_pixels(n_maps, H, W));
+    if (ws_bytes < need) return fail(TL_ERR_ARG, "workspace %zu < %zu bytes (tl_edt_workspace_bytes)", ws_bytes, need);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint32_t* h = static_cast<uint32_t*>(ws);
+    rc = edt_rows<tl::EdtMaskSrc, 1>(tl::EdtMaskSrc{mask}, n_maps, H, W, h, st);
+    if (rc != TL_OK) return rc;
+    tl::EdtColArgs a = {};
+    a.h = h; a.n_maps = n_maps; a.H = H; a.W = W; a.field = out; a.spacing = spacing;
+    return edt_cols<tl::kEdtField, kSp>(a, st);
+}
+
+// tl_hausdorff_dt_forward and its _spaced form
+template <bool kSp>
+int hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
+                         const double* spacing, void* state, size_t state_bytes, void* scratch, size_t scratch_bytes,
+                         float* cost, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!logits || !target || !state || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
+    if (!(alpha > 0.0) || !(alpha < HUGE_VAL)) return fail(TL_ERR_ARG, "alpha must be finite and positive, got %g", alpha);
+    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
+        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
+    const size_t ns = align_up(sizeof(float) * edt_pixels(n_maps, H, W)), nc = align_up(sizeof(uint2) * edt_pixels(n_maps, H, W));
+    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", state_bytes, ns);
+    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", scratch_bytes, nc);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    tl::EdtColArgs a = {};
+    a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W;
+    a.sp = static_cast<int32_t*>(state); a.D = static_cast<float*>(state);
+    a.x = logits; a.t = target; a.half_alpha = 0.5 * alpha; a.cost = cost; a.spacing = spacing;
+    rc = edt_rows<tl::EdtLogitSrc, 2>(tl::EdtLogitSrc{logits}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtPred, kSp>(a, st);
+    if (rc == TL_OK) rc = edt_rows<tl::EdtTargetSrc, 2>(tl::EdtTargetSrc{target}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtTarget, kSp>(a, st);
+    return rc;
 }
 
 }  // namespace
@@ -1247,19 +1292,14 @@ int tl_edt_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
 }
 
 int tl_edt(const uint8_t* mask, int n_maps, int H, int W, void* ws, size_t ws_bytes, float* out, void* stream) {
-    int rc = edt_shape(n_maps, H, W);
-    if (rc != TL_OK) return rc;
-    if (!mask || !ws || !out) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(ws) & 3) return fail(TL_ERR_ARG, "workspace must be 4-byte aligned");
-    const size_t need = align_up(sizeof(uint32_t) * edt_pixels(n_maps, H, W));
-    if (ws_bytes < need) return fail(TL_ERR_ARG, "workspace %zu < %zu bytes (tl_edt_workspace_bytes)", ws_bytes, need);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    uint32_t* h = static_cast<uint32_t*>(ws);
-    rc = edt_rows<tl::EdtMaskSrc, 1>(tl::EdtMaskSrc{mask}, n_maps, H, W, h, st);
-    if (rc != TL_OK) return rc;
-    tl::EdtColArgs a = {};
-    a.h = h; a.n_maps = n_maps; a.H = H; a.W = W; a.field = out;
-    return edt_cols<tl::kEdtField>(a, st);
+    return edt_field<false>(mask, n_maps, H, W, nullptr, ws, ws_bytes, out, stream);
+}
+
+int tl_edt_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes,
+                  float* out, void* stream) {
+    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
+    return edt_field<true>(mask, n_maps, H, W, spacing, ws, ws_bytes, out, stream);
 }
 
 int tl_hausdorff_dt_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes) {
@@ -1274,25 +1314,17 @@ int tl_hausdorff_dt_workspace_bytes(int n_maps, int H, int W, size_t* state_byte
 int tl_hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
                             void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
                             void* stream) {
-    int rc = edt_shape(n_maps, H, W);
-    if (rc != TL_OK) return rc;
-    if (!logits || !target || !state || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
-    if (!(alpha > 0.0) || !(alpha < HUGE_VAL)) return fail(TL_ERR_ARG, "alpha must be finite and positive, got %g", alpha);
-    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
-        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
-    const size_t ns = align_up(sizeof(float) * edt_pixels(n_maps, H, W)), nc = align_up(sizeof(uint2) * edt_pixels(n_maps, H, W));
-    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", state_bytes, ns);
-    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", scratch_bytes, nc);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    tl::EdtColArgs a = {};
-    a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W;
-    a.sp = static_cast<int32_t*>(state); a.D = static_cast<float*>(state);
-    a.x = logits; a.t = target; a.half_alpha = 0.5 * alpha; a.cost = cost;
-    rc = edt_rows<tl::EdtLogitSrc, 2>(tl::EdtLogitSrc{logits}, n_maps, H, W, a.h, st);
-    if (rc == TL_OK) rc = edt_cols<tl::kEdtPred>(a, st);
-    if (rc == TL_OK) rc = edt_rows<tl::EdtTargetSrc, 2>(tl::EdtTargetSrc{target}, n_maps, H, W, a.h, st);
-    if (rc == TL_OK) rc = edt_cols<tl::kEdtTarget>(a, st);
-    return rc;
+    return hausdorff_dt_forward<false>(logits, target, n_maps, H, W, alpha, nullptr, state, state_bytes, scratch,
+                                       scratch_bytes, cost, stream);
+}
+
+int tl_hausdorff_dt_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
+                                   const double* spacing, void* state, size_t state_bytes, void* scratch,
+                                   size_t scratch_bytes, float* cost, void* stream) {
+    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
+    return hausdorff_dt_forward<true>(logits, target, n_maps, H, W, alpha, spacing, state, state_bytes, scratch,
+                                      scratch_bytes, cost, stream);
 }
 
 int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_maps, int H, int W, const void* state,
@@ -1330,20 +1362,9 @@ SurfLayout surface_layout(int n_maps, int H, int W) {
     return L;
 }
 
-}  // namespace
-
-extern "C" {
-
-int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
-    if (!bytes) return fail(TL_ERR_ARG, "null pointer");
-    int rc = edt_shape(n_maps, H, W);
-    if (rc != TL_OK) return rc;
-    *bytes = surface_layout(n_maps, H, W).total;
-    return TL_OK;
-}
-
-int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
-                         double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
+template <bool kSp>
+int surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, const double* spacing,
+                      double percentile, double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
     int rc = edt_shape(n_maps, H, W);
     if (rc != TL_OK) return rc;
     if (!pred || !target || !ws || !out) return fail(TL_ERR_ARG, "null pointer");
@@ -1359,16 +1380,41 @@ int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps,
     a.keys = reinterpret_cast<uint32_t*>(base + L.keys);
     a.stats = reinterpret_cast<uint32_t*>(base + L.stats);
     a.n_maps = n_maps; a.H = H; a.W = W;
-    a.tol = tolerance; a.qq = percentile / 100.0; a.out = out;
+    a.tol = tolerance; a.qq = percentile / 100.0; a.out = out; a.spacing = spacing;
     rc = edt_rows<tl::SurfSrc, 1>(tl::SurfSrc{pred, H, W}, n_maps, H, W, a.h, st);
     if (rc == TL_OK) rc = edt_rows<tl::SurfSrc, 1>(tl::SurfSrc{target, H, W}, n_maps, H, W, a.h + edt_pixels(n_maps, H, W), st);
     if (rc != TL_OK) return rc;
     const int grid = n_maps < (1 << 20) ? n_maps : (1 << 20);
-    tl::surface_col_kernel<<<grid, tl::kEdtColThreads, 0, st>>>(a);
+    tl::surface_col_kernel<kSp><<<grid, tl::kEdtColThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
-    tl::surface_select_kernel<<<grid, tl::kSurfSelThreads, 0, st>>>(a);
+    tl::surface_select_kernel<kSp><<<grid, tl::kSurfSelThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
+    if (!bytes) return fail(TL_ERR_ARG, "null pointer");
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    *bytes = surface_layout(n_maps, H, W).total;
+    return TL_OK;
+}
+
+int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
+                         double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
+    return surface_distances<false>(pred, target, n_maps, H, W, nullptr, percentile, tolerance, ws, ws_bytes, out, stream);
+}
+
+int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W,
+                                const double* spacing, double percentile, double tolerance, void* ws, size_t ws_bytes,
+                                float* out, void* stream) {
+    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
+    return surface_distances<true>(pred, target, n_maps, H, W, spacing, percentile, tolerance, ws, ws_bytes, out, stream);
 }
 
 }  // extern "C"

@@ -433,6 +433,33 @@ int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes);
 int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
                          double tolerance, void* ws, size_t ws_bytes, float* out, void* stream);
 
+/*
+ * Physical pixel spacing for the three entry points above (DESIGN §3.10).  spacing is a device array
+ * [n_maps][2] of fp64 (sy, sx), 8-byte aligned: the size of a pixel along dim -2 (rows) and along dim -1 (columns),
+ * scipy's `sampling` order.  For a zero pixel at offset (dy, dx) the squared distance is the fp64 value
+ *   a = float64(dy) * sy;  b = float64(dx) * sx;  s = a*a + b*b        (each operation rounded, no contraction)
+ * and the distance is float32(sqrt(min s)): what scipy.ndimage.distance_transform_edt(m, sampling=(sy, sx)) gives,
+ * bit for bit.  The device cannot check the values: each must be finite and in [1e-6, 1e6], which keeps every square
+ * normal in fp64 and every output finite in fp32; that is the caller's contract.
+ *
+ * tl_edt_spaced                    as tl_edt, with the workspace of tl_edt_workspace_bytes.
+ * tl_hausdorff_dt_forward_spaced   as tl_hausdorff_dt_forward with F the spaced distance (D and the cost in physical
+ *                                  units), with the buffers of tl_hausdorff_dt_workspace_bytes; the backward is
+ *                                  tl_hausdorff_dt_backward.
+ * tl_surface_distances_spaced      as tl_surface_distances with d_pt, d_tp the spaced distances and tolerance in the
+ *                                  same units, with the workspace of tl_surface_workspace_bytes.
+ *
+ * Every argument error of the unspaced entry, and a null or misaligned spacing, returns TL_ERR_ARG before any launch.
+ */
+int tl_edt_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes,
+                  float* out, void* stream);
+int tl_hausdorff_dt_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
+                                   const double* spacing, void* state, size_t state_bytes, void* scratch,
+                                   size_t scratch_bytes, float* cost, void* stream);
+int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W,
+                                const double* spacing, double percentile, double tolerance, void* ws, size_t ws_bytes,
+                                float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
