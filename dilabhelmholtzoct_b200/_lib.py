@@ -80,6 +80,14 @@ SIGNATURES = {
                                                       ctypes.c_size_t, c_fp, ctypes.c_size_t, c_fp, c_fp]),
     "tl_surface_distances_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_double,
                                                    ctypes.c_double, c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_boundary_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)] * 2),
+    "tl_boundary_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp,
+                                           ctypes.c_size_t, c_fp, c_fp]),
+    "tl_boundary_forward_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp,
+                                                  ctypes.c_size_t, c_fp, c_fp]),
+    "tl_boundary_backward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
+    "tl_signed_distance": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_signed_distance_spaced": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp, c_fp]),
 }
 
 

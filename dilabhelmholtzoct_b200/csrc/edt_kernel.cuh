@@ -1,5 +1,6 @@
-// Exact Euclidean distance transform of 2-D binary maps (tl_edt) and the Hausdorff distance-transform loss
-// (tl_hausdorff_dt_*).  Separable, in the style of Meijster et al. (2000) / Felzenszwalb & Huttenlocher (2012):
+// Exact Euclidean distance transform of 2-D binary maps (tl_edt), the Hausdorff distance-transform loss
+// (tl_hausdorff_dt_*), and the signed distance map and boundary loss (tl_signed_distance*, tl_boundary_*).
+// Separable, in the style of Meijster et al. (2000) / Felzenszwalb & Huttenlocher (2012):
 //
 // edt_row_kernel<Src, NL>   one warp per row: per pixel, the horizontal distance h_L to the nearest pixel of label L
 //                           in its row (kEdtNone if the row has none), from 32-pixel ballots; NL = 1: label 0 only
@@ -9,6 +10,8 @@
 //                           stored in place over the column's h words, then queried top to bottom: the exact squared
 //                           distance s of every pixel to the nearest pixel of that label
 // hausdorff_dt_backward_kernel  elementwise: d cost / d x from the field D saved by the forward
+// edt_col_kernel<kEdtSigned>    the signed distance map phi (tl_signed_distance) and the boundary loss's cost
+//                               (tl_boundary_forward); boundary_backward_kernel: d cost / d x from the saved phi
 //
 // Every quantity of the envelope is an integer below 2^26 (H, W <= 4096: s <= 2 * 4095^2), so int32 holds all of it
 // and no float enters before the final root.  Entry point checks keep H and W in [1, 4096].
@@ -290,7 +293,8 @@ struct EdtWalkW {
     }
 };
 
-enum EdtMode { kEdtField = 0, kEdtPred = 1, kEdtTarget = 2 };
+// kEdtSigned: the signed distance map phi of the boundary loss (DESIGN §3.11) and, given logits, its cost
+enum EdtMode { kEdtField = 0, kEdtPred = 1, kEdtTarget = 2, kEdtSigned = 3 };
 
 // s^(alpha / 2) = F^alpha in fp64
 __device__ __forceinline__ double edt_pow(double d, double half_alpha) {
@@ -298,16 +302,17 @@ __device__ __forceinline__ double edt_pow(double d, double half_alpha) {
 }
 
 struct EdtColArgs {
-    uint32_t* h;            // row pass output: [n][H][W] words (kEdtField) or uint2 (kEdtPred, kEdtTarget)
+    uint32_t* h;            // row pass output: [n][H][W] words (kEdtField) or uint2 (kEdtPred, kEdtTarget, kEdtSigned)
     int n_maps, H, W;
-    float* field;           // kEdtField: out [n][H][W]
+    float* field;           // kEdtField: out [n][H][W]; kEdtSigned: phi [n][H][W]
     int32_t* sp;            // kEdtPred: s of P per pixel (0 where P is not mixed), in the D buffer
     float* D;               // kEdtTarget: F(P)^a + F(T)^a, overwriting sp
-    const float* x;         // kEdtTarget: logits
+    const float* x;         // kEdtTarget: logits; kEdtSigned: logits, or null for phi alone
     const float* t;         // kEdtTarget: targets
     double half_alpha;
-    float* cost;            // kEdtTarget: [n]
+    float* cost;            // kEdtTarget, kEdtSigned with x: [n]
     const double* spacing;  // kSp: [n][2] (sy, sx) per map
+    double inv_hw;          // kEdtSigned with x: 1 / HW (a device fp64 division would bring a slow-path call that spills)
 };
 
 // kSp: the weighted envelope of the map's spacing; sp then holds the packed offset of P's nearest other-label pixel
@@ -355,6 +360,25 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                         A.field[o + (size_t)u * W] = env[0].top < 0 ? __int_as_float(0x7F800000)
                                                                     : (float)sqrt((double)walk[0].at(env[0], u));
                 }
+            } else if constexpr (Mode == kEdtSigned) {
+                // label 0 is the background: on a mixed map s1 == 0 exactly on the foreground, where phi = 1 - d_in
+                // (d_in = sqrt(s0)); elsewhere phi = d_out = sqrt(s1).  fp64, rounded once; __dsub_rn / __dmul_rn /
+                // __dadd_rn keep nvcc from contracting (DESIGN §3.11)
+                const bool mixed = env[0].top >= 0 && env[1].top >= 0;
+                for (int u = 0; u < H; ++u) {
+                    const size_t q = o + (size_t)u * W;
+                    float phi = 0.f;
+                    if (mixed) {  // s (or the packed offset) is 0 exactly at the label's own pixels
+                        const auto e0 = walk[0].at(env[0], u), e1 = walk[1].at(env[1], u);
+                        const auto e = e1 == 0 ? e0 : e1;
+                        double d;
+                        if constexpr (kSp) d = sqrt(edt_packed_sq(e, sp));
+                        else d = sqrt((double)e);
+                        phi = (float)(e1 == 0 ? __dsub_rn(1.0, d) : d);
+                    }
+                    A.field[q] = phi;
+                    if (A.x) acc = __dadd_rn(acc, __dmul_rn((double)edt_sigmoid(__ldg(A.x + q)), (double)phi));
+                }
             } else {
                 // a map with both labels: exactly one of s0, s1 is 0 per pixel; with one label only the field is 0
                 const bool mixed = env[0].top >= 0 && env[1].top >= 0;
@@ -377,9 +401,9 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                 }
             }
         }
-        if (Mode == kEdtTarget) {
+        if (Mode == kEdtTarget || (Mode == kEdtSigned && A.x)) {
             const double s = block_sum(acc, s_red);
-            if (threadIdx.x == 0) A.cost[map] = (float)(s / (double)N);
+            if (threadIdx.x == 0) A.cost[map] = Mode == kEdtTarget ? (float)(s / (double)N) : (float)__dmul_rn(s, A.inv_hw);
             __syncthreads();  // s_red is reused by the next map
         }
     }
@@ -398,6 +422,23 @@ __global__ void __launch_bounds__(256) hausdorff_dt_backward_kernel(const float*
         for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) {
             const double p = (double)edt_sigmoid(__ldg(x + base + i));
             grad[base + i] = (float)(scale * (p - (double)__ldg(t + base + i)) * (double)__ldg(D + base + i) * p * (1.0 - p));
+        }
+    }
+}
+
+// the boundary loss: grad_x = grad_cost[map] * (1 / HW) * phi * p (1 - p), fp64, rounded to fp32, from the phi saved by
+// the forward (recomputing it would repeat the transform); blocks of 1024 pixels
+__global__ void __launch_bounds__(256) boundary_backward_kernel(const float* x, const float* phi, const float* grad_cost,
+                                                                 int n_maps, long long N, float* grad) {
+    const long long per_map = (N + 1023) / 1024;
+    for (long long b = blockIdx.x; b < (long long)n_maps * per_map; b += gridDim.x) {
+        const int map = (int)(b / per_map);
+        const long long lo = (b - (long long)map * per_map) * 1024, hi = min(lo + 1024, N);
+        const double scale = (double)__ldg(grad_cost + map) / (double)N;
+        const size_t base = (size_t)map * N;
+        for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) {
+            const double p = (double)edt_sigmoid(__ldg(x + base + i));
+            grad[base + i] = (float)(scale * (double)__ldg(phi + base + i) * p * (1.0 - p));
         }
     }
 }

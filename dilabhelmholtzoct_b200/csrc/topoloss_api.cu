@@ -1418,3 +1418,114 @@ int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int 
 }
 
 }  // extern "C"
+
+// ---- the signed distance map (tl_signed_distance*) and the boundary loss (tl_boundary_*), DESIGN §3.11
+namespace {
+
+// STATE: phi, fp32 per pixel (the backward reads it); SCRATCH: the row pass's h0 / h1, a uint2 per pixel
+size_t boundary_state_bytes(int n_maps, int H, int W) { return align_up(sizeof(float) * edt_pixels(n_maps, H, W)); }
+size_t boundary_scratch_bytes(int n_maps, int H, int W) { return align_up(sizeof(uint2) * edt_pixels(n_maps, H, W)); }
+
+int spacing_ok(const double* spacing) {
+    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
+    return TL_OK;
+}
+
+// tl_signed_distance and its _spaced form (kSp: spacing checked by the caller)
+template <bool kSp>
+int signed_distance(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
+                    size_t scratch_bytes, float* out, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!mask || !scratch || !out) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(scratch) & 7) return fail(TL_ERR_ARG, "scratch must be 8-byte aligned");
+    const size_t nc = boundary_scratch_bytes(n_maps, H, W);
+    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_boundary_workspace_bytes)", scratch_bytes, nc);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    tl::EdtColArgs a = {};
+    a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W; a.field = out; a.spacing = spacing;
+    rc = edt_rows<tl::EdtMaskSrc, 2>(tl::EdtMaskSrc{mask}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtSigned, kSp>(a, st);
+    return rc;
+}
+
+// tl_boundary_forward and its _spaced form
+template <bool kSp>
+int boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, const double* spacing,
+                     void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!logits || !target || !state || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
+    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
+        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
+    const size_t ns = boundary_state_bytes(n_maps, H, W), nc = boundary_scratch_bytes(n_maps, H, W);
+    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_boundary_workspace_bytes)", state_bytes, ns);
+    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_boundary_workspace_bytes)", scratch_bytes, nc);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    tl::EdtColArgs a = {};
+    a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W;
+    a.field = static_cast<float*>(state); a.x = logits; a.cost = cost; a.spacing = spacing;
+    a.inv_hw = 1.0 / ((double)H * W);
+    rc = edt_rows<tl::EdtTargetSrc, 2>(tl::EdtTargetSrc{target}, n_maps, H, W, a.h, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtSigned, kSp>(a, st);
+    return rc;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tl_boundary_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes) {
+    if (!state_bytes || !scratch_bytes) return fail(TL_ERR_ARG, "null pointer");
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    *state_bytes = boundary_state_bytes(n_maps, H, W);
+    *scratch_bytes = boundary_scratch_bytes(n_maps, H, W);
+    return TL_OK;
+}
+
+int tl_signed_distance(const uint8_t* mask, int n_maps, int H, int W, void* scratch, size_t scratch_bytes, float* out,
+                       void* stream) {
+    return signed_distance<false>(mask, n_maps, H, W, nullptr, scratch, scratch_bytes, out, stream);
+}
+
+int tl_signed_distance_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
+                              size_t scratch_bytes, float* out, void* stream) {
+    const int rc = spacing_ok(spacing);
+    if (rc != TL_OK) return rc;
+    return signed_distance<true>(mask, n_maps, H, W, spacing, scratch, scratch_bytes, out, stream);
+}
+
+int tl_boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, void* state,
+                        size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream) {
+    return boundary_forward<false>(logits, target, n_maps, H, W, nullptr, state, state_bytes, scratch, scratch_bytes,
+                                   cost, stream);
+}
+
+int tl_boundary_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W,
+                               const double* spacing, void* state, size_t state_bytes, void* scratch,
+                               size_t scratch_bytes, float* cost, void* stream) {
+    const int rc = spacing_ok(spacing);
+    if (rc != TL_OK) return rc;
+    return boundary_forward<true>(logits, target, n_maps, H, W, spacing, state, state_bytes, scratch, scratch_bytes,
+                                  cost, stream);
+}
+
+int tl_boundary_backward(const float* logits, int n_maps, int H, int W, const void* state, size_t state_bytes,
+                         const float* grad_cost, float* grad_logits, void* stream) {
+    int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    if (!logits || !state || !grad_cost || !grad_logits) return fail(TL_ERR_ARG, "null pointer");
+    if (reinterpret_cast<uintptr_t>(state) & 3) return fail(TL_ERR_ARG, "state must be 4-byte aligned");
+    const size_t ns = boundary_state_bytes(n_maps, H, W);
+    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_boundary_workspace_bytes)", state_bytes, ns);
+    const long long N = (long long)H * W;
+    tl::boundary_backward_kernel<<<edt_grid((long long)n_maps * ((N + 1023) / 1024), 1), 256, 0,
+                                   static_cast<cudaStream_t>(stream)>>>(logits, static_cast<const float*>(state),
+                                                                         grad_cost, n_maps, N, grad_logits);
+    TL_CUDA(cudaGetLastError());
+    return TL_OK;
+}
+
+}  // extern "C"

@@ -6,9 +6,11 @@ loss of Karimi & Salcudean (IEEE TMI 2020) per ``(b, c)`` map of decoder logits,
 logits (``tl_hausdorff_dt_*``).  Both transforms of each map (prediction and target, foreground and background) run
 in the same kernels as the loss; nothing goes through the host.  ``surface_distances(pred, target)`` gives the
 boundary metrics of mask pairs -- Hausdorff distance, percentile Hausdorff distance, ASSD and normalized surface Dice
--- from the same transform measured at surface pixels (``tl_surface_distances``).
+-- from the same transform measured at surface pixels (``tl_surface_distances``).  ``signed_distance_map(mask)`` is
+the signed distance map of Kervadec et al.'s boundary loss, and ``boundary_loss(masks, gt_masks)`` that loss on
+logits (``tl_signed_distance``, ``tl_boundary_*``, DESIGN §3.11).
 
-All three measure in pixels by default.  Given a physical pixel spacing (``sampling=`` for the transform, as scipy
+All of them measure in pixels by default.  Given a physical pixel spacing (``sampling=`` for the transform, as scipy
 names it; ``spacing=`` for the loss and the metrics, as monai names it) they measure in its units instead, through
 the ``tl_*_spaced`` entry points (DESIGN §3.10).
 
@@ -296,3 +298,148 @@ def hausdorff_dt_loss(masks: torch.Tensor, gt_masks: torch.Tensor, alpha: float 
     if B * C == 0:
         return masks.sum((2, 3))  # empty, still attached to autograd
     return _HausdorffDtFn.apply(masks.contiguous(), gt_masks.detach().to(torch.float32).contiguous(), alpha, sp)
+
+
+def signed_distance_map(mask: torch.Tensor, sampling=None) -> torch.Tensor:
+    """Signed distance map of every ``[H, W]`` map of ``mask`` (``[..., H, W]``, bool or uint8, CUDA; a nonzero pixel
+    is foreground), as the boundary loss of Kervadec et al. (MIDL 2019, MedIA 2021) uses it.  Returns float32 of the
+    same shape, without autograd.  On a map that holds both labels, with ``M`` the foreground and ``edt`` scipy's
+    ``distance_transform_edt``, it is the float64 expression of Kervadec's ``one_hot2dist`` (by recollection, unpinned)
+    rounded to float32::
+
+        phi = edt(~M, sampling) * ~M - (edt(M, sampling) - 1) * M
+
+    so a background pixel gets its distance to the nearest foreground pixel, and a foreground pixel gets ``1 - d_in``,
+    ``d_in`` its distance to the nearest background pixel: 0 on the inner boundary, negative deeper inside.  It equals
+    that numpy / scipy expression bit for bit, the sign of zero included.  A map with one label only gets 0 everywhere:
+    for an all-background map this is Kervadec's rule (an all-zero padded mask adds nothing to the loss); for an
+    all-foreground map Kervadec's code would measure to scipy's phantom pixel, which is not reproduced.
+
+    ``sampling`` (scipy's name and order) is a physical pixel spacing ``(sy, sx)`` in the forms and with the checks of
+    ``distance_transform_edt``; the distances are then that op's distances in the spacing's units, and the ``- 1`` is
+    in the same units, as in Kervadec's code: it is one unit, not one pixel.  With an absolute spacing in mm such as
+    ``(3.9e-3, 11.7e-3)`` the ``- 1`` is 1 mm, hundreds of rows, so ``phi`` stays positive deep inside the foreground;
+    a relative spacing such as ``(1.0, 3.0)`` keeps one row as the unit and still weighs a column three times.  ``None``
+    (the default) is unit spacing through the integer path.  H and W must each be in [1, 4096].  No host
+    synchronisation; 8 bytes per pixel of scratch are taken from PyTorch's caching allocator for the duration of the
+    call."""
+    if not torch.is_tensor(mask):
+        raise TypeError("mask must be a tensor")
+    if mask.dim() < 2:
+        raise ValueError("signed_distance_map expects [..., H, W] maps")
+    if not mask.is_cuda:
+        raise ValueError("signed_distance_map runs on a CUDA device only: there is no CPU fallback")
+    if mask.dtype not in (torch.bool, torch.uint8):
+        raise ValueError(f"signed_distance_map expects a bool or uint8 mask, got {mask.dtype}")
+    H, W = int(mask.shape[-2]), int(mask.shape[-1])
+    _check_hw(H, W, "signed_distance_map")
+    n = mask.numel() // (H * W)
+    dev = mask.device
+    out = torch.empty(mask.shape, dtype=torch.float32, device=dev)
+    sp = None if sampling is None else _spacing_tensor(sampling, mask.shape[:-2], dev, "signed_distance_map")
+    if n == 0:
+        return out
+    m = mask.detach().contiguous()
+    if m.dtype == torch.bool:
+        m = m.view(torch.uint8)
+    L = _lib.lib()
+    ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
+    _lib.check(L.tl_boundary_workspace_bytes(n, H, W, ctypes.byref(ns), ctypes.byref(nc)), "tl_boundary_workspace_bytes")
+    with torch.cuda.device(dev):
+        scratch = torch.empty(nc.value, dtype=torch.uint8, device=dev)  # per call: released to the caching allocator
+        if sp is None:
+            rc = L.tl_signed_distance(m.data_ptr(), n, H, W, scratch.data_ptr(), scratch.numel(), out.data_ptr(),
+                                      _stream_ptr(dev))
+        else:
+            rc = L.tl_signed_distance_spaced(m.data_ptr(), n, H, W, sp.data_ptr(), scratch.data_ptr(), scratch.numel(),
+                                             out.data_ptr(), _stream_ptr(dev))
+    _lib.check(rc, "tl_signed_distance" if sp is None else "tl_signed_distance_spaced")
+    return out
+
+
+class _BoundaryFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, t, sp):
+        B, C, H, W = (int(d) for d in x.shape)
+        n = B * C
+        dev = x.device
+        L = _lib.lib()
+        ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
+        _lib.check(L.tl_boundary_workspace_bytes(n, H, W, ctypes.byref(ns), ctypes.byref(nc)),
+                   "tl_boundary_workspace_bytes")
+        with torch.cuda.device(dev):
+            state = torch.empty(ns.value, dtype=torch.uint8, device=dev)  # phi per pixel: the backward reads it
+            scratch = torch.empty(nc.value, dtype=torch.uint8, device=dev)  # per call, freed when the forward returns
+            cost = torch.empty((B, C), dtype=torch.float32, device=dev)
+            if sp is None:
+                rc = L.tl_boundary_forward(x.data_ptr(), t.data_ptr(), n, H, W, state.data_ptr(), state.numel(),
+                                           scratch.data_ptr(), scratch.numel(), cost.data_ptr(), _stream_ptr(dev))
+            else:
+                rc = L.tl_boundary_forward_spaced(x.data_ptr(), t.data_ptr(), n, H, W, sp.data_ptr(), state.data_ptr(),
+                                                  state.numel(), scratch.data_ptr(), scratch.numel(), cost.data_ptr(),
+                                                  _stream_ptr(dev))
+        _lib.check(rc, "tl_boundary_forward" if sp is None else "tl_boundary_forward_spaced")
+        ctx.save_for_backward(x, state)
+        return cost
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_cost):
+        x, state = ctx.saved_tensors
+        B, C, H, W = (int(d) for d in x.shape)
+        dev = x.device
+        with torch.cuda.device(dev):
+            gc = g_cost.to(device=dev, dtype=torch.float32).contiguous()
+            grad = torch.empty_like(x)
+            rc = _lib.lib().tl_boundary_backward(x.data_ptr(), B * C, H, W, state.data_ptr(), state.numel(),
+                                                 gc.data_ptr(), grad.data_ptr(), _stream_ptr(dev))
+        _lib.check(rc, "tl_boundary_backward")
+        return grad, None, None
+
+
+def boundary_loss(masks: torch.Tensor, gt_masks: torch.Tensor, spacing=None) -> torch.Tensor:
+    """Boundary loss (Kervadec et al., MIDL 2019, MedIA 2021) of every ``(b, c)`` map: float32 ``[B, C]``,
+    differentiable with respect to ``masks`` only.
+
+    ``masks`` are float32 decoder logits ``[B, C, H, W]`` on CUDA; ``gt_masks`` has the same shape and any real or
+    bool dtype, and is cast to float32 (as ``hausdorff_dt_loss`` does).  Per map, with ``p = torch.sigmoid(x)``
+    (fp32) and ``phi = signed_distance_map(t > 0.5, spacing)`` (float32)::
+
+        cost = (1 / HW) * sum_i float64(p_i) * float64(phi_i)
+
+    summed in fp64 in a fixed order and rounded to fp32, so the cost is bit-identical from run to run; the gradient is
+    ``(1 / HW) * phi * p * (1 - p)`` in fp64, rounded to fp32.  The loss is linear in the probabilities: it is lowest
+    when the foreground probability sits inside the target and falls off outside it in proportion to the distance.
+    ``.mean()`` of the result is, by recollection (unpinned: the reference code is not a dependency), Kervadec's
+    ``SurfaceLoss`` over all channels with sigmoid probabilities in place of softmax.  ``phi`` follows
+    ``signed_distance_map``: 0 on a map whose target holds one label only, so an all-zero padded target gives cost 0
+    and gradient 0 (Kervadec's rule for an empty target; an all-foreground target, where Kervadec's code would measure
+    to scipy's phantom pixel, is not reproduced).  It is usually added to a region loss, as
+    ``dice_ce_loss(...) + w * boundary_loss(...).mean()``.
+
+    ``spacing`` measures ``phi`` in physical units instead of pixels, so the cost is in those units, and the ``- 1`` of
+    ``phi`` is one such unit (see ``signed_distance_map``).  It takes the forms of ``surface_distances``'s ``spacing``,
+    broadcast to ``[B, C, 2]``, with the same checks.  ``None`` (the default) is unit spacing through the integer path.
+
+    H and W must each be in [1, 4096].  A NaN logit makes that map's cost NaN and leaves the other maps alone.  Neither
+    the forward nor the backward synchronises the host.  The forward keeps phi (4 bytes per pixel) for the backward,
+    and takes 8 bytes per pixel of scratch from PyTorch's caching allocator for the duration of the call; nothing is
+    kept between calls."""
+    if not (torch.is_tensor(masks) and torch.is_tensor(gt_masks)):
+        raise TypeError("masks and gt_masks must be tensors")
+    if masks.dim() != 4 or masks.shape != gt_masks.shape:
+        raise ValueError("expected two [B, C, H, W] tensors of the same shape")
+    if not masks.is_cuda or not gt_masks.is_cuda:
+        raise ValueError("boundary_loss runs on a CUDA device only: there is no CPU fallback")
+    if masks.device != gt_masks.device:
+        raise ValueError(f"masks are on {masks.device}, gt_masks on {gt_masks.device}")
+    if masks.dtype != torch.float32:
+        raise ValueError(f"boundary_loss expects float32 logits, got {masks.dtype}")
+    if gt_masks.dtype.is_complex:
+        raise ValueError(f"boundary_loss expects a real or bool gt_masks, got {gt_masks.dtype}")
+    B, C, H, W = (int(d) for d in masks.shape)
+    _check_hw(H, W, "boundary_loss")
+    sp = None if spacing is None else _spacing_tensor(spacing, masks.shape[:2], masks.device, "boundary_loss")
+    if B * C == 0:
+        return masks.sum((2, 3))  # empty, still attached to autograd
+    return _BoundaryFn.apply(masks.contiguous(), gt_masks.detach().to(torch.float32).contiguous(), sp)

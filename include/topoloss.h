@@ -460,6 +460,45 @@ int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int 
                                 const double* spacing, double percentile, double tolerance, void* ws, size_t ws_bytes,
                                 float* out, void* stream);
 
+/*
+ * Signed distance map and the boundary loss of Kervadec et al. (MIDL 2019, MedIA 2021) on n_maps HxW maps (H, W in
+ * [1, 4096]), DESIGN §3.11.  For a mask M (foreground = label 1) holding both labels, per pixel, in fp64 rounded once
+ * to fp32:
+ *   phi = d_out                on the background, d_out the distance to the nearest foreground pixel
+ *       = 1 - d_in             on the foreground, d_in the distance to the nearest background pixel
+ * -- scipy's edt(~M) * ~M - (edt(M) - 1) * M bit for bit, with the distances of tl_edt (unit) or tl_edt_spaced (the
+ * `1` is then in the spacing's units).  A map with one label only gets phi = 0 everywhere.
+ * The loss, per map of fp32 logits x and targets t: p = sigmoid(x) (fp32, as torch.sigmoid), phi = phi(t > 0.5) and
+ *   cost = (1 / HW) * sum_i p_i * phi_i      (fp64, fixed order, rounded to fp32)
+ *
+ * tl_boundary_workspace_bytes  *state_bytes (phi, 4 bytes per pixel: written by the forward, read by the backward) and
+ *                              *scratch_bytes (8 bytes per pixel, only live inside a call).
+ * tl_boundary_forward          cost[n_maps] (fp32, device).  state 4-byte, scratch 8-byte aligned.  A NaN logit makes
+ *                              its map's cost NaN.  The cost is bit-identical from run to run.
+ * tl_boundary_backward         grad_logits[n_maps][H][W], fully overwritten with grad_cost[i] * (1 / HW) * phi * p *
+ *                              (1 - p) (fp64, rounded to fp32); logits and state are those of the forward; state 4-byte
+ *                              aligned.
+ * tl_signed_distance           mask[n_maps][H][W] (uint8, device; nonzero = foreground) -> out[n_maps][H][W] (fp32,
+ *                              device): phi, with the scratch of tl_boundary_workspace_bytes (8-byte aligned).
+ * tl_*_spaced                  the same with a device fp64 spacing [n_maps][2] (sy, sx), 8-byte aligned, as for
+ *                              tl_edt_spaced; tl_boundary_backward serves both forwards.
+ *
+ * Every argument error (null pointer, H or W out of range, a buffer smaller than the query asks for or misaligned, a
+ * null or misaligned spacing) returns TL_ERR_ARG before any launch.  No entry point synchronises the host.
+ */
+int tl_boundary_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes);
+int tl_boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, void* state,
+                        size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream);
+int tl_boundary_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W,
+                               const double* spacing, void* state, size_t state_bytes, void* scratch,
+                               size_t scratch_bytes, float* cost, void* stream);
+int tl_boundary_backward(const float* logits, int n_maps, int H, int W, const void* state, size_t state_bytes,
+                         const float* grad_cost, float* grad_logits, void* stream);
+int tl_signed_distance(const uint8_t* mask, int n_maps, int H, int W, void* scratch, size_t scratch_bytes, float* out,
+                       void* stream);
+int tl_signed_distance_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
+                              size_t scratch_bytes, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
