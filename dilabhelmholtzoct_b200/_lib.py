@@ -11,7 +11,7 @@ _LIB = None
 
 c_fp = ctypes.c_void_p  # device pointers travel as integers
 TL_OK = 0
-ABI_VERSION = 4
+ABI_VERSION = 5
 OPT_FORCE_GLOBAL_KERNEL, OPT_PROFILE, OPT_NO_BINARY_PATH, OPT_WORST_CASE_WORKSPACE, OPT_NO_FUSED_MATCH, OPT_NO_FUSED_GRAD = 0, 1, 2, 3, 4, 5
 OPT_LIST_MODE = 6
 STATUS_BITS = {1: "pair arena exhausted (pass a larger state buffer: TL_ARENA_FACTOR / set_arena_factor)",
@@ -67,27 +67,19 @@ SIGNATURES = {
                                         c_fp, c_fp]),
     "tl_prior_backward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 4 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
     "tl_edt_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)]),
-    "tl_edt": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_edt": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp, c_fp]),
     "tl_hausdorff_dt_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)] * 2),
-    "tl_hausdorff_dt_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, c_fp, ctypes.c_size_t,
-                                               c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_hausdorff_dt_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, c_fp, c_fp,
+                                               ctypes.c_size_t, c_fp, ctypes.c_size_t, c_fp, c_fp]),
     "tl_hausdorff_dt_backward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
     "tl_surface_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)]),
-    "tl_surface_distances": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, ctypes.c_double, c_fp,
-                                            ctypes.c_size_t, c_fp, c_fp]),
-    "tl_edt_spaced": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp, c_fp]),
-    "tl_hausdorff_dt_forward_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [ctypes.c_double, c_fp, c_fp,
-                                                      ctypes.c_size_t, c_fp, ctypes.c_size_t, c_fp, c_fp]),
-    "tl_surface_distances_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_double,
-                                                   ctypes.c_double, c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_surface_distances": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_double, ctypes.c_double,
+                                            c_fp, ctypes.c_size_t, c_fp, c_fp]),
     "tl_boundary_workspace_bytes": (ctypes.c_int, [ctypes.c_int] * 3 + [ctypes.POINTER(ctypes.c_size_t)] * 2),
-    "tl_boundary_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp,
+    "tl_boundary_forward": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp,
                                            ctypes.c_size_t, c_fp, c_fp]),
-    "tl_boundary_forward_spaced": (ctypes.c_int, [c_fp, c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp,
-                                                  ctypes.c_size_t, c_fp, c_fp]),
     "tl_boundary_backward": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp, c_fp]),
-    "tl_signed_distance": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, ctypes.c_size_t, c_fp, c_fp]),
-    "tl_signed_distance_spaced": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp, c_fp]),
+    "tl_signed_distance": (ctypes.c_int, [c_fp] + [ctypes.c_int] * 3 + [c_fp, c_fp, ctypes.c_size_t, c_fp, c_fp]),
 }
 
 

@@ -1,11 +1,11 @@
 // Exact Euclidean distance transform of 2-D binary maps (tl_edt), the Hausdorff distance-transform loss
-// (tl_hausdorff_dt_*), and the signed distance map and boundary loss (tl_signed_distance*, tl_boundary_*).
+// (tl_hausdorff_dt_*), and the signed distance map and boundary loss (tl_signed_distance, tl_boundary_*).
 // Separable, in the style of Meijster et al. (2000) / Felzenszwalb & Huttenlocher (2012):
 //
 // edt_row_kernel<Src, NL>   one warp per row: per pixel, the horizontal distance h_L to the nearest pixel of label L
 //                           in its row (kEdtNone if the row has none), from 32-pixel ballots; NL = 1: label 0 only
 //                           (uint32 per pixel), NL = 2: labels 0 and 1 (uint2 per pixel)
-// edt_col_kernel<Mode>      one CTA per map, one thread per column: per label, the lower envelope of the parabolas
+// edt_col_kernel<Mode, M>   one CTA per map, one thread per column: per label, the lower envelope of the parabolas
 //                           (u - i)^2 + h_i^2 over the rows i with a finite h_i, built top to bottom with its stack
 //                           stored in place over the column's h words, then queried top to bottom: the exact squared
 //                           distance s of every pixel to the nearest pixel of that label
@@ -16,8 +16,8 @@
 // Every quantity of the envelope is an integer below 2^26 (H, W <= 4096: s <= 2 * 4095^2), so int32 holds all of it
 // and no float enters before the final root.  Entry point checks keep H and W in [1, 4096].
 //
-// With a physical pixel spacing (sy, sx) per map (tl_*_spaced, DESIGN §3.10) the row pass is the same, and the column
-// pass builds the weighted envelope (EdtEnvW / EdtWalkW) instead: row i's parabola is the fp64 value
+// With a physical pixel spacing (sy, sx) per map (a non-null spacing, DESIGN §3.10) the row pass is the same, and the
+// column pass builds the weighted envelope (metric EdtSpacing, not EdtUnit): row i's parabola is the fp64 value
 // s(u) = (float64(u - i) * sy)^2 + (float64(h_i) * sx)^2, each operation rounded, and the walk yields the offset
 // (|u - v|, h) of the nearest pixel, packed in 24 bits (edt_pack), from which s is recomputed where it is needed.
 #pragma once
@@ -119,84 +119,12 @@ __device__ __forceinline__ int edt_sep(int v, int hv, int i, int hi) {
     return edt_ceil_div(i * i + hi * hi - v * v - hv * hv, 2 * (i - v));
 }
 
-// The lower envelope of one label over one column.  Entry k of the stack (row v_k, distance h_k, packed v | h << 16)
-// lives in the column's word of row k: when row i is pushed the stack holds at most i + 1 entries, and rows <= i have
-// been read, so the stack only overwrites consumed input.  The start z_k of entry k (the first u it is the minimum at;
-// z_0 = 0) is recomputed from entries k - 1 and k when it is needed.
-struct EdtEnv {
-    uint32_t* col;
-    size_t stride;
-    int top, v, h, z;  // top entry and its start; top = -1: empty
-
-    __device__ __forceinline__ void load(int k, int& vk, int& hk) const {
-        const uint32_t e = col[(size_t)k * stride];
-        vk = (int)(e & 0xFFFFu);
-        hk = (int)(e >> 16);
-    }
-    __device__ __forceinline__ void put(int k, int vk, int hk) { col[(size_t)k * stride] = (uint32_t)vk | ((uint32_t)hk << 16); }
-
-    __device__ __forceinline__ void push(int i, int hi, int H) {
-        while (top >= 0) {
-            const int s = edt_sep(v, h, i, hi);
-            if (s > z) {  // row i is the minimum from s on; past the last row it never is
-                if (s < H) { put(++top, i, hi); v = i; h = hi; z = s; }
-                return;
-            }
-            if (--top >= 0) {  // row i is <= the top over the top's whole range: pop it
-                load(top, v, h);
-                if (top == 0) {
-                    z = 0;
-                } else {
-                    int pv, ph;
-                    load(top - 1, pv, ph);
-                    z = edt_sep(pv, ph, v, h);
-                }
-            }
-        }
-        top = 0;
-        put(0, i, hi);
-        v = i; h = hi; z = 0;
-    }
-};
-
-// Walks an envelope top to bottom: s(u) for u = 0, 1, ..., H - 1 in that order.
-struct EdtWalk {
-    int k, top, v, h, nv, nh, znext, H;
-    __device__ __forceinline__ void start(const EdtEnv& e, int H_) {
-        top = e.top; H = H_; k = 0;
-        if (top < 0) return;
-        e.load(0, v, h);
-        znext = H;
-        if (top >= 1) { e.load(1, nv, nh); znext = edt_sep(v, h, nv, nh); }
-    }
-    __device__ __forceinline__ int at(const EdtEnv& e, int u) {
-        while (u >= znext) {
-            ++k; v = nv; h = nh; znext = H;
-            if (k < top) { e.load(k + 1, nv, nh); znext = edt_sep(v, h, nv, nh); }
-        }
-        return (u - v) * (u - v) + h * h;
-    }
-};
-
-// ---- the weighted envelope (physical spacing)
-
-struct EdtSpacing {
-    double sy, sx;  // size of a pixel along rows (dim -2) and along columns (dim -1)
-};
+// ---- the weighted parabolas (physical spacing)
 
 // float64(d) * sp, squared, each operation rounded to fp64 (no contraction)
 __device__ __forceinline__ double edt_sq1(int d, double sp) {
     const double a = __dmul_rn((double)d, sp);
     return __dmul_rn(a, a);
-}
-// the squared distance of offset (dy, dx) as scipy's distance_transform_edt(sampling=...) evaluates it
-__device__ __forceinline__ double edt_sq(int dy, int dx, const EdtSpacing& sp) {
-    return __dadd_rn(edt_sq1(dy, sp.sy), edt_sq1(dx, sp.sx));
-}
-// offsets below 4096 each, packed in 24 bits; 0 exactly at offset (0, 0)
-__device__ __forceinline__ uint32_t edt_pack(int dy, int dx) { return (uint32_t)dy | ((uint32_t)dx << 12); }
-__device__ __forceinline__ double edt_packed_sq(uint32_t p, const EdtSpacing& sp) {
-    return edt_sq((int)(p & 0xFFFu), (int)(p >> 12), sp);
 }
 
 // a1 + b1 <= a2 + b2 for doubles, exactly as real numbers: a rounded sum orders the reals (round to nearest is
@@ -219,25 +147,67 @@ __device__ __forceinline__ bool edt_beats(int i, double bi, int v, double bv, in
 
 // The first u in [0, H] at which row i > v beats row v (H: none): the crossing of the exact parabolas as an fp64
 // estimate, then corrected by the exact predicate, which is monotone in u, so the answer does not depend on the estimate
-__device__ __forceinline__ int edt_sep_w(int v, int hv, int i, int hi, int H, const EdtSpacing& sp) {
-    const double bv = edt_sq1(hv, sp.sx), bi = edt_sq1(hi, sp.sx);
+__device__ __forceinline__ int edt_sep_w(int v, int hv, int i, int hi, int H, double sy, double sx) {
+    const double bv = edt_sq1(hv, sx), bi = edt_sq1(hi, sx);
     // the estimate only has to land near the answer, so fp32 does (|error| << 1 wherever it is in [0, H]); the fp64
     // division or reciprocal would bring a slow-path call, which spills
-    const float est = 0.5f * (float)(i + v) + __fdividef((float)(bi - bv), (float)(2.0 * (double)(i - v) * (sp.sy * sp.sy)));
+    const float est = 0.5f * (float)(i + v) + __fdividef((float)(bi - bv), (float)(2.0 * (double)(i - v) * (sy * sy)));
     int u = (int)fminf(fmaxf(ceilf(est), 0.f), (float)H);
-    while (u > 0 && edt_beats(i, bi, v, bv, u - 1, sp.sy)) --u;
-    while (u < H && !edt_beats(i, bi, v, bv, u, sp.sy)) ++u;
+    while (u > 0 && edt_beats(i, bi, v, bv, u - 1, sy)) --u;
+    while (u < H && !edt_beats(i, bi, v, bv, u, sy)) ++u;
     return u;
 }
 
-// EdtEnv with the weighted parabolas: same stack, same in-place layout, same order of pushes and pops.  The pop test
-// and the skip test are single comparisons at the top's start and at the last row; the separator (with its division)
-// is only computed for an entry that is pushed or becomes the top.
-struct EdtEnvW {
+// offsets below 4096 each, packed in 24 bits; 0 exactly at offset (0, 0)
+__device__ __forceinline__ uint32_t edt_pack(int dy, int dx) { return (uint32_t)dy | ((uint32_t)dx << 12); }
+
+// ---- the metric of the column pass
+//
+// What differs between unit and physical spacing.  EdtUnit: the integer parabolas; the walk yields s itself.
+// EdtSpacing: the weighted parabolas of the map's spacing; the walk yields the packed offset (|u - v|, h) of the nearest
+// pixel (edt_pack), from which s is recomputed where it is needed.  Each metric gives
+//   sep(v, hv, i, hi, H)          the first u at which row i > v is <= row v (EdtSpacing: in [0, H], H for none)
+//   at(dy, h)                     what the walk yields at row offset dy = u - v and distance h; 0 exactly at (0, 0)
+//   sq(e)                         the fp64 squared distance s of a walk value
+//   key(e), key_sq(k)             walk values as unsigned integers in the order of s, kEdtNone above all of them,
+//                                 and the fp64 s of a key
+
+struct EdtUnit {
+    using Key = uint32_t;
+    static __device__ __forceinline__ EdtUnit of(const double*, int) { return {}; }
+    __device__ __forceinline__ int sep(int v, int hv, int i, int hi, int) const { return edt_sep(v, hv, i, hi); }
+    __device__ __forceinline__ int at(int dy, int h) const { return dy * dy + h * h; }
+    __device__ __forceinline__ double sq(int s) const { return (double)s; }
+    __device__ __forceinline__ Key key(uint32_t s) const { return s; }
+    __device__ __forceinline__ double key_sq(Key k) const { return (double)k; }
+};
+
+struct EdtSpacing {
+    using Key = unsigned long long;  // the bits of s, monotone as uint64 for s >= 0
+    double sy, sx;                   // size of a pixel along rows (dim -2) and along columns (dim -1)
+    static __device__ __forceinline__ EdtSpacing of(const double* spacing, int map) {
+        return {__ldg(spacing + 2 * map), __ldg(spacing + 2 * map + 1)};
+    }
+    __device__ __forceinline__ int sep(int v, int hv, int i, int hi, int H) const { return edt_sep_w(v, hv, i, hi, H, sy, sx); }
+    __device__ __forceinline__ uint32_t at(int dy, int h) const { return edt_pack(abs(dy), h); }
+    // the squared distance of offset (dy, dx) as scipy's distance_transform_edt(sampling=...) evaluates it
+    __device__ __forceinline__ double sq(uint32_t p) const {
+        return __dadd_rn(edt_sq1((int)(p & 0xFFFu), sy), edt_sq1((int)(p >> 12), sx));
+    }
+    __device__ __forceinline__ Key key(uint32_t p) const { return p == kEdtNone ? ~0ull : (Key)__double_as_longlong(sq(p)); }
+    __device__ __forceinline__ double key_sq(Key k) const { return __longlong_as_double((long long)k); }
+};
+
+// The lower envelope of one label over one column.  Entry k of the stack (row v_k, distance h_k, packed v | h << 16)
+// lives in the column's word of row k: when row i is pushed the stack holds at most i + 1 entries, and rows <= i have
+// been read, so the stack only overwrites consumed input.  The start z_k of entry k (the first u it is the minimum at;
+// z_0 = 0) is recomputed from entries k - 1 and k when it is needed.
+template <class Metric>
+struct EdtEnv {
     uint32_t* col;
     size_t stride;
-    int top, v, h, z;
-    EdtSpacing sp;
+    int top, v, h, z;  // top entry and its start; top = -1: empty
+    Metric m;
 
     __device__ __forceinline__ void load(int k, int& vk, int& hk) const {
         const uint32_t e = col[(size_t)k * stride];
@@ -247,15 +217,27 @@ struct EdtEnvW {
     __device__ __forceinline__ void put(int k, int vk, int hk) { col[(size_t)k * stride] = (uint32_t)vk | ((uint32_t)hk << 16); }
 
     __device__ __forceinline__ void push(int i, int hi, int H) {
-        const double bi = edt_sq1(hi, sp.sx);
         while (top >= 0) {
-            const double bv = edt_sq1(h, sp.sx);
-            if (!edt_beats(i, bi, v, bv, z, sp.sy)) {  // row i is above the top at its start: it starts later, if at all
-                if (edt_beats(i, bi, v, bv, H - 1, sp.sy)) {
-                    const int s = edt_sep_w(v, h, i, hi, H, sp);
-                    put(++top, i, hi); v = i; h = hi; z = s;
+            // Row i against the top: pushed from its start s if that is below H, skipped if it never is the
+            // minimum, or else the top is popped.  Written once per metric: folded into one metric method, the test
+            // cost either a spill in the unit signed-map kernel or about 1% of the weighted Hausdorff DT loss (B200).
+            if constexpr (std::is_same_v<Metric, EdtUnit>) {
+                const int s = edt_sep(v, h, i, hi);
+                if (s > z) {  // row i is the minimum from s on; past the last row it never is
+                    if (s < H) { put(++top, i, hi); v = i; h = hi; z = s; }
+                    return;
                 }
-                return;
+            } else {
+                // the pop test and the skip test are single comparisons at the top's start and at the last row; the
+                // separator (with its division) is only computed for an entry that is pushed
+                const double bi = edt_sq1(hi, m.sx), bv = edt_sq1(h, m.sx);
+                if (!edt_beats(i, bi, v, bv, z, m.sy)) {
+                    if (edt_beats(i, bi, v, bv, H - 1, m.sy)) {
+                        const int s = m.sep(v, h, i, hi, H);
+                        put(++top, i, hi); v = i; h = hi; z = s;
+                    }
+                    return;
+                }
             }
             if (--top >= 0) {  // row i is <= the top over the top's whole range: pop it
                 load(top, v, h);
@@ -264,7 +246,7 @@ struct EdtEnvW {
                 } else {
                     int pv, ph;
                     load(top - 1, pv, ph);
-                    z = edt_sep_w(pv, ph, v, h, H, sp);
+                    z = m.sep(pv, ph, v, h, H);
                 }
             }
         }
@@ -274,22 +256,23 @@ struct EdtEnvW {
     }
 };
 
-// Walks a weighted envelope top to bottom: the packed offset (|u - v|, h) of the nearest pixel for u = 0, 1, ..., H - 1
-struct EdtWalkW {
+// Walks an envelope top to bottom: the walk value of the nearest pixel for u = 0, 1, ..., H - 1 in that order.
+template <class Metric>
+struct EdtWalk {
     int k, top, v, h, nv, nh, znext, H;
-    __device__ __forceinline__ void start(const EdtEnvW& e, int H_) {
+    __device__ __forceinline__ void start(const EdtEnv<Metric>& e, int H_) {
         top = e.top; H = H_; k = 0;
         if (top < 0) return;
         e.load(0, v, h);
         znext = H;
-        if (top >= 1) { e.load(1, nv, nh); znext = edt_sep_w(v, h, nv, nh, H, e.sp); }
+        if (top >= 1) { e.load(1, nv, nh); znext = e.m.sep(v, h, nv, nh, H); }
     }
-    __device__ __forceinline__ uint32_t at(const EdtEnvW& e, int u) {
+    __device__ __forceinline__ auto at(const EdtEnv<Metric>& e, int u) {
         while (u >= znext) {
             ++k; v = nv; h = nh; znext = H;
-            if (k < top) { e.load(k + 1, nv, nh); znext = edt_sep_w(v, h, nv, nh, H, e.sp); }
+            if (k < top) { e.load(k + 1, nv, nh); znext = e.m.sep(v, h, nv, nh, H); }
         }
-        return edt_pack(abs(u - v), h);
+        return e.m.at(u - v, h);
     }
 };
 
@@ -311,31 +294,28 @@ struct EdtColArgs {
     const float* t;         // kEdtTarget: targets
     double half_alpha;
     float* cost;            // kEdtTarget, kEdtSigned with x: [n]
-    const double* spacing;  // kSp: [n][2] (sy, sx) per map
+    const double* spacing;  // EdtSpacing: [n][2] (sy, sx) per map
     double inv_hw;          // kEdtSigned with x: 1 / HW (a device fp64 division would bring a slow-path call that spills)
 };
 
-// kSp: the weighted envelope of the map's spacing; sp then holds the packed offset of P's nearest other-label pixel
-template <int Mode, bool kSp = false>
+// Metric: EdtUnit, or EdtSpacing of each map's spacing; sp then holds the packed offset of P's nearest other-label pixel
+template <int Mode, class Metric>
 __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
     constexpr int NL = Mode == kEdtField ? 1 : 2;
-    using Env = std::conditional_t<kSp, EdtEnvW, EdtEnv>;
-    using Walk = std::conditional_t<kSp, EdtWalkW, EdtWalk>;
     __shared__ double s_red[32];
     const int H = A.H, W = A.W;
     const size_t N = (size_t)H * W;
     for (int map = blockIdx.x; map < A.n_maps; map += gridDim.x) {
         double acc = 0.0;
-        EdtSpacing sp{};
-        if constexpr (kSp) sp = EdtSpacing{__ldg(A.spacing + 2 * map), __ldg(A.spacing + 2 * map + 1)};
+        const Metric m = Metric::of(A.spacing, map);
         for (int j = threadIdx.x; j < W; j += blockDim.x) {
-            Env env[NL];
+            EdtEnv<Metric> env[NL];
 #pragma unroll
             for (int L = 0; L < NL; ++L) {
                 env[L].col = A.h + ((size_t)map * N + j) * NL + L;
                 env[L].stride = (size_t)W * NL;
                 env[L].top = -1;
-                if constexpr (kSp) env[L].sp = sp;
+                env[L].m = m;
             }
             for (int i = 0; i < H; ++i) {
 #pragma unroll
@@ -344,21 +324,22 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                     if (hi != kEdtNone) env[L].push(i, (int)hi, H);
                 }
             }
-            Walk walk[NL];
+            EdtWalk<Metric> walk[NL];
 #pragma unroll
             for (int L = 0; L < NL; ++L) walk[L].start(env[L], H);
             const size_t o = (size_t)map * N + j;
             if (Mode == kEdtField) {
-                if constexpr (kSp) {
-                    if (env[0].top < 0) {
-                        for (int u = 0; u < H; ++u) A.field[o + (size_t)u * W] = __int_as_float(0x7F800000);
-                    } else {
-                        for (int u = 0; u < H; ++u) A.field[o + (size_t)u * W] = (float)sqrt(edt_packed_sq(walk[0].at(env[0], u), sp));
-                    }
-                } else {
+                // the same loop in two shapes, each the one that compiles tightest for its metric: testing the empty
+                // envelope per pixel takes EdtUnit fewer registers than hoisting the test, and hoisting it keeps
+                // EdtSpacing from spilling around sqrt's slow path
+                if constexpr (std::is_same_v<Metric, EdtUnit>) {
                     for (int u = 0; u < H; ++u)
                         A.field[o + (size_t)u * W] = env[0].top < 0 ? __int_as_float(0x7F800000)
-                                                                    : (float)sqrt((double)walk[0].at(env[0], u));
+                                                                    : (float)sqrt(m.sq(walk[0].at(env[0], u)));
+                } else if (env[0].top < 0) {
+                    for (int u = 0; u < H; ++u) A.field[o + (size_t)u * W] = __int_as_float(0x7F800000);
+                } else {
+                    for (int u = 0; u < H; ++u) A.field[o + (size_t)u * W] = (float)sqrt(m.sq(walk[0].at(env[0], u)));
                 }
             } else if constexpr (Mode == kEdtSigned) {
                 // label 0 is the background: on a mixed map s1 == 0 exactly on the foreground, where phi = 1 - d_in
@@ -368,12 +349,9 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                 for (int u = 0; u < H; ++u) {
                     const size_t q = o + (size_t)u * W;
                     float phi = 0.f;
-                    if (mixed) {  // s (or the packed offset) is 0 exactly at the label's own pixels
+                    if (mixed) {  // the walk value is 0 exactly at the label's own pixels
                         const auto e0 = walk[0].at(env[0], u), e1 = walk[1].at(env[1], u);
-                        const auto e = e1 == 0 ? e0 : e1;
-                        double d;
-                        if constexpr (kSp) d = sqrt(edt_packed_sq(e, sp));
-                        else d = sqrt((double)e);
+                        const double d = sqrt(m.sq(e1 == 0 ? e0 : e1));
                         phi = (float)(e1 == 0 ? __dsub_rn(1.0, d) : d);
                     }
                     A.field[q] = phi;
@@ -388,12 +366,7 @@ __global__ void __launch_bounds__(kEdtColThreads) edt_col_kernel(EdtColArgs A) {
                     if (Mode == kEdtPred) {
                         A.sp[q] = s;
                     } else {
-                        double d;
-                        if constexpr (kSp)
-                            d = edt_pow(edt_packed_sq((uint32_t)A.sp[q], sp), A.half_alpha) +
-                                edt_pow(edt_packed_sq((uint32_t)s, sp), A.half_alpha);
-                        else
-                            d = edt_pow(A.sp[q], A.half_alpha) + edt_pow(s, A.half_alpha);
+                        const double d = edt_pow(m.sq(A.sp[q]), A.half_alpha) + edt_pow(m.sq(s), A.half_alpha);
                         const double p = (double)edt_sigmoid(__ldg(A.x + q)), diff = p - (double)__ldg(A.t + q);
                         acc += diff * diff * d;
                         A.D[q] = (float)d;

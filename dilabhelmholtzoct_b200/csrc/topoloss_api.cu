@@ -1210,9 +1210,54 @@ int edt_shape(int n_maps, int H, int W) {
     return TL_OK;
 }
 
-// STATE: D = F(P)^alpha + F(T)^alpha, fp32 per pixel (the backward reads it); SCRATCH: the row pass's h0 / h1 of one
-// mask, a uint2 per pixel (P, then T)
 size_t edt_pixels(int n_maps, int H, int W) { return (size_t)n_maps * H * W; }
+
+// The buffers of both losses (tl_hausdorff_dt_*, tl_boundary_*).  STATE: fp32 per pixel, D or phi, written by the
+// forward and read by the backward; SCRATCH: the row pass's h0 / h1 of one mask, a uint2 per pixel
+struct LossBytes {
+    size_t state, scratch;
+};
+
+LossBytes loss_bytes(int n_maps, int H, int W) {
+    return {align_up(sizeof(float) * edt_pixels(n_maps, H, W)), align_up(sizeof(uint2) * edt_pixels(n_maps, H, W))};
+}
+
+int loss_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes) {
+    if (!state_bytes || !scratch_bytes) return fail(TL_ERR_ARG, "null pointer");
+    const int rc = edt_shape(n_maps, H, W);
+    if (rc != TL_OK) return rc;
+    const LossBytes b = loss_bytes(n_maps, H, W);
+    *state_bytes = b.state;
+    *scratch_bytes = b.scratch;
+    return TL_OK;
+}
+
+// the forward's state and scratch against loss_bytes; query names the workspace query in the message
+int loss_buffers(int n_maps, int H, int W, const void* state, size_t state_bytes, const void* scratch,
+                 size_t scratch_bytes, const char* query) {
+    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
+        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
+    const LossBytes b = loss_bytes(n_maps, H, W);
+    if (state_bytes < b.state) return fail(TL_ERR_ARG, "state %zu < %zu bytes (%s)", state_bytes, b.state, query);
+    if (scratch_bytes < b.scratch) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (%s)", scratch_bytes, b.scratch, query);
+    return TL_OK;
+}
+
+// the backward's state against loss_bytes
+int loss_state(int n_maps, int H, int W, const void* state, size_t state_bytes, const char* query) {
+    if (reinterpret_cast<uintptr_t>(state) & 3) return fail(TL_ERR_ARG, "state must be 4-byte aligned");
+    const size_t ns = loss_bytes(n_maps, H, W).state;
+    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (%s)", state_bytes, ns, query);
+    return TL_OK;
+}
+
+// The one place a distance entry point chooses its path: a null spacing is unit spacing through the integer envelope
+// (op(tl::EdtUnit)), anything else a device fp64 [n][2] spacing through the weighted one (op(tl::EdtSpacing)).
+template <class Op>
+int by_spacing(const double* spacing, Op op) {
+    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
+    return spacing ? op(tl::EdtSpacing{}) : op(tl::EdtUnit{});
+}
 
 int edt_grid(long long work, int per_block) {
     const long long b = (work + per_block - 1) / per_block;
@@ -1227,15 +1272,14 @@ int edt_rows(Src src, int n_maps, int H, int W, uint32_t* h, cudaStream_t st) {
     return TL_OK;
 }
 
-template <int Mode, bool kSp = false>
+template <int Mode, class Metric>
 int edt_cols(const tl::EdtColArgs& a, cudaStream_t st) {
-    tl::edt_col_kernel<Mode, kSp><<<a.n_maps < (1 << 20) ? a.n_maps : (1 << 20), tl::kEdtColThreads, 0, st>>>(a);
+    tl::edt_col_kernel<Mode, Metric><<<a.n_maps < (1 << 20) ? a.n_maps : (1 << 20), tl::kEdtColThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }
 
-// tl_edt and tl_edt_spaced (kSp: spacing is a device [n][2] array, checked non-null by the caller)
-template <bool kSp>
+template <class Metric>
 int edt_field(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes,
               float* out, void* stream) {
     int rc = edt_shape(n_maps, H, W);
@@ -1250,11 +1294,10 @@ int edt_field(const uint8_t* mask, int n_maps, int H, int W, const double* spaci
     if (rc != TL_OK) return rc;
     tl::EdtColArgs a = {};
     a.h = h; a.n_maps = n_maps; a.H = H; a.W = W; a.field = out; a.spacing = spacing;
-    return edt_cols<tl::kEdtField, kSp>(a, st);
+    return edt_cols<tl::kEdtField, Metric>(a, st);
 }
 
-// tl_hausdorff_dt_forward and its _spaced form
-template <bool kSp>
+template <class Metric>
 int hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
                          const double* spacing, void* state, size_t state_bytes, void* scratch, size_t scratch_bytes,
                          float* cost, void* stream) {
@@ -1262,20 +1305,17 @@ int hausdorff_dt_forward(const float* logits, const float* target, int n_maps, i
     if (rc != TL_OK) return rc;
     if (!logits || !target || !state || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
     if (!(alpha > 0.0) || !(alpha < HUGE_VAL)) return fail(TL_ERR_ARG, "alpha must be finite and positive, got %g", alpha);
-    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
-        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
-    const size_t ns = align_up(sizeof(float) * edt_pixels(n_maps, H, W)), nc = align_up(sizeof(uint2) * edt_pixels(n_maps, H, W));
-    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", state_bytes, ns);
-    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", scratch_bytes, nc);
+    rc = loss_buffers(n_maps, H, W, state, state_bytes, scratch, scratch_bytes, "tl_hausdorff_dt_workspace_bytes");
+    if (rc != TL_OK) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     tl::EdtColArgs a = {};
     a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W;
     a.sp = static_cast<int32_t*>(state); a.D = static_cast<float*>(state);
     a.x = logits; a.t = target; a.half_alpha = 0.5 * alpha; a.cost = cost; a.spacing = spacing;
     rc = edt_rows<tl::EdtLogitSrc, 2>(tl::EdtLogitSrc{logits}, n_maps, H, W, a.h, st);
-    if (rc == TL_OK) rc = edt_cols<tl::kEdtPred, kSp>(a, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtPred, Metric>(a, st);
     if (rc == TL_OK) rc = edt_rows<tl::EdtTargetSrc, 2>(tl::EdtTargetSrc{target}, n_maps, H, W, a.h, st);
-    if (rc == TL_OK) rc = edt_cols<tl::kEdtTarget, kSp>(a, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtTarget, Metric>(a, st);
     return rc;
 }
 
@@ -1291,40 +1331,24 @@ int tl_edt_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
     return TL_OK;
 }
 
-int tl_edt(const uint8_t* mask, int n_maps, int H, int W, void* ws, size_t ws_bytes, float* out, void* stream) {
-    return edt_field<false>(mask, n_maps, H, W, nullptr, ws, ws_bytes, out, stream);
-}
-
-int tl_edt_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes,
-                  float* out, void* stream) {
-    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
-    return edt_field<true>(mask, n_maps, H, W, spacing, ws, ws_bytes, out, stream);
+int tl_edt(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes, float* out,
+           void* stream) {
+    return by_spacing(spacing, [&](auto m) {
+        return edt_field<decltype(m)>(mask, n_maps, H, W, spacing, ws, ws_bytes, out, stream);
+    });
 }
 
 int tl_hausdorff_dt_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes) {
-    if (!state_bytes || !scratch_bytes) return fail(TL_ERR_ARG, "null pointer");
-    int rc = edt_shape(n_maps, H, W);
-    if (rc != TL_OK) return rc;
-    *state_bytes = align_up(sizeof(float) * edt_pixels(n_maps, H, W));
-    *scratch_bytes = align_up(sizeof(uint2) * edt_pixels(n_maps, H, W));
-    return TL_OK;
+    return loss_workspace_bytes(n_maps, H, W, state_bytes, scratch_bytes);
 }
 
 int tl_hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
-                            void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
-                            void* stream) {
-    return hausdorff_dt_forward<false>(logits, target, n_maps, H, W, alpha, nullptr, state, state_bytes, scratch,
-                                       scratch_bytes, cost, stream);
-}
-
-int tl_hausdorff_dt_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
-                                   const double* spacing, void* state, size_t state_bytes, void* scratch,
-                                   size_t scratch_bytes, float* cost, void* stream) {
-    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
-    return hausdorff_dt_forward<true>(logits, target, n_maps, H, W, alpha, spacing, state, state_bytes, scratch,
-                                      scratch_bytes, cost, stream);
+                            const double* spacing, void* state, size_t state_bytes, void* scratch,
+                            size_t scratch_bytes, float* cost, void* stream) {
+    return by_spacing(spacing, [&](auto m) {
+        return hausdorff_dt_forward<decltype(m)>(logits, target, n_maps, H, W, alpha, spacing, state, state_bytes,
+                                                 scratch, scratch_bytes, cost, stream);
+    });
 }
 
 int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_maps, int H, int W, const void* state,
@@ -1332,9 +1356,8 @@ int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_map
     int rc = edt_shape(n_maps, H, W);
     if (rc != TL_OK) return rc;
     if (!logits || !target || !state || !grad_cost || !grad_logits) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(state) & 3) return fail(TL_ERR_ARG, "state must be 4-byte aligned");
-    const size_t ns = align_up(sizeof(float) * edt_pixels(n_maps, H, W));
-    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_hausdorff_dt_workspace_bytes)", state_bytes, ns);
+    rc = loss_state(n_maps, H, W, state, state_bytes, "tl_hausdorff_dt_workspace_bytes");
+    if (rc != TL_OK) return rc;
     const long long N = (long long)H * W;
     tl::hausdorff_dt_backward_kernel<<<edt_grid((long long)n_maps * ((N + 1023) / 1024), 1), 256, 0,
                                        static_cast<cudaStream_t>(stream)>>>(
@@ -1362,7 +1385,7 @@ SurfLayout surface_layout(int n_maps, int H, int W) {
     return L;
 }
 
-template <bool kSp>
+template <class Metric>
 int surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, const double* spacing,
                       double percentile, double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
     int rc = edt_shape(n_maps, H, W);
@@ -1385,9 +1408,9 @@ int surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, in
     if (rc == TL_OK) rc = edt_rows<tl::SurfSrc, 1>(tl::SurfSrc{target, H, W}, n_maps, H, W, a.h + edt_pixels(n_maps, H, W), st);
     if (rc != TL_OK) return rc;
     const int grid = n_maps < (1 << 20) ? n_maps : (1 << 20);
-    tl::surface_col_kernel<kSp><<<grid, tl::kEdtColThreads, 0, st>>>(a);
+    tl::surface_col_kernel<Metric><<<grid, tl::kEdtColThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
-    tl::surface_select_kernel<kSp><<<grid, tl::kSurfSelThreads, 0, st>>>(a);
+    tl::surface_select_kernel<Metric><<<grid, tl::kSurfSelThreads, 0, st>>>(a);
     TL_CUDA(cudaGetLastError());
     return TL_OK;
 }
@@ -1404,71 +1427,51 @@ int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes) {
     return TL_OK;
 }
 
-int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
-                         double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
-    return surface_distances<false>(pred, target, n_maps, H, W, nullptr, percentile, tolerance, ws, ws_bytes, out, stream);
-}
-
-int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W,
-                                const double* spacing, double percentile, double tolerance, void* ws, size_t ws_bytes,
-                                float* out, void* stream) {
-    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
-    return surface_distances<true>(pred, target, n_maps, H, W, spacing, percentile, tolerance, ws, ws_bytes, out, stream);
+int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, const double* spacing,
+                         double percentile, double tolerance, void* ws, size_t ws_bytes, float* out, void* stream) {
+    return by_spacing(spacing, [&](auto m) {
+        return surface_distances<decltype(m)>(pred, target, n_maps, H, W, spacing, percentile, tolerance, ws, ws_bytes,
+                                              out, stream);
+    });
 }
 
 }  // extern "C"
 
-// ---- the signed distance map (tl_signed_distance*) and the boundary loss (tl_boundary_*), DESIGN §3.11
+// ---- the signed distance map (tl_signed_distance) and the boundary loss (tl_boundary_*), DESIGN §3.11
 namespace {
 
-// STATE: phi, fp32 per pixel (the backward reads it); SCRATCH: the row pass's h0 / h1, a uint2 per pixel
-size_t boundary_state_bytes(int n_maps, int H, int W) { return align_up(sizeof(float) * edt_pixels(n_maps, H, W)); }
-size_t boundary_scratch_bytes(int n_maps, int H, int W) { return align_up(sizeof(uint2) * edt_pixels(n_maps, H, W)); }
-
-int spacing_ok(const double* spacing) {
-    if (!spacing) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(spacing) & 7) return fail(TL_ERR_ARG, "spacing must be 8-byte aligned");
-    return TL_OK;
-}
-
-// tl_signed_distance and its _spaced form (kSp: spacing checked by the caller)
-template <bool kSp>
+template <class Metric>
 int signed_distance(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
                     size_t scratch_bytes, float* out, void* stream) {
     int rc = edt_shape(n_maps, H, W);
     if (rc != TL_OK) return rc;
     if (!mask || !scratch || !out) return fail(TL_ERR_ARG, "null pointer");
     if (reinterpret_cast<uintptr_t>(scratch) & 7) return fail(TL_ERR_ARG, "scratch must be 8-byte aligned");
-    const size_t nc = boundary_scratch_bytes(n_maps, H, W);
+    const size_t nc = loss_bytes(n_maps, H, W).scratch;
     if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_boundary_workspace_bytes)", scratch_bytes, nc);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     tl::EdtColArgs a = {};
     a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W; a.field = out; a.spacing = spacing;
     rc = edt_rows<tl::EdtMaskSrc, 2>(tl::EdtMaskSrc{mask}, n_maps, H, W, a.h, st);
-    if (rc == TL_OK) rc = edt_cols<tl::kEdtSigned, kSp>(a, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtSigned, Metric>(a, st);
     return rc;
 }
 
-// tl_boundary_forward and its _spaced form
-template <bool kSp>
+template <class Metric>
 int boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, const double* spacing,
                      void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream) {
     int rc = edt_shape(n_maps, H, W);
     if (rc != TL_OK) return rc;
     if (!logits || !target || !state || !scratch || !cost) return fail(TL_ERR_ARG, "null pointer");
-    if ((reinterpret_cast<uintptr_t>(state) & 3) || (reinterpret_cast<uintptr_t>(scratch) & 7))
-        return fail(TL_ERR_ARG, "state must be 4-byte and scratch 8-byte aligned");
-    const size_t ns = boundary_state_bytes(n_maps, H, W), nc = boundary_scratch_bytes(n_maps, H, W);
-    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_boundary_workspace_bytes)", state_bytes, ns);
-    if (scratch_bytes < nc) return fail(TL_ERR_ARG, "scratch %zu < %zu bytes (tl_boundary_workspace_bytes)", scratch_bytes, nc);
+    rc = loss_buffers(n_maps, H, W, state, state_bytes, scratch, scratch_bytes, "tl_boundary_workspace_bytes");
+    if (rc != TL_OK) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     tl::EdtColArgs a = {};
     a.h = static_cast<uint32_t*>(scratch); a.n_maps = n_maps; a.H = H; a.W = W;
     a.field = static_cast<float*>(state); a.x = logits; a.cost = cost; a.spacing = spacing;
     a.inv_hw = 1.0 / ((double)H * W);
     rc = edt_rows<tl::EdtTargetSrc, 2>(tl::EdtTargetSrc{target}, n_maps, H, W, a.h, st);
-    if (rc == TL_OK) rc = edt_cols<tl::kEdtSigned, kSp>(a, st);
+    if (rc == TL_OK) rc = edt_cols<tl::kEdtSigned, Metric>(a, st);
     return rc;
 }
 
@@ -1477,39 +1480,23 @@ int boundary_forward(const float* logits, const float* target, int n_maps, int H
 extern "C" {
 
 int tl_boundary_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes) {
-    if (!state_bytes || !scratch_bytes) return fail(TL_ERR_ARG, "null pointer");
-    int rc = edt_shape(n_maps, H, W);
-    if (rc != TL_OK) return rc;
-    *state_bytes = boundary_state_bytes(n_maps, H, W);
-    *scratch_bytes = boundary_scratch_bytes(n_maps, H, W);
-    return TL_OK;
+    return loss_workspace_bytes(n_maps, H, W, state_bytes, scratch_bytes);
 }
 
-int tl_signed_distance(const uint8_t* mask, int n_maps, int H, int W, void* scratch, size_t scratch_bytes, float* out,
-                       void* stream) {
-    return signed_distance<false>(mask, n_maps, H, W, nullptr, scratch, scratch_bytes, out, stream);
+int tl_signed_distance(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
+                       size_t scratch_bytes, float* out, void* stream) {
+    return by_spacing(spacing, [&](auto m) {
+        return signed_distance<decltype(m)>(mask, n_maps, H, W, spacing, scratch, scratch_bytes, out, stream);
+    });
 }
 
-int tl_signed_distance_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
-                              size_t scratch_bytes, float* out, void* stream) {
-    const int rc = spacing_ok(spacing);
-    if (rc != TL_OK) return rc;
-    return signed_distance<true>(mask, n_maps, H, W, spacing, scratch, scratch_bytes, out, stream);
-}
-
-int tl_boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, void* state,
-                        size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream) {
-    return boundary_forward<false>(logits, target, n_maps, H, W, nullptr, state, state_bytes, scratch, scratch_bytes,
-                                   cost, stream);
-}
-
-int tl_boundary_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W,
-                               const double* spacing, void* state, size_t state_bytes, void* scratch,
-                               size_t scratch_bytes, float* cost, void* stream) {
-    const int rc = spacing_ok(spacing);
-    if (rc != TL_OK) return rc;
-    return boundary_forward<true>(logits, target, n_maps, H, W, spacing, state, state_bytes, scratch, scratch_bytes,
-                                  cost, stream);
+int tl_boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, const double* spacing,
+                        void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
+                        void* stream) {
+    return by_spacing(spacing, [&](auto m) {
+        return boundary_forward<decltype(m)>(logits, target, n_maps, H, W, spacing, state, state_bytes, scratch,
+                                             scratch_bytes, cost, stream);
+    });
 }
 
 int tl_boundary_backward(const float* logits, int n_maps, int H, int W, const void* state, size_t state_bytes,
@@ -1517,9 +1504,8 @@ int tl_boundary_backward(const float* logits, int n_maps, int H, int W, const vo
     int rc = edt_shape(n_maps, H, W);
     if (rc != TL_OK) return rc;
     if (!logits || !state || !grad_cost || !grad_logits) return fail(TL_ERR_ARG, "null pointer");
-    if (reinterpret_cast<uintptr_t>(state) & 3) return fail(TL_ERR_ARG, "state must be 4-byte aligned");
-    const size_t ns = boundary_state_bytes(n_maps, H, W);
-    if (state_bytes < ns) return fail(TL_ERR_ARG, "state %zu < %zu bytes (tl_boundary_workspace_bytes)", state_bytes, ns);
+    rc = loss_state(n_maps, H, W, state, state_bytes, "tl_boundary_workspace_bytes");
+    if (rc != TL_OK) return rc;
     const long long N = (long long)H * W;
     tl::boundary_backward_kernel<<<edt_grid((long long)n_maps * ((N + 1023) / 1024), 1), 256, 0,
                                    static_cast<cudaStream_t>(stream)>>>(logits, static_cast<const float*>(state),

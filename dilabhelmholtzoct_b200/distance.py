@@ -11,8 +11,8 @@ the signed distance map of Kervadec et al.'s boundary loss, and ``boundary_loss(
 logits (``tl_signed_distance``, ``tl_boundary_*``, DESIGN §3.11).
 
 All of them measure in pixels by default.  Given a physical pixel spacing (``sampling=`` for the transform, as scipy
-names it; ``spacing=`` for the loss and the metrics, as monai names it) they measure in its units instead, through
-the ``tl_*_spaced`` entry points (DESIGN §3.10).
+names it; ``spacing=`` for the loss and the metrics, as monai names it) they measure in its units instead (DESIGN
+§3.10).
 
 There is no CPU path: the inputs must be CUDA tensors.
 """
@@ -34,9 +34,47 @@ MAX_DIM = 4096
 SPACING_MIN, SPACING_MAX = 1e-6, 1e6
 
 
-def _check_hw(H: int, W: int, what: str) -> None:
+def _check_hw(shape: torch.Size, what: str) -> tuple[int, int, int]:
+    """The number of ``[H, W]`` maps of ``shape`` and H and W, which must each be in [1, MAX_DIM]."""
+    H, W = int(shape[-2]), int(shape[-1])
     if not (1 <= H <= MAX_DIM and 1 <= W <= MAX_DIM):
         raise ValueError(f"{what}: H and W must each be in [1, {MAX_DIM}], got {H} x {W}")
+    return math.prod(int(d) for d in shape[:-2]), H, W
+
+
+def _mask_maps(mask, what: str, name: str = "mask") -> torch.Tensor:
+    """Checks ``mask`` as ``[..., H, W]`` maps in a bool or uint8 CUDA tensor; returns its contiguous uint8 view."""
+    if not torch.is_tensor(mask):
+        raise TypeError(f"{name} must be a tensor")
+    if mask.dim() < 2:
+        raise ValueError(f"{what} expects [..., H, W] maps")
+    if not mask.is_cuda:
+        raise ValueError(f"{what} runs on a CUDA device only: there is no CPU fallback")
+    if mask.dtype not in (torch.bool, torch.uint8):
+        raise ValueError(f"{what} expects a bool or uint8 {name}, got {mask.dtype}")
+    m = mask.detach().contiguous()
+    return m.view(torch.uint8) if m.dtype == torch.bool else m
+
+
+def _logits_and_target(masks, gt_masks, what: str) -> None:
+    """Checks float32 logits ``masks`` and a real or bool ``gt_masks``, both ``[B, C, H, W]`` on the same CUDA device."""
+    if not (torch.is_tensor(masks) and torch.is_tensor(gt_masks)):
+        raise TypeError("masks and gt_masks must be tensors")
+    if masks.dim() != 4 or masks.shape != gt_masks.shape:
+        raise ValueError("expected two [B, C, H, W] tensors of the same shape")
+    if not masks.is_cuda or not gt_masks.is_cuda:
+        raise ValueError(f"{what} runs on a CUDA device only: there is no CPU fallback")
+    if masks.device != gt_masks.device:
+        raise ValueError(f"masks are on {masks.device}, gt_masks on {gt_masks.device}")
+    if masks.dtype != torch.float32:
+        raise ValueError(f"{what} expects float32 logits, got {masks.dtype}")
+    if gt_masks.dtype.is_complex:
+        raise ValueError(f"{what} expects a real or bool gt_masks, got {gt_masks.dtype}")
+
+
+def _ptr(t: torch.Tensor | None) -> int | None:
+    """A device pointer for the library, or None (NULL) for no tensor: a spacing of None is unit spacing."""
+    return None if t is None else t.data_ptr()
 
 
 def _spacing_tensor(spacing, lead: torch.Size, dev: torch.device, what: str) -> torch.Tensor:
@@ -120,36 +158,25 @@ def surface_distances(pred: torch.Tensor, target: torch.Tensor, percentile: floa
         raise ValueError("surface_distances runs on a CUDA device only: there is no CPU fallback")
     if pred.device != target.device:
         raise ValueError(f"pred is on {pred.device}, target on {target.device}")
-    for name, m in (("pred", pred), ("target", target)):
-        if m.dtype not in (torch.bool, torch.uint8):
-            raise ValueError(f"surface_distances expects a bool or uint8 {name}, got {m.dtype}")
+    p, t = (_mask_maps(m, "surface_distances", name) for name, m in (("pred", pred), ("target", target)))
     percentile, tolerance = float(percentile), float(tolerance)
     if not 0.0 <= percentile <= 100.0:
         raise ValueError(f"percentile must be in [0, 100], got {percentile}")
     if not (math.isfinite(tolerance) and tolerance >= 0.0):
         raise ValueError(f"tolerance must be finite and >= 0, got {tolerance}")
-    H, W = int(pred.shape[-2]), int(pred.shape[-1])
-    _check_hw(H, W, "surface_distances")
-    n = pred.numel() // (H * W)
+    n, H, W = _check_hw(pred.shape, "surface_distances")
     dev = pred.device
     out = torch.empty((4, n), dtype=torch.float32, device=dev)
     sp = None if spacing is None else _spacing_tensor(spacing, pred.shape[:-2], dev, "surface_distances")
     if n > 0:
-        p, t = (m.detach().contiguous() for m in (pred, target))
-        p, t = (m.view(torch.uint8) if m.dtype == torch.bool else m for m in (p, t))
         L = _lib.lib()
         nb = ctypes.c_size_t(0)
         _lib.check(L.tl_surface_workspace_bytes(n, H, W, ctypes.byref(nb)), "tl_surface_workspace_bytes")
         with torch.cuda.device(dev):
             ws = torch.empty(nb.value, dtype=torch.uint8, device=dev)  # per call: released to the caching allocator
-            if sp is None:
-                rc = L.tl_surface_distances(p.data_ptr(), t.data_ptr(), n, H, W, percentile, tolerance, ws.data_ptr(),
-                                            ws.numel(), out.data_ptr(), _stream_ptr(dev))
-            else:
-                rc = L.tl_surface_distances_spaced(p.data_ptr(), t.data_ptr(), n, H, W, sp.data_ptr(), percentile,
-                                                   tolerance, ws.data_ptr(), ws.numel(), out.data_ptr(),
-                                                   _stream_ptr(dev))
-        _lib.check(rc, "tl_surface_distances" if sp is None else "tl_surface_distances_spaced")
+            rc = L.tl_surface_distances(p.data_ptr(), t.data_ptr(), n, H, W, _ptr(sp), percentile, tolerance,
+                                        ws.data_ptr(), ws.numel(), out.data_ptr(), _stream_ptr(dev))
+        _lib.check(rc, "tl_surface_distances")
     lead = pred.shape[:-2]
     return SurfaceDistances(*(o.view(lead) for o in out))
 
@@ -173,62 +200,46 @@ def distance_transform_edt(mask: torch.Tensor, sampling=None) -> torch.Tensor:
     ``scipy.ndimage.distance_transform_edt(m, sampling=sampling).astype(np.float32)`` bit for bit.  A map without a
     zero pixel gets ``+inf``.  Values must be finite and in [1e-6, 1e6] (checked on the host; ``ValueError``
     otherwise).  ``None`` (the default) is unit spacing through the integer path."""
-    if not torch.is_tensor(mask):
-        raise TypeError("mask must be a tensor")
-    if mask.dim() < 2:
-        raise ValueError("distance_transform_edt expects [..., H, W] maps")
-    if not mask.is_cuda:
-        raise ValueError("distance_transform_edt runs on a CUDA device only: there is no CPU fallback")
-    if mask.dtype not in (torch.bool, torch.uint8):
-        raise ValueError(f"distance_transform_edt expects a bool or uint8 mask, got {mask.dtype}")
-    H, W = int(mask.shape[-2]), int(mask.shape[-1])
-    _check_hw(H, W, "distance_transform_edt")
-    n = mask.numel() // (H * W)
+    m = _mask_maps(mask, "distance_transform_edt")
+    n, H, W = _check_hw(mask.shape, "distance_transform_edt")
     dev = mask.device
     out = torch.empty(mask.shape, dtype=torch.float32, device=dev)
     sp = None if sampling is None else _spacing_tensor(sampling, mask.shape[:-2], dev, "distance_transform_edt")
     if n == 0:
         return out
-    m = mask.detach().contiguous()
-    if m.dtype == torch.bool:
-        m = m.view(torch.uint8)
     L = _lib.lib()
     nb = ctypes.c_size_t(0)
     _lib.check(L.tl_edt_workspace_bytes(n, H, W, ctypes.byref(nb)), "tl_edt_workspace_bytes")
     with torch.cuda.device(dev):
         ws = torch.empty(nb.value, dtype=torch.uint8, device=dev)  # per call: released to the caching allocator
-        if sp is None:
-            rc = L.tl_edt(m.data_ptr(), n, H, W, ws.data_ptr(), ws.numel(), out.data_ptr(), _stream_ptr(dev))
-        else:
-            rc = L.tl_edt_spaced(m.data_ptr(), n, H, W, sp.data_ptr(), ws.data_ptr(), ws.numel(), out.data_ptr(),
-                                 _stream_ptr(dev))
-    _lib.check(rc, "tl_edt" if sp is None else "tl_edt_spaced")
+        rc = L.tl_edt(m.data_ptr(), n, H, W, _ptr(sp), ws.data_ptr(), ws.numel(), out.data_ptr(), _stream_ptr(dev))
+    _lib.check(rc, "tl_edt")
     return out
+
+
+def _loss_forward(name: str, query: str, x: torch.Tensor, t: torch.Tensor, *args) -> tuple[torch.Tensor, torch.Tensor]:
+    """Runs the forward entry point ``name`` (``logits, target, n, H, W, *args, state, ..., cost, stream``) with the
+    buffers the workspace query ``query`` asks for; returns the cost ``[B, C]`` and the state the backward reads."""
+    B, C, H, W = (int(d) for d in x.shape)
+    n = B * C
+    dev = x.device
+    L = _lib.lib()
+    ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
+    _lib.check(getattr(L, query)(n, H, W, ctypes.byref(ns), ctypes.byref(nc)), query)
+    with torch.cuda.device(dev):
+        state = torch.empty(ns.value, dtype=torch.uint8, device=dev)  # per pixel: the backward reads it
+        scratch = torch.empty(nc.value, dtype=torch.uint8, device=dev)  # per call, freed when the forward returns
+        cost = torch.empty((B, C), dtype=torch.float32, device=dev)
+        rc = getattr(L, name)(x.data_ptr(), t.data_ptr(), n, H, W, *args, state.data_ptr(), state.numel(),
+                              scratch.data_ptr(), scratch.numel(), cost.data_ptr(), _stream_ptr(dev))
+    _lib.check(rc, name)
+    return cost, state
 
 
 class _HausdorffDtFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, t, alpha, sp):
-        B, C, H, W = (int(d) for d in x.shape)
-        n = B * C
-        dev = x.device
-        L = _lib.lib()
-        ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
-        _lib.check(L.tl_hausdorff_dt_workspace_bytes(n, H, W, ctypes.byref(ns), ctypes.byref(nc)),
-                   "tl_hausdorff_dt_workspace_bytes")
-        with torch.cuda.device(dev):
-            state = torch.empty(ns.value, dtype=torch.uint8, device=dev)  # D per pixel: the backward reads it
-            scratch = torch.empty(nc.value, dtype=torch.uint8, device=dev)  # per call, freed when the forward returns
-            cost = torch.empty((B, C), dtype=torch.float32, device=dev)
-            if sp is None:
-                rc = L.tl_hausdorff_dt_forward(x.data_ptr(), t.data_ptr(), n, H, W, alpha, state.data_ptr(),
-                                               state.numel(), scratch.data_ptr(), scratch.numel(), cost.data_ptr(),
-                                               _stream_ptr(dev))
-            else:
-                rc = L.tl_hausdorff_dt_forward_spaced(x.data_ptr(), t.data_ptr(), n, H, W, alpha, sp.data_ptr(),
-                                                      state.data_ptr(), state.numel(), scratch.data_ptr(),
-                                                      scratch.numel(), cost.data_ptr(), _stream_ptr(dev))
-        _lib.check(rc, "tl_hausdorff_dt_forward" if sp is None else "tl_hausdorff_dt_forward_spaced")
+        cost, state = _loss_forward("tl_hausdorff_dt_forward", "tl_hausdorff_dt_workspace_bytes", x, t, alpha, _ptr(sp))
         ctx.save_for_backward(x, t, state)
         return cost
 
@@ -277,25 +288,13 @@ def hausdorff_dt_loss(masks: torch.Tensor, gt_masks: torch.Tensor, alpha: float 
     Neither the forward nor the backward synchronises the host.  The forward keeps D (4 bytes per pixel) for the
     backward, and takes 8 bytes per pixel of scratch from PyTorch's caching allocator for the duration of the call
     (about 1.8 GB at 64 x 14 x 496 x 512); nothing is kept between calls."""
-    if not (torch.is_tensor(masks) and torch.is_tensor(gt_masks)):
-        raise TypeError("masks and gt_masks must be tensors")
-    if masks.dim() != 4 or masks.shape != gt_masks.shape:
-        raise ValueError("expected two [B, C, H, W] tensors of the same shape")
-    if not masks.is_cuda or not gt_masks.is_cuda:
-        raise ValueError("hausdorff_dt_loss runs on a CUDA device only: there is no CPU fallback")
-    if masks.device != gt_masks.device:
-        raise ValueError(f"masks are on {masks.device}, gt_masks on {gt_masks.device}")
-    if masks.dtype != torch.float32:
-        raise ValueError(f"hausdorff_dt_loss expects float32 logits, got {masks.dtype}")
-    if gt_masks.dtype.is_complex:
-        raise ValueError(f"hausdorff_dt_loss expects a real or bool gt_masks, got {gt_masks.dtype}")
+    _logits_and_target(masks, gt_masks, "hausdorff_dt_loss")
     alpha = float(alpha)
     if not (math.isfinite(alpha) and alpha > 0.0):
         raise ValueError(f"alpha must be finite and > 0, got {alpha}")
-    B, C, H, W = (int(d) for d in masks.shape)
-    _check_hw(H, W, "hausdorff_dt_loss")
+    n, _, _ = _check_hw(masks.shape, "hausdorff_dt_loss")
     sp = None if spacing is None else _spacing_tensor(spacing, masks.shape[:2], masks.device, "hausdorff_dt_loss")
-    if B * C == 0:
+    if n == 0:
         return masks.sum((2, 3))  # empty, still attached to autograd
     return _HausdorffDtFn.apply(masks.contiguous(), gt_masks.detach().to(torch.float32).contiguous(), alpha, sp)
 
@@ -323,62 +322,28 @@ def signed_distance_map(mask: torch.Tensor, sampling=None) -> torch.Tensor:
     (the default) is unit spacing through the integer path.  H and W must each be in [1, 4096].  No host
     synchronisation; 8 bytes per pixel of scratch are taken from PyTorch's caching allocator for the duration of the
     call."""
-    if not torch.is_tensor(mask):
-        raise TypeError("mask must be a tensor")
-    if mask.dim() < 2:
-        raise ValueError("signed_distance_map expects [..., H, W] maps")
-    if not mask.is_cuda:
-        raise ValueError("signed_distance_map runs on a CUDA device only: there is no CPU fallback")
-    if mask.dtype not in (torch.bool, torch.uint8):
-        raise ValueError(f"signed_distance_map expects a bool or uint8 mask, got {mask.dtype}")
-    H, W = int(mask.shape[-2]), int(mask.shape[-1])
-    _check_hw(H, W, "signed_distance_map")
-    n = mask.numel() // (H * W)
+    m = _mask_maps(mask, "signed_distance_map")
+    n, H, W = _check_hw(mask.shape, "signed_distance_map")
     dev = mask.device
     out = torch.empty(mask.shape, dtype=torch.float32, device=dev)
     sp = None if sampling is None else _spacing_tensor(sampling, mask.shape[:-2], dev, "signed_distance_map")
     if n == 0:
         return out
-    m = mask.detach().contiguous()
-    if m.dtype == torch.bool:
-        m = m.view(torch.uint8)
     L = _lib.lib()
     ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
     _lib.check(L.tl_boundary_workspace_bytes(n, H, W, ctypes.byref(ns), ctypes.byref(nc)), "tl_boundary_workspace_bytes")
     with torch.cuda.device(dev):
         scratch = torch.empty(nc.value, dtype=torch.uint8, device=dev)  # per call: released to the caching allocator
-        if sp is None:
-            rc = L.tl_signed_distance(m.data_ptr(), n, H, W, scratch.data_ptr(), scratch.numel(), out.data_ptr(),
-                                      _stream_ptr(dev))
-        else:
-            rc = L.tl_signed_distance_spaced(m.data_ptr(), n, H, W, sp.data_ptr(), scratch.data_ptr(), scratch.numel(),
-                                             out.data_ptr(), _stream_ptr(dev))
-    _lib.check(rc, "tl_signed_distance" if sp is None else "tl_signed_distance_spaced")
+        rc = L.tl_signed_distance(m.data_ptr(), n, H, W, _ptr(sp), scratch.data_ptr(), scratch.numel(), out.data_ptr(),
+                                  _stream_ptr(dev))
+    _lib.check(rc, "tl_signed_distance")
     return out
 
 
 class _BoundaryFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, t, sp):
-        B, C, H, W = (int(d) for d in x.shape)
-        n = B * C
-        dev = x.device
-        L = _lib.lib()
-        ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
-        _lib.check(L.tl_boundary_workspace_bytes(n, H, W, ctypes.byref(ns), ctypes.byref(nc)),
-                   "tl_boundary_workspace_bytes")
-        with torch.cuda.device(dev):
-            state = torch.empty(ns.value, dtype=torch.uint8, device=dev)  # phi per pixel: the backward reads it
-            scratch = torch.empty(nc.value, dtype=torch.uint8, device=dev)  # per call, freed when the forward returns
-            cost = torch.empty((B, C), dtype=torch.float32, device=dev)
-            if sp is None:
-                rc = L.tl_boundary_forward(x.data_ptr(), t.data_ptr(), n, H, W, state.data_ptr(), state.numel(),
-                                           scratch.data_ptr(), scratch.numel(), cost.data_ptr(), _stream_ptr(dev))
-            else:
-                rc = L.tl_boundary_forward_spaced(x.data_ptr(), t.data_ptr(), n, H, W, sp.data_ptr(), state.data_ptr(),
-                                                  state.numel(), scratch.data_ptr(), scratch.numel(), cost.data_ptr(),
-                                                  _stream_ptr(dev))
-        _lib.check(rc, "tl_boundary_forward" if sp is None else "tl_boundary_forward_spaced")
+        cost, state = _loss_forward("tl_boundary_forward", "tl_boundary_workspace_bytes", x, t, _ptr(sp))
         ctx.save_for_backward(x, state)
         return cost
 
@@ -425,21 +390,9 @@ def boundary_loss(masks: torch.Tensor, gt_masks: torch.Tensor, spacing=None) -> 
     the forward nor the backward synchronises the host.  The forward keeps phi (4 bytes per pixel) for the backward,
     and takes 8 bytes per pixel of scratch from PyTorch's caching allocator for the duration of the call; nothing is
     kept between calls."""
-    if not (torch.is_tensor(masks) and torch.is_tensor(gt_masks)):
-        raise TypeError("masks and gt_masks must be tensors")
-    if masks.dim() != 4 or masks.shape != gt_masks.shape:
-        raise ValueError("expected two [B, C, H, W] tensors of the same shape")
-    if not masks.is_cuda or not gt_masks.is_cuda:
-        raise ValueError("boundary_loss runs on a CUDA device only: there is no CPU fallback")
-    if masks.device != gt_masks.device:
-        raise ValueError(f"masks are on {masks.device}, gt_masks on {gt_masks.device}")
-    if masks.dtype != torch.float32:
-        raise ValueError(f"boundary_loss expects float32 logits, got {masks.dtype}")
-    if gt_masks.dtype.is_complex:
-        raise ValueError(f"boundary_loss expects a real or bool gt_masks, got {gt_masks.dtype}")
-    B, C, H, W = (int(d) for d in masks.shape)
-    _check_hw(H, W, "boundary_loss")
+    _logits_and_target(masks, gt_masks, "boundary_loss")
+    n, _, _ = _check_hw(masks.shape, "boundary_loss")
     sp = None if spacing is None else _spacing_tensor(spacing, masks.shape[:2], masks.device, "boundary_loss")
-    if B * C == 0:
+    if n == 0:
         return masks.sum((2, 3))  # empty, still attached to autograd
     return _BoundaryFn.apply(masks.contiguous(), gt_masks.detach().to(torch.float32).contiguous(), sp)

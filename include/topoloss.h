@@ -52,7 +52,7 @@ extern "C" {
 #define TL_ERR_WORKSPACE (-2) /* workspace too small */
 #define TL_ERR_CUDA (-3)      /* a CUDA runtime call failed; see tl_last_error() */
 
-#define TL_ABI_VERSION 4
+#define TL_ABI_VERSION 5
 
 /* ABI version of the loaded library (TL_ABI_VERSION it was built with). */
 int tl_version(void);
@@ -373,12 +373,22 @@ int tl_prior_backward(const float* maps, int n_maps, int H, int W, int dim, cons
                       const float* grad_cost, float* grad_maps, void* stream);
 
 /*
- * Exact Euclidean distance transform of n_maps HxW binary maps (H, W in [1, 4096]), unit spacing, pixel centres.
+ * Physical pixel spacing (DESIGN §3.10).  Every distance entry point below takes `spacing`: NULL for unit spacing,
+ * computed in integers; otherwise a device array [n_maps][2] of fp64 (sy, sx), 8-byte aligned: the size of a pixel
+ * along dim -2 (rows) and along dim -1 (columns), scipy's `sampling` order.  For a zero pixel at offset (dy, dx) the
+ * squared distance is then the fp64 value
+ *   a = float64(dy) * sy;  b = float64(dx) * sx;  s = a*a + b*b        (each operation rounded, no contraction)
+ * and the distance is float32(sqrt(min s)): what scipy.ndimage.distance_transform_edt(m, sampling=(sy, sx)) gives,
+ * bit for bit.  The device cannot check the values: each must be finite and in [1e-6, 1e6], which keeps every square
+ * normal in fp64 and every output finite in fp32; that is the caller's contract.  Distances, and every quantity made
+ * from them, are then in the spacing's units.  The backward entry points and the workspace queries take no spacing.
+ *
+ * Exact Euclidean distance transform of n_maps HxW binary maps (H, W in [1, 4096]), pixel centres.
  *
  * tl_edt_workspace_bytes  *bytes (host pointer): the scratch tl_edt needs, 4 bytes per pixel.
  * tl_edt                  mask[n_maps][H][W] (uint8, device; nonzero = feature) -> out[n_maps][H][W] (fp32, device):
- *                         0 at a zero pixel; at a nonzero pixel float32(sqrt(float64(s))) with s the exact integer
- *                         squared distance to the nearest zero pixel of the same map -- what
+ *                         0 at a zero pixel; at a nonzero pixel float32(sqrt(float64(s))) with s the exact squared
+ *                         distance to the nearest zero pixel of the same map -- what
  *                         scipy.ndimage.distance_transform_edt(m).astype(float32) gives, bit for bit, on a map with a
  *                         zero pixel.  A map without a zero pixel gets +inf everywhere.  ws must be 4-byte aligned.
  *
@@ -398,22 +408,24 @@ int tl_prior_backward(const float* maps, int n_maps, int H, int W, int dim, cons
  *                                  those of the forward; state 4-byte aligned.
  *
  * Every argument error (null pointer, H or W out of range, a non-finite or non-positive alpha, a buffer smaller than
- * the query asks for or misaligned) returns TL_ERR_ARG before any launch.
+ * the query asks for or misaligned, a misaligned spacing) returns TL_ERR_ARG before any launch.
  */
 int tl_edt_workspace_bytes(int n_maps, int H, int W, size_t* bytes);
-int tl_edt(const uint8_t* mask, int n_maps, int H, int W, void* ws, size_t ws_bytes, float* out, void* stream);
+int tl_edt(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes, float* out,
+           void* stream);
 int tl_hausdorff_dt_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes);
 int tl_hausdorff_dt_forward(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
-                            void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
-                            void* stream);
+                            const double* spacing, void* state, size_t state_bytes, void* scratch,
+                            size_t scratch_bytes, float* cost, void* stream);
 int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_maps, int H, int W, const void* state,
                              size_t state_bytes, const float* grad_cost, float* grad_logits, void* stream);
 
 /*
- * Surface-distance metrics of n_maps pairs of HxW binary maps (H, W in [1, 4096]), unit spacing, pixel centres.
- * Per map: the surface S(M) = M & ~binary_erosion(M) (cross structure, outside = 0) -- the nonzero pixels with a zero
- * or an outside 4-neighbour; d_pt the exact distance sqrt(float64(s)) from each pixel of S(pred) to the nearest pixel
- * of S(target), d_tp the same the other way; n_p = |S(pred)|, n_t = |S(target)|.  Computed in fp64, rounded to fp32:
+ * Surface-distance metrics of n_maps pairs of HxW binary maps (H, W in [1, 4096]), pixel centres, with the spacing
+ * above.  Per map: the surface S(M) = M & ~binary_erosion(M) (cross structure, outside = 0) -- the nonzero pixels with
+ * a zero or an outside 4-neighbour; d_pt the exact distance sqrt(float64(s)) from each pixel of S(pred) to the nearest
+ * pixel of S(target), d_tp the same the other way; n_p = |S(pred)|, n_t = |S(target)|.  Computed in fp64, rounded to
+ * fp32:
  *   hausdorff             max(max d_pt, max d_tp)
  *   hausdorff_percentile  max(pct(d_pt, q), pct(d_tp, q)), pct numpy's default (linear) percentile, q = percentile
  *   assd                  (sum d_pt + sum d_tp) / (n_p + n_t)
@@ -423,42 +435,16 @@ int tl_hausdorff_dt_backward(const float* logits, const float* target, int n_map
  * tl_surface_workspace_bytes  *bytes (host pointer): the scratch tl_surface_distances needs, about 16 bytes per pixel.
  * tl_surface_distances        pred, target [n_maps][H][W] (uint8, device; nonzero = foreground) -> out[4][n_maps]
  *                             (fp32, device): hausdorff, hausdorff_percentile, assd, nsd.  percentile in [0, 100],
- *                             tolerance finite and >= 0; ws 4-byte aligned.  Four launches, no host synchronisation,
- *                             bit-identical from run to run.
+ *                             tolerance finite and >= 0, in the spacing's units; ws 4-byte aligned.  Four launches, no
+ *                             host synchronisation, bit-identical from run to run.
  *
  * Every argument error (null pointer, H or W out of range, a percentile outside [0, 100] or NaN, a negative or
- * non-finite tolerance, a workspace smaller than the query asks for or misaligned) returns TL_ERR_ARG before any launch.
+ * non-finite tolerance, a workspace smaller than the query asks for or misaligned, a misaligned spacing) returns
+ * TL_ERR_ARG before any launch.
  */
 int tl_surface_workspace_bytes(int n_maps, int H, int W, size_t* bytes);
-int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, double percentile,
-                         double tolerance, void* ws, size_t ws_bytes, float* out, void* stream);
-
-/*
- * Physical pixel spacing for the three entry points above (DESIGN §3.10).  spacing is a device array
- * [n_maps][2] of fp64 (sy, sx), 8-byte aligned: the size of a pixel along dim -2 (rows) and along dim -1 (columns),
- * scipy's `sampling` order.  For a zero pixel at offset (dy, dx) the squared distance is the fp64 value
- *   a = float64(dy) * sy;  b = float64(dx) * sx;  s = a*a + b*b        (each operation rounded, no contraction)
- * and the distance is float32(sqrt(min s)): what scipy.ndimage.distance_transform_edt(m, sampling=(sy, sx)) gives,
- * bit for bit.  The device cannot check the values: each must be finite and in [1e-6, 1e6], which keeps every square
- * normal in fp64 and every output finite in fp32; that is the caller's contract.
- *
- * tl_edt_spaced                    as tl_edt, with the workspace of tl_edt_workspace_bytes.
- * tl_hausdorff_dt_forward_spaced   as tl_hausdorff_dt_forward with F the spaced distance (D and the cost in physical
- *                                  units), with the buffers of tl_hausdorff_dt_workspace_bytes; the backward is
- *                                  tl_hausdorff_dt_backward.
- * tl_surface_distances_spaced      as tl_surface_distances with d_pt, d_tp the spaced distances and tolerance in the
- *                                  same units, with the workspace of tl_surface_workspace_bytes.
- *
- * Every argument error of the unspaced entry, and a null or misaligned spacing, returns TL_ERR_ARG before any launch.
- */
-int tl_edt_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* ws, size_t ws_bytes,
-                  float* out, void* stream);
-int tl_hausdorff_dt_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W, double alpha,
-                                   const double* spacing, void* state, size_t state_bytes, void* scratch,
-                                   size_t scratch_bytes, float* cost, void* stream);
-int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W,
-                                const double* spacing, double percentile, double tolerance, void* ws, size_t ws_bytes,
-                                float* out, void* stream);
+int tl_surface_distances(const uint8_t* pred, const uint8_t* target, int n_maps, int H, int W, const double* spacing,
+                         double percentile, double tolerance, void* ws, size_t ws_bytes, float* out, void* stream);
 
 /*
  * Signed distance map and the boundary loss of Kervadec et al. (MIDL 2019, MedIA 2021) on n_maps HxW maps (H, W in
@@ -466,8 +452,8 @@ int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int 
  * to fp32:
  *   phi = d_out                on the background, d_out the distance to the nearest foreground pixel
  *       = 1 - d_in             on the foreground, d_in the distance to the nearest background pixel
- * -- scipy's edt(~M) * ~M - (edt(M) - 1) * M bit for bit, with the distances of tl_edt (unit) or tl_edt_spaced (the
- * `1` is then in the spacing's units).  A map with one label only gets phi = 0 everywhere.
+ * -- scipy's edt(~M) * ~M - (edt(M) - 1) * M bit for bit, with the distances of tl_edt (with a spacing, the `1` is in
+ * the spacing's units).  A map with one label only gets phi = 0 everywhere.
  * The loss, per map of fp32 logits x and targets t: p = sigmoid(x) (fp32, as torch.sigmoid), phi = phi(t > 0.5) and
  *   cost = (1 / HW) * sum_i p_i * phi_i      (fp64, fixed order, rounded to fp32)
  *
@@ -480,24 +466,18 @@ int tl_surface_distances_spaced(const uint8_t* pred, const uint8_t* target, int 
  *                              aligned.
  * tl_signed_distance           mask[n_maps][H][W] (uint8, device; nonzero = foreground) -> out[n_maps][H][W] (fp32,
  *                              device): phi, with the scratch of tl_boundary_workspace_bytes (8-byte aligned).
- * tl_*_spaced                  the same with a device fp64 spacing [n_maps][2] (sy, sx), 8-byte aligned, as for
- *                              tl_edt_spaced; tl_boundary_backward serves both forwards.
  *
  * Every argument error (null pointer, H or W out of range, a buffer smaller than the query asks for or misaligned, a
- * null or misaligned spacing) returns TL_ERR_ARG before any launch.  No entry point synchronises the host.
+ * misaligned spacing) returns TL_ERR_ARG before any launch.  No entry point synchronises the host.
  */
 int tl_boundary_workspace_bytes(int n_maps, int H, int W, size_t* state_bytes, size_t* scratch_bytes);
-int tl_boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, void* state,
-                        size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost, void* stream);
-int tl_boundary_forward_spaced(const float* logits, const float* target, int n_maps, int H, int W,
-                               const double* spacing, void* state, size_t state_bytes, void* scratch,
-                               size_t scratch_bytes, float* cost, void* stream);
+int tl_boundary_forward(const float* logits, const float* target, int n_maps, int H, int W, const double* spacing,
+                        void* state, size_t state_bytes, void* scratch, size_t scratch_bytes, float* cost,
+                        void* stream);
 int tl_boundary_backward(const float* logits, int n_maps, int H, int W, const void* state, size_t state_bytes,
                          const float* grad_cost, float* grad_logits, void* stream);
-int tl_signed_distance(const uint8_t* mask, int n_maps, int H, int W, void* scratch, size_t scratch_bytes, float* out,
-                       void* stream);
-int tl_signed_distance_spaced(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
-                              size_t scratch_bytes, float* out, void* stream);
+int tl_signed_distance(const uint8_t* mask, int n_maps, int H, int W, const double* spacing, void* scratch,
+                       size_t scratch_bytes, float* out, void* stream);
 
 #ifdef __cplusplus
 }

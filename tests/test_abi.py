@@ -34,6 +34,19 @@ def test_library_exports_every_declared_symbol():
     assert set(_lib.SIGNATURES) <= set(_declared())
 
 
+def test_distance_ops_have_one_entry_point_each():
+    """ABI 5: each distance op takes its spacing as an argument (NULL: unit spacing); the _spaced twins are gone."""
+    from dilabhelmholtzoct_b200 import _lib, build
+    if not os.path.exists(build.LIB_PATH):
+        build.build()
+    L = ctypes.CDLL(build.LIB_PATH)
+    assert _lib.ABI_VERSION == 5
+    for op in ("tl_edt", "tl_hausdorff_dt_forward", "tl_surface_distances", "tl_signed_distance", "tl_boundary_forward"):
+        assert op in _declared() and hasattr(L, op) and op in _lib.SIGNATURES, op
+        gone = op + "_spaced"
+        assert gone not in _declared() and not hasattr(L, gone) and gone not in _lib.SIGNATURES, gone
+
+
 def _ws(L, B, C, H, W, d):
     ns, nc = ctypes.c_size_t(0), ctypes.c_size_t(0)
     rc = L.tl_workspace_bytes(B, C, H, W, d, ctypes.byref(ns), ctypes.byref(nc))

@@ -86,8 +86,7 @@ def test_kat_cost():
 
 # ---------------------------------------------------------------- CPU: the C ABI
 
-NEW_NAMES = ("tl_boundary_workspace_bytes", "tl_boundary_forward", "tl_boundary_forward_spaced", "tl_boundary_backward",
-             "tl_signed_distance", "tl_signed_distance_spaced")
+NEW_NAMES = ("tl_boundary_workspace_bytes", "tl_boundary_forward", "tl_boundary_backward", "tl_signed_distance")
 BAD_SHAPES = ((0, 16, 16), (-1, 16, 16), (2, 0, 16), (2, 16, 0), (2, 4097, 16), (2, 16, 4097))
 
 
@@ -100,7 +99,9 @@ def test_new_entry_points_are_declared_exported_and_bound():
     src = re.sub(r"/\*.*?\*/", "", open(os.path.join(root, "include", "topoloss.h")).read(), flags=re.S)
     for name in NEW_NAMES:
         assert re.search(rf"\b{name}\s*\(", src) and name in _lib.SIGNATURES and hasattr(_lib.lib(), name), name
-    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 4
+    for name in ("tl_boundary_forward_spaced", "tl_signed_distance_spaced"):  # ABI 5: spacing is an argument
+        assert not re.search(rf"\b{name}\s*\(", src) and name not in _lib.SIGNATURES and not hasattr(_lib.lib(), name)
+    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 5
     for name in ("boundary_loss", "signed_distance_map"):
         assert name in tlb.__all__ and callable(getattr(tlb, name))
 
@@ -139,20 +140,16 @@ def test_new_entry_points_reject_bad_arguments():
     ns, nc = 3 * 256 * 4, 3 * 256 * 8
     shapes = lambda at: [(slice(at, at + 3), s) for s in BAD_SHAPES]  # noqa: E731
 
-    # tl_boundary_forward(logits, target, n, H, W, state, state_bytes, scratch, scratch_bytes, cost, stream)
-    ok = [fake, fake, 3, 16, 16, fake, ns, fake, nc, fake, None]
-    _all_fail(L.tl_boundary_forward, ok, [(0, None), (1, None), (5, None), (7, None), (9, None), (5, fake + 2),
-                                          (7, fake + 4), (6, ns - 1), (8, nc - 1)] + shapes(2))
-    for i, bad in ((6, ns - 1), (8, nc - 1)):
-        a = list(ok)
-        a[i] = bad
-        _short_buffer_names_the_query(L.tl_boundary_forward, a)
-
-    # tl_boundary_forward_spaced(logits, target, n, H, W, spacing, state, state_bytes, scratch, scratch_bytes, cost, s)
-    ok = [fake, fake, 3, 16, 16, fake, fake, ns, fake, nc, fake, None]
-    _all_fail(L.tl_boundary_forward_spaced, ok,
-              [(0, None), (1, None), (5, None), (6, None), (8, None), (10, None), (5, fake + 4), (6, fake + 2),
-               (8, fake + 4), (7, ns - 1), (9, nc - 1)] + shapes(2))
+    # tl_boundary_forward(logits, target, n, H, W, spacing, state, state_bytes, scratch, scratch_bytes, cost, stream);
+    # every case fails with a null (unit) or a device spacing
+    for sp in (None, fake):
+        ok = [fake, fake, 3, 16, 16, sp, fake, ns, fake, nc, fake, None]
+        _all_fail(L.tl_boundary_forward, ok, [(0, None), (1, None), (6, None), (8, None), (10, None), (5, fake + 4),
+                                              (6, fake + 2), (8, fake + 4), (7, ns - 1), (9, nc - 1)] + shapes(2))
+        for i, bad in ((7, ns - 1), (9, nc - 1)):
+            a = list(ok)
+            a[i] = bad
+            _short_buffer_names_the_query(L.tl_boundary_forward, a)
 
     # tl_boundary_backward(logits, n, H, W, state, state_bytes, grad_cost, grad_logits, stream)
     ok = [fake, 3, 16, 16, fake, ns, fake, fake, None]
@@ -162,17 +159,14 @@ def test_new_entry_points_reject_bad_arguments():
     a[5] = ns - 1
     _short_buffer_names_the_query(L.tl_boundary_backward, a)
 
-    # tl_signed_distance(mask, n, H, W, scratch, scratch_bytes, out, stream)
-    ok = [fake, 3, 16, 16, fake, nc, fake, None]
-    _all_fail(L.tl_signed_distance, ok, [(0, None), (4, None), (6, None), (4, fake + 4), (5, nc - 1)] + shapes(1))
-    a = list(ok)
-    a[5] = nc - 1
-    _short_buffer_names_the_query(L.tl_signed_distance, a)
-
-    # tl_signed_distance_spaced(mask, n, H, W, spacing, scratch, scratch_bytes, out, stream)
-    ok = [fake, 3, 16, 16, fake, fake, nc, fake, None]
-    _all_fail(L.tl_signed_distance_spaced, ok,
-              [(0, None), (4, None), (5, None), (7, None), (4, fake + 4), (5, fake + 4), (6, nc - 1)] + shapes(1))
+    # tl_signed_distance(mask, n, H, W, spacing, scratch, scratch_bytes, out, stream)
+    for sp in (None, fake):
+        ok = [fake, 3, 16, 16, sp, fake, nc, fake, None]
+        _all_fail(L.tl_signed_distance, ok, [(0, None), (5, None), (7, None), (4, fake + 4), (5, fake + 4), (6, nc - 1)]
+                  + shapes(1))
+        a = list(ok)
+        a[6] = nc - 1
+        _short_buffer_names_the_query(L.tl_signed_distance, a)
 
 
 def test_python_checks_raise_on_the_cpu():

@@ -93,7 +93,7 @@ def test_new_entry_points_are_declared_exported_and_bound():
     L = ctypes.CDLL(build.LIB_PATH)
     for name in NEW:
         assert name in declared and hasattr(L, name) and name in _lib.SIGNATURES, name
-    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 4
+    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 5
     for name in ("distance_transform_edt", "hausdorff_dt_loss"):
         assert name in tlb.__all__ and callable(getattr(tlb, name))
 
@@ -121,25 +121,31 @@ def test_new_entry_points_reject_bad_arguments():
     L = _lib.lib()
     fake = 4096  # never dereferenced: every call below fails its host-side checks before any launch
     nw = 4 * 3 * 16 * 16
-    ok = [fake, 3, 16, 16, fake, nw, fake, None]
-    cases = [(0, None), (4, None), (6, None), (4, fake + 2), (5, nw - 1)] + [(slice(1, 4), s) for s in BAD_SHAPES]
-    for i, bad in cases:
-        a = list(ok)
-        a[i] = bad
-        assert L.tl_edt(*a) == -1, (i, bad)
-    assert L.tl_edt(*(ok[:5] + [nw - 1] + ok[6:])) == -1 and b"tl_edt_workspace_bytes" in L.tl_last_error()
+    # tl_edt(mask, n, H, W, spacing, ws, ws_bytes, out, stream); every case fails with a null (unit) or a device spacing
+    cases = [(0, None), (5, None), (7, None), (4, fake + 4), (5, fake + 2), (6, nw - 1)]
+    cases += [(slice(1, 4), s) for s in BAD_SHAPES]
+    for sp in (None, fake):
+        ok = [fake, 3, 16, 16, sp, fake, nw, fake, None]
+        for i, bad in cases:
+            a = list(ok)
+            a[i] = bad
+            assert L.tl_edt(*a) == -1, (sp, i, bad)
+        assert L.tl_edt(*(ok[:6] + [nw - 1] + ok[7:])) == -1 and b"tl_edt_workspace_bytes" in L.tl_last_error()
 
     ns, nc = 3 * 256 * 4, 3 * 256 * 8
-    ok = [fake, fake, 3, 16, 16, 2.0, fake, ns, fake, nc, fake, None]
-    cases = [(0, None), (1, None), (6, None), (8, None), (10, None), (6, fake + 2), (8, fake + 4),
-             (5, 0.0), (5, -1.0), (5, math.inf), (5, -math.inf), (5, math.nan), (7, ns - 1), (9, nc - 1)]
+    # tl_hausdorff_dt_forward(logits, target, n, H, W, alpha, spacing, state, state_bytes, scratch, scratch_bytes,
+    # cost, stream)
+    cases = [(0, None), (1, None), (7, None), (9, None), (11, None), (6, fake + 4), (7, fake + 2), (9, fake + 4),
+             (5, 0.0), (5, -1.0), (5, math.inf), (5, -math.inf), (5, math.nan), (8, ns - 1), (10, nc - 1)]
     cases += [(slice(2, 5), s) for s in BAD_SHAPES]
-    for i, bad in cases:
-        a = list(ok)
-        a[i] = bad
-        assert L.tl_hausdorff_dt_forward(*a) == -1, (i, bad)
-    assert L.tl_hausdorff_dt_forward(*(ok[:9] + [nc - 1] + ok[10:])) == -1
-    assert b"tl_hausdorff_dt_workspace_bytes" in L.tl_last_error()
+    for sp in (None, fake):
+        ok = [fake, fake, 3, 16, 16, 2.0, sp, fake, ns, fake, nc, fake, None]
+        for i, bad in cases:
+            a = list(ok)
+            a[i] = bad
+            assert L.tl_hausdorff_dt_forward(*a) == -1, (sp, i, bad)
+        assert L.tl_hausdorff_dt_forward(*(ok[:10] + [nc - 1] + ok[11:])) == -1
+        assert b"tl_hausdorff_dt_workspace_bytes" in L.tl_last_error()
 
     ok = [fake, fake, 3, 16, 16, fake, ns, fake, fake, None]
     cases = [(0, None), (1, None), (5, None), (7, None), (8, None), (6, ns - 1), (5, fake + 2)]

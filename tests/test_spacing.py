@@ -119,45 +119,34 @@ def test_new_entry_points_are_declared_and_bound():
     from dilabhelmholtzoct_b200 import _lib
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     src = re.sub(r"/\*.*?\*/", "", open(os.path.join(root, "include", "topoloss.h")).read(), flags=re.S)
-    for name in ("tl_edt_spaced", "tl_hausdorff_dt_forward_spaced", "tl_surface_distances_spaced"):
-        assert re.search(rf"\b{name}\s*\(", src) and name in _lib.SIGNATURES and hasattr(_lib.lib(), name)
-    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 4
+    for name in ("tl_edt", "tl_hausdorff_dt_forward", "tl_surface_distances"):
+        # the spacing is an argument of the op's one entry point, right after the shape
+        assert re.search(rf"\b{name}\s*\([^)]*int W,\s*(double alpha,\s*)?const double\* spacing", src), name
+        assert name in _lib.SIGNATURES and hasattr(_lib.lib(), name)
+        assert not re.search(rf"\b{name}_spaced\s*\(", src) and not hasattr(_lib.lib(), name + "_spaced")
+    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 5
 
 
 BAD_SHAPES = ((0, 16, 16), (-1, 16, 16), (2, 0, 16), (2, 16, 0), (2, 4097, 16), (2, 16, 4097))
 
 
-def _all_fail(fn, ok, cases):
-    for i, bad in cases:
-        a = list(ok)
-        a[i] = bad
-        assert fn(*a) == -1, (i, bad)
-
-
 def test_new_entry_points_reject_bad_arguments():
+    """A misaligned spacing fails before any launch, and says so; the other argument errors of these entry points,
+    with a null or a device spacing, are in test_distance_transform.py and test_surface_distance.py."""
     from dilabhelmholtzoct_b200 import _lib
     L = _lib.lib()
     fake = 4096  # never dereferenced: every call below fails its host-side checks before any launch
-    nw = 4 * 3 * 16 * 16
-    ok = [fake, 3, 16, 16, fake, fake, nw, fake, None]
-    _all_fail(L.tl_edt_spaced, ok, [(0, None), (4, None), (5, None), (7, None), (4, fake + 4), (5, fake + 2),
-                                    (6, nw - 1)] + [(slice(1, 4), s) for s in BAD_SHAPES])
-
-    ns, nc = 3 * 256 * 4, 3 * 256 * 8
-    ok = [fake, fake, 3, 16, 16, 2.0, fake, fake, ns, fake, nc, fake, None]
-    _all_fail(L.tl_hausdorff_dt_forward_spaced, ok,
-              [(0, None), (1, None), (6, None), (7, None), (9, None), (11, None), (6, fake + 4), (7, fake + 2),
-               (9, fake + 4), (5, 0.0), (5, -1.0), (5, math.inf), (5, math.nan), (8, ns - 1), (10, nc - 1)]
-              + [(slice(2, 5), s) for s in BAD_SHAPES])
-
+    nw, ns, nc = 4 * 3 * 16 * 16, 3 * 256 * 4, 3 * 256 * 8
     nb = ctypes.c_size_t(0)
     assert L.tl_surface_workspace_bytes(3, 16, 16, ctypes.byref(nb)) == 0
-    nw = nb.value
-    ok = [fake, fake, 3, 16, 16, fake, 95.0, 1.0, fake, nw, fake, None]
-    _all_fail(L.tl_surface_distances_spaced, ok,
-              [(0, None), (1, None), (5, None), (8, None), (10, None), (5, fake + 4), (8, fake + 2), (9, nw - 1),
-               (6, -1e-9), (6, 100.5), (6, math.nan), (7, -0.5), (7, math.inf), (7, math.nan)]
-              + [(slice(2, 5), s) for s in BAD_SHAPES])
+    calls = [(L.tl_edt, [fake, 3, 16, 16, fake, fake, nw, fake, None], 4),
+             (L.tl_hausdorff_dt_forward, [fake, fake, 3, 16, 16, 2.0, fake, fake, ns, fake, nc, fake, None], 6),
+             (L.tl_surface_distances, [fake, fake, 3, 16, 16, fake, 95.0, 1.0, fake, nb.value, fake, None], 5)]
+    for fn, ok, at in calls:
+        for off in (1, 2, 4):
+            a = list(ok)
+            a[at] = fake + off
+            assert fn(*a) == -1 and b"spacing" in L.tl_last_error(), (fn, off)
 
 
 def test_python_checks_raise_value_errors_on_the_cpu():

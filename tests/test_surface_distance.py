@@ -149,7 +149,7 @@ def test_new_entry_points_are_declared_exported_and_bound():
     L = ctypes.CDLL(build.LIB_PATH)
     for name in NEW:
         assert name in declared and hasattr(L, name) and name in _lib.SIGNATURES, name
-    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 4
+    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 5
     for name in ("surface_distances", "SurfaceDistances"):
         assert name in tlb.__all__ and callable(getattr(tlb, name))
     assert tlb.SurfaceDistances._fields == FIELDS
@@ -169,23 +169,26 @@ def test_workspace_query_and_bad_arguments():
     nw = nb.value
     assert nw >= 16 * 3 * 256 + 16 * 3
     fake = 4096  # never dereferenced: every call below fails its host-side checks before any launch
-    ok = [fake, fake, 3, 16, 16, 95.0, 1.0, fake, nw, fake, None]
-    cases = [(0, None), (1, None), (7, None), (9, None), (7, fake + 2), (8, nw - 1),
-             (5, -1e-9), (5, 100.5), (5, math.nan), (5, math.inf), (5, -math.inf),
-             (6, -0.5), (6, math.inf), (6, math.nan)]
+    # tl_surface_distances(pred, target, n, H, W, spacing, percentile, tolerance, ws, ws_bytes, out, stream); every
+    # case fails with a null (unit) or a device spacing
+    cases = [(0, None), (1, None), (8, None), (10, None), (5, fake + 4), (8, fake + 2), (9, nw - 1),
+             (6, -1e-9), (6, 100.5), (6, math.nan), (6, math.inf), (6, -math.inf),
+             (7, -0.5), (7, math.inf), (7, math.nan)]
     cases += [(slice(2, 5), s) for s in BAD_SHAPES]
-    for i, bad in cases:
+    for sp in (None, fake):
+        ok = [fake, fake, 3, 16, 16, sp, 95.0, 1.0, fake, nw, fake, None]
+        for i, bad in cases:
+            a = list(ok)
+            a[i] = bad
+            assert L.tl_surface_distances(*a) == -1, (sp, i, bad)
+        assert L.tl_surface_distances(*(ok[:9] + [nw - 1] + ok[10:])) == -1
+        assert b"tl_surface_workspace_bytes" in L.tl_last_error()
         a = list(ok)
-        a[i] = bad
-        assert L.tl_surface_distances(*a) == -1, (i, bad)
-    assert L.tl_surface_distances(*(ok[:8] + [nw - 1] + ok[9:])) == -1
-    assert b"tl_surface_workspace_bytes" in L.tl_last_error()
-    a = list(ok)
-    a[5] = 101.0
-    assert L.tl_surface_distances(*a) == -1 and b"percentile" in L.tl_last_error()
-    a = list(ok)
-    a[6] = -1.0
-    assert L.tl_surface_distances(*a) == -1 and b"tolerance" in L.tl_last_error()
+        a[6] = 101.0
+        assert L.tl_surface_distances(*a) == -1 and b"percentile" in L.tl_last_error()
+        a = list(ok)
+        a[7] = -1.0
+        assert L.tl_surface_distances(*a) == -1 and b"tolerance" in L.tl_last_error()
 
 
 def test_python_checks_raise_value_errors_on_the_cpu():

@@ -113,7 +113,7 @@ def test_new_entry_points_are_declared_exported_and_bound():
     L = ctypes.CDLL(build.LIB_PATH)
     for name in NEW:
         assert name in declared and hasattr(L, name) and name in _lib.SIGNATURES, name
-    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 4
+    assert _lib.lib().tl_version() == _lib.ABI_VERSION == 5
     assert "topological_prior" in tlb.__all__ and callable(tlb.topological_prior)
 
 
